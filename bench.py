@@ -2,7 +2,7 @@
 """Benchmark of the fused max-mean similarity + symmetric InfoNCE path (fwd + bwd).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl triad|reference] [--config auto|cfg2|cfg3|cfg4]
-                    [--verify] [--no-extras] [--no-cpu-baseline]
+                    [--verify] [--no-extras] [--no-cpu-baseline] [--dump-outputs DIR]
 
 metric: clip-pairs/sec = B_global^2 / t(step)   (BASELINE.json).  One "step" = one forward + backward of the hot path
 over one synthetic batch.  N=1 runs BASELINE cfg 2 (B=256, 250 frames x 256 patches, D=512, bf16); N>1 (launched by
@@ -20,6 +20,8 @@ N=1 extras (each with its own clock sample and roofline): `full_loss`, `cfg3`, `
 N>1 extras: `parity` (the W-rank step vs the single-GPU step on the gathered batch, on the GPUs, before timing)
 and `cfg5_sharded` (gallery sharded by images, local top-k + all-gather merge).
 `--impl reference`: only the CPU arm, as its own JSON line.   `--verify`: only the N-rank parity check.
+`--dump-outputs DIR` (N=1): what the last timed step returned to its caller, as DIR/<name>.npy (see dump_outputs).  The
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -265,6 +267,25 @@ def rel_err(a, b):
     return ((a - b).norm() / b.norm().clamp(min=1e-30)).item()
 
 
+DUMP_ROWS = 32          # batch rows that --dump-outputs writes of the batch-sized outputs
+
+
+def dump_outputs(path, outs):
+    """Writes one step's results as path/<name>.npy, float32: `loss`, `grad_temperature`, and on DUMP_ROWS batch rows
+    drawn with a fixed seed (listed in `sample_rows`) `clip_sims` [DUMP_ROWS, B], `grad_q` [DUMP_ROWS, Nq, D] and
+    `grad_v` [DUMP_ROWS, Nv, D].  Whole, the two gradients of cfg 2 would take 130 MB each, clip_sims of cfg 4 268 MB."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    B = outs["clip_sims"].shape[0]
+    rows = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    arrays = {"loss": outs["loss"], "grad_temperature": outs["grad_temperature"], "sample_rows": rows}
+    for name in ("clip_sims", "grad_q", "grad_v"):
+        arrays[name] = outs[name][rows.to(outs[name].device)]
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def verify_sharded(world, rank, dev, group=None):
     """N-rank parity on the GPUs (NCCL): sharded_contrastive_step on W shards vs the single-GPU drop-in on the gathered
     batch (every rank recomputes it), unmasked and masked; and, at a small size, vs the CPU oracle on rank 0.
@@ -381,9 +402,11 @@ def run_triad(args, cfg_key):
     model.triad_regularizers = False       # BASELINE.json's metric: max-mean similarity + InfoNCE, fwd + bwd
     T = model.temperature
     fwd_ev = []
+    last_step = {}
 
     def api_step(m, q, v, mask, record=False):
-        """One step through the drop-in methods (the calls forward_audio_visual / forward_text_visual make)."""
+        """One step through the drop-in methods (the calls forward_audio_visual / forward_text_visual make); its results
+        are kept in last_step until the next step."""
         q.grad = v.grad = m.temperature.grad = None
         if record:
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -396,6 +419,7 @@ def run_triad(args, cfg_key):
             e1.record(); fwd_ev.append((e0, e1))
         total = m.compute_contrastive_loss_av(clip, tok)[0] if mask is None else m.compute_contrastive_loss_tv(clip, tok)[0]
         total.backward()
+        last_step.update(loss=total, clip_sims=clip, grad_q=q.grad, grad_v=v.grad, grad_temperature=m.temperature.grad)
         return total
 
     def step_single(q, v, mask, record=False):
@@ -433,6 +457,8 @@ def run_triad(args, cfg_key):
         ms = timed(lambda i: step(*sets[i % n_sets], record=True), args.steps)
     gpu_launches = int(lib.triad_launch_count() - launches0)     # libtriad_b200.so kernels inside the timed region (this rank)
     value = float(B) * B / (ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_step)
 
     # ---- end-to-end arm: pinned host inputs -> H2D -> step -> loss D2H --------------------------
     # Every step's embeddings start in PINNED HOST memory and its loss is read back on the host.  As in any
@@ -491,7 +517,8 @@ def run_triad(args, cfg_key):
         assert seen["n"] == K and seen["last"] == seen["last"]      # K losses read on the host, finite
         staged.clear()                        # the look-ahead copy issued by the last step is not used
 
-    e2e_run(min(args.warmup, 3))
+    if args.warmup > 0:
+        e2e_run(min(args.warmup, 3))
     sync_all()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
@@ -788,10 +815,16 @@ def main():
     ap.add_argument("--no-cfg4-1gpu", action="store_true", help="skip the B=8192 single-GPU step (about 20 s)")
     ap.add_argument("--no-cfg5", action="store_true", help="skip the 104.9 GB retrieval block")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (single GPU, --impl triad)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.gpus != world and world > 1:
         args.gpus = world
+    if args.dump_outputs and (max(args.gpus, world) > 1 or args.impl != "triad" or args.verify):
+        ap.error("--dump-outputs needs --gpus 1 and --impl triad, without --verify")
     cfg_key = args.config if args.config != "auto" else ("cfg2" if max(args.gpus, world) == 1 else "cfg4")
     if args.impl == "reference":
         run_reference(args, cfg_key)

@@ -5,6 +5,7 @@ import hashlib
 import json
 import os
 import pickle
+import shutil
 
 import pytest
 import torch
@@ -41,15 +42,32 @@ def test_merge_topk_order():
     assert mi.tolist() == [2, 4, 7, 5] and ms.tolist() == [3.0, 3.0, 3.0, 2.0]   # score desc, ties to the lower id
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not present (GPU box)")
+# SHA-256 of the reference's src/model.py and src/retrieval.py, taken from the reference tree when oracle/_ref/ was staged
+REFERENCE_SHA256 = {
+    "model.py": "5d5d00fccac98ce98fe474ff25569cc2f5b715776cfb7b5850f275d9a1b5eafc",
+    "retrieval.py": "9029727c6c9729adf8f5dbace7fa95a0e69de17f26ea401c89ff19c2dc8871a2",
+}
+
+
 def test_staged_reference_is_the_reference_byte_for_byte(tmp_path, monkeypatch):
     from oracle import build_ref, ref_loader
+    for name, digest in REFERENCE_SHA256.items():
+        with open(os.path.join(build_ref.OUT, name), "rb") as f:
+            assert hashlib.sha256(f.read()).hexdigest() == digest, name
+    # the staging recipe, run on a reference tree laid out like the original: byte-for-byte copies, and the manifest
+    # that is kept in oracle/_ref/
+    src_root = tmp_path / "reference"
+    for rel in build_ref.FILES:
+        (src_root / rel).parent.mkdir(parents=True, exist_ok=True)
+        shutil.copyfile(os.path.join(build_ref.OUT, os.path.basename(rel)), src_root / rel)
+    staged = tmp_path / "staged"
+    monkeypatch.setattr(build_ref, "REF_ROOT", str(src_root))
+    monkeypatch.setattr(build_ref, "OUT", str(staged))
     assert build_ref.build()
-    man = json.load(open(os.path.join(build_ref.OUT, "MANIFEST.json")))
-    for name, meta in man.items():
-        src = open(os.path.join(build_ref.REF_ROOT, meta["source"]), "rb").read()
-        assert hashlib.sha256(src).hexdigest() == meta["sha256"]
-        assert open(os.path.join(build_ref.OUT, name), "rb").read() == src
+    with open(staged / "MANIFEST.json") as f, open(os.path.join(ref_loader.REF_DIR, "MANIFEST.json")) as g:
+        assert json.load(f) == json.load(g)
+    for rel in build_ref.FILES:
+        assert (staged / os.path.basename(rel)).read_bytes() == (src_root / rel).read_bytes()
     ref = ref_loader.load()
     assert ref is not None and hasattr(ref[0], "MultiModalModel") and hasattr(ref[1], "compute_recall_at_k")
 
