@@ -142,19 +142,17 @@ int triad_contrastive_head(const float* clip, int B, const float* temperature,
  *   dT        = sum_ij g[i,j]*clip[i,j] / T
  * g fp32 [Bq,Bv] is dLoss/dclip.  dq is written in `dtype` ([Bq,Nq,D]); dv is written as
  * fp32 [Bv,Nv,D] when dv_f32 != 0 (partial to be reduce-scattered across ranks) else in
- * `dtype`; dT fp32 [1].  Any of dq / dv / dT may be NULL to skip it. */
+ * `dtype`; dT fp32 [1].  Any of dq / dv / dT may be NULL to skip it.  `flags` is an OR of the
+ * TRIAD_BWD_* bits below; any other bit (4, 8 and 64 are retired) fails with TRIAD_ERR_BAD_ARG. */
 #define TRIAD_BWD_DEFAULT      0
 #define TRIAD_BWD_GENERIC_DQ   1   /* L2-served gather kernel for dq (always used for fp32 / D % 64 != 0) */
 #define TRIAD_BWD_GENERIC_DV   2   /* per-segment L2-served gather for dv                                 */
-#define TRIAD_BWD_DQ_L1        8   /* tiled dq gathering through L1 instead of the TMA/shared-memory ring  */
 #define TRIAD_BWD_SMALL_BLOCKS 16   /* dv: 64 KB query blocks instead of 64 MB (test aid: multi-block path) */
-#define TRIAD_BWD_NO_PREFETCH  4   /* tiled dq without the prefetch.global.L1 look-ahead (A/B timing)      */
 #define TRIAD_BWD_PACK_ROWS   32   /* dq sweeps only the rows whose row_scale is non-zero (masked text tokens
                                       get an exact zero gradient without being gathered for)                */
 #define TRIAD_BWD_UNIFORM_SCALE 128  /* the caller guarantees row_scale has no zeros (no attention mask): the dv sort then
                                       does not read it per row to decide which rows to list                            */
 #define TRIAD_BWD_TEST_TRIP_WATCHDOG 256 /* test aid: raise the watchdog flag before the kernels run: dq must come back NaN */
-#define TRIAD_BWD_DQ_STAGED    64   /* dq: the round-1 kernel (winners/weights staged through shared memory) — cross-check */
 size_t triad_maxmean_bwd_workspace_bytes(int Bq, int Bv, int Nq, int Nv, int D, int dtype);
 int triad_maxmean_bwd(const void* q, const void* v, const void* idx, const float* g,
                       const float* clip, const float* row_scale, const float* temperature,

@@ -80,6 +80,10 @@ def test_argument_validation_without_gpu(lib):
     b = lib.triad_maxmean_bwd
     assert b(one, one, null, one, one, one, one, 2, 2, 4, 8, 64, 1, one, one, 0, one, one, 256, 0, null) == E["arg"]
     assert b(one, one, one, one, one, one, one, 2, 2, 4, 8, 63, 1, one, one, 0, one, one, 256, 0, null) == E["shape"]
+    # a flag bit the library does not define is rejected, not ignored (these reach the workspace check otherwise)
+    assert b(one, one, one, one, one, one, one, 2, 2, 4, 8, 64, 1, one, one, 0, one, one, 256, 32, null) == E["ws"]
+    for bad in (4, 8, 64, 512, 32 | 64):
+        assert b(one, one, one, one, one, one, one, 2, 2, 4, 8, 64, 1, one, one, 0, one, one, 256, bad, null) == E["arg"], bad
     assert lib.triad_topk(one, 10, 11, one, one, one, 1 << 20, null) == E["shape"]
     assert lib.triad_diag_ranks(null, 4, one, null) == E["arg"]
     assert lib.triad_similarity_matrix(one, one, one, 0, 1, 1, 8, one, null) == E["shape"]

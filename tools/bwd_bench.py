@@ -70,8 +70,7 @@ def main():
         return ops.maxmean_bwd(q, v, idx, g, clip, scale, T, need_dq=dq, need_dv=dv, need_dT=False, flags=flags)
 
     outs = {}
-    for name, dq_, dv_, fl in (("dq tiled", True, False, pack_b), ("dq unpacked", True, False, 0), ("dq tiled L1", True, False, _lib.BWD_DQ_L1),
-                               ("dq tiled L1 nopf", True, False, _lib.BWD_DQ_L1 | _lib.BWD_NO_PREFETCH),
+    for name, dq_, dv_, fl in (("dq tiled", True, False, pack_b), ("dq unpacked", True, False, 0),
                                ("dq generic", True, False, _lib.BWD_GENERIC_DQ),
                                ("dv default", False, True, 0), ("dv generic", False, True, _lib.BWD_GENERIC_DV)):
         t = timeit(lambda: bwd(dq_, dv_, fl), iters)

@@ -21,6 +21,5 @@ timeout 200 python tools/timeline.py cfg2 6 > $OUT/timeline_cfg2.txt 2>&1
 timeout 200 python tools/timeline.py cfg3 6 > $OUT/timeline_cfg3.txt 2>&1
 timeout 200 python tools/timeline.py cfg2 4 full > $OUT/timeline_cfg2_full_loss.txt 2>&1
 timeout 200 python tools/step_trace.py 100 > $OUT/step_trace.txt 2>&1
-timeout 300 python tools/dq_ab.py 0 1 2 > $OUT/dq_ab.txt 2>&1
 timeout 200 python tools/power_probe.py > $OUT/power_probe.txt 2>&1
 ls -la $OUT

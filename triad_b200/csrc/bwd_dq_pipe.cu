@@ -3,30 +3,28 @@
 //
 //   dq[r, :] = T * row_scale[r] * sum_j g[i(r), j] * v[j, idx[j][r], :]
 //
-// Same tiling as dq3::dq_smem_kernel (bwd_dq_tile.cu): a CTA owns 512 token rows x one 64-element
-// slice of D, keeps the 512 x 64 fp32 accumulators in registers for the whole sweep over the
-// images, and gathers from a TMA ring of V slices (Nv x 128 B per image) in shared memory.  ncu on
-// that kernel (profiles/r01b_cfg2_ncu_summary.txt): issue slots 65 % busy, shared-memory pipe 60 %,
-// FMA 40 %, ALU 45 % — nothing saturated: with 4 warps per scheduler and a dependent chain per image
-// (barrier wait -> staged offsets -> gathered rows -> FMAs) the warps sit in latencies.  This
-// kernel removes the chain instead of adding warps (there are no registers for more):
+// A CTA owns 512 token rows x one 64-element slice of D, keeps the 512 x 64 fp32 accumulators in
+// registers for the whole sweep over the images, and gathers from a TMA ring of V slices (Nv x 128 B
+// per image) in shared memory.  Staging each image's winners and weights through shared memory (the
+// round-1 kernel, DESIGN.md K3a) left every warp waiting on a dependent chain per image (barrier wait
+// -> staged offsets -> gathered rows -> FMAs) with nothing saturated, and there are no registers for
+// more warps.  This kernel removes the chain instead:
 //
 //   * ROWS ARE ADDRESSED IN THE PADDED INDEX SPACE of the argmax buffer (x = i*nq_pad + a, nq_pad a
 //     multiple of 16), so the 8 rows of an 8-lane group always belong to ONE query: their weight
-//     g[i, j] is one register per image (was 8 + 8 staged through shared memory), and their 8 winners
-//     are 8 consecutive bytes of idx[j] — one 8-byte load per image, prefetched two images ahead
-//     straight into registers.  No shared-memory staging, no staging registers, no __syncthreads.
+//     g[i, j] is one register per image, and their 8 winners are 8 consecutive bytes of idx[j] — one
+//     8-byte load per image, prefetched two images ahead straight into registers.  No shared-memory
+//     staging, no staging registers, no __syncthreads.
 //   * the byte -> shared-memory address conversion is one IDP.4A per row (dot product of the packed
 //     winners with a one-hot 0x80 selector, added to the lane's base): no unpacking, no table.
-//   * the gather is SOFTWARE PIPELINED by half an image: the LDS.128s of rows 4..7 of image j are
-//     in flight while rows 0..3 are accumulated, and rows 0..3 of image j+1 (whose barrier is
-//     tested in between) while rows 4..7 are — a warp never waits for its own loads.
-//   * the ring is refilled WITHOUT tying the warps together.  In dq3 warp 0 refilled the slot image j-1 used
-//     while at image j, so it blocked on the slowest warp's release every image and all warps ran within
-//     one image of each other.  Here either a dedicated producer warpgroup streams the slices
-//     (setmaxnreg: 24 registers for it, 112 for the consumers) or warp 0 refills the slot image j-kLag
-//     used (kLag = 2: its wait blocks only if some warp is more than two images behind).
-//   * the pipeline watchdog no longer votes: a timed-out wait marks the launch (abort flag) and the
+//   * the gather is SOFTWARE PIPELINED by a quarter image: rows 2k..2k+1 of image j are accumulated
+//     while rows 2k+2..2k+3 are in flight, and the first pair of image j+1 (whose barrier is tested in
+//     between) is requested before the last pair of image j is consumed — a warp never waits for its
+//     own loads.
+//   * a dedicated producer warpgroup refills the 7-deep ring (setmaxnreg: 24 registers for it, 112 for
+//     the consumers), so no consumer warp blocks on the slowest warp's release of a slot and the warps
+//     drift freely.
+//   * the pipeline watchdog does not vote: a timed-out wait marks the launch (abort flag) and the
 //     kernel finishes with NaNs in dq, so a pipeline bug is LOUD downstream instead of silent.
 //
 // Masked text queries: the launcher passes a list of the 8-row groups that hold at least one
@@ -40,13 +38,12 @@ using namespace ptx;
 
 constexpr int kGroupsPerTile = 64;                  // 8-row groups per CTA = 512 padded rows
 constexpr int kConsumerWarps = 16;
-constexpr int kThreadsWG = (kConsumerWarps + 4) * 32;   // producer-warpgroup mode: + 4 warps (one lane of them works)
-constexpr int kThreadsIn = kConsumerWarps * 32;          // in-warp refill mode
+constexpr int kThreads = (kConsumerWarps + 4) * 32;     // + the producer warpgroup (one lane of it works)
 constexpr int kSlice = 64;                          // bf16 elements of D per CTA (one 128-byte line)
 constexpr int kMaxNv = 256;
 constexpr uint32_t kStageBytes = kMaxNv * kSlice * 2;   // 32 KB per image slice
-
-template <int kVS> constexpr uint32_t smem_bytes() { return kVS * kStageBytes + 16 * kVS + 128; }
+constexpr int kVS = 7;                              // ring depth (images)
+constexpr uint32_t kSmemBytes = kVS * kStageBytes + 16 * kVS + 128;
 
 __device__ __forceinline__ uint4 lds128(uint32_t addr) {
     uint4 u;
@@ -77,10 +74,8 @@ __device__ __forceinline__ void fma_row(float2 (&a)[4], float w, const uint4& u)
     ffma2(a[0], w, u.x); ffma2(a[1], w, u.y); ffma2(a[2], w, u.z); ffma2(a[3], w, u.w);
 }
 // shared-memory address of winner byte k (0..3) of `packed`: base + 128 * byte_k
-template <bool kDp4a>
 __device__ __forceinline__ uint32_t row_addr(uint32_t packed, int k, uint32_t base) {
-    if constexpr (kDp4a) return __dp4a(packed, 0x80u << (8 * k), base);
-    return base + (((packed >> (8 * k)) & 0xffu) << 7);
+    return __dp4a(packed, 0x80u << (8 * k), base);
 }
 
 // The guarded wait of ptx.cuh with its slow path INLINED: ptxas cannot allocate registers per role
@@ -110,13 +105,9 @@ struct Params {
     int Bq, Bv, Nq, Nv, D, nq_pad, gq;     // gq = ceil(Nq / 8) groups per query
 };
 
-// kLag == 0: a dedicated producer warpgroup streams the V slices (640 threads; setmaxnreg gives the consumers 112
-//            registers — 512*112 + 128*24 is exactly the 640*96 the CTA is launched with).
-// kLag >= 1: 512 threads, 128 registers; warp 0 refills the ring itself, but the slot it refills at image j is the
-//            one image j-kLag used: its (guarded) wait on that slot's release only blocks when some warp is more
-//            than kLag images behind warp 0, so the warps still drift freely; look-ahead = kVS - kLag images.
-template <int kVS, bool kDp4a, int kLag, int kRowsPerStep>
-__global__ void __launch_bounds__(kLag == 0 ? kThreadsWG : kThreadsIn, 1)
+// 640 threads: 16 consumer warps and the producer warpgroup.  setmaxnreg gives the consumers 112 registers —
+// 512*112 + 128*24 is exactly the 640*96 the CTA is launched with.
+__global__ void __launch_bounds__(kThreads, 1)
 dq_pipe_kernel(const __grid_constant__ CUtensorMap tmap_v, const Params p) {
     const int n_groups = p.glist ? *p.n_groups : p.Bq * p.gq;
     if ((int)blockIdx.y * kGroupsPerTile >= n_groups) return;
@@ -142,8 +133,7 @@ dq_pipe_kernel(const __grid_constant__ CUtensorMap tmap_v, const Params p) {
     __syncthreads();                                   // the only CTA-wide barrier
 
     const uint32_t stage_tx = (uint32_t)p.Nv * (kSlice * 2);
-    if constexpr (kLag == 0) {
-      if (warp >= kConsumerWarps) {
+    if (warp >= kConsumerWarps) {
         // ---- producer warpgroup: hands its registers to the consumers; one lane streams the V slices ----
         asm volatile("setmaxnreg.dec.sync.aligned.u32 24;");
         if (warp == kConsumerWarps && lane == 0) {
@@ -157,16 +147,8 @@ dq_pipe_kernel(const __grid_constant__ CUtensorMap tmap_v, const Params p) {
             }
         }
         return;
-      }
-      asm volatile("setmaxnreg.inc.sync.aligned.u32 112;");
-    } else {
-        if (tid == 0) {                                  // prologue: the whole ring
-            for (int j = 0; j < kVS && j < Bv; ++j) {
-                mbar_expect_tx(bar_full + 8 * j, stage_tx);
-                tma_load_3d<1>(sbase + j * kStageBytes, &tmap_v, bar_full + 8 * j, slice * kSlice, 0, j);
-            }
-        }
     }
+    asm volatile("setmaxnreg.inc.sync.aligned.u32 112;");
 
     // ---- consumer: 8-lane group gi owns 8 consecutive padded rows of one query; lane c owns 8 elements ----
     const int gi = warp * 4 + (lane >> 3), c = lane & 7;
@@ -206,99 +188,47 @@ dq_pipe_kernel(const __grid_constant__ CUtensorMap tmap_v, const Params p) {
     uint32_t fbar = bar_full;                              // full barrier of image j's slot (empty = +8*kVS)
     uint32_t par = 0;                                      // parity of image j's slot
     int slot = 0;
-    // in-warp refill (kLag > 0, warp 0): next image to load, its slot, that slot's full barrier, and the parity of the
-    // release that frees it
-    int jfill = kVS;
-    uint32_t rdst = sbase, rbar = bar_full, rpar = 0;
     auto advance = [&]() {
         cur += kStageBytes; fbar += 8;
         if (++slot == kVS) { slot = 0; cur = lane_base; fbar = bar_full; par ^= 1u; }
     };
-#define TRIAD_DQ_REFILL()                                                                                \
-        if (kLag > 0 && warp == 0 && jfill < Bv) {                                                       \
-            if (jfill - kVS + kLag <= j) { /* the slot of image jfill - kVS: released by all warps? */     \
-                wait_guarded(rbar + 8 * kVS, rpar, p.abort_flag, 12);                                    \
-                if (lane0) {                                                                             \
-                    mbar_expect_tx(rbar, stage_tx);                                                      \
-                    tma_load_3d<1>(rdst, &tmap_v, rbar, slice * kSlice, 0, jfill);                       \
-                }                                                                                        \
-                ++jfill; rdst += kStageBytes; rbar += 8;                                                 \
-                if (rdst == sbase + kVS * kStageBytes) { rdst = sbase; rbar = bar_full; rpar ^= 1u; }    \
-            }                                                                                            \
-        }
 
-    int j = 0;
-    if constexpr (kRowsPerStep == 4) {
-        // ---- half-image pipelining: two 4-row buffers (32 registers) ----
-        uint4 dA[4], dB[4];
+    // Quarter-image pipelining: two 2-row buffers (16 registers; half-image buffers spill at 112 registers).
+    uint4 dX[2], dY[2];
 #pragma unroll
-        for (int r = 0; r < 4; ++r) dA[r] = lds128(row_addr<kDp4a>(W0.x, r, lane_base));
-// One image.  HAS_NEXT: image j+1 exists (its first half is requested in the middle); PREFETCH: image j+2 exists.
+    for (int r = 0; r < 2; ++r) dX[r] = lds128(row_addr(W0.x, r, lane_base));
+// One image.  HAS_NEXT: image j+1 exists (its first pair is requested before the last pair of j is consumed);
+// PREFETCH: image j+2 exists.
 #define TRIAD_DQ_IMAGE(Wc, wc, Wn, HAS_NEXT, PREFETCH)                                                   \
     {                                                                                                    \
-        _Pragma("unroll") for (int r = 0; r < 4; ++r) dB[r] = lds128(row_addr<kDp4a>(Wc.y, r, cur));     \
+        _Pragma("unroll") for (int r = 0; r < 2; ++r) dY[r] = lds128(row_addr(Wc.x, 2 + r, cur));        \
+        _Pragma("unroll") for (int r = 0; r < 2; ++r) fma_row(acc[r], wc, dX[r]);                        \
+        _Pragma("unroll") for (int r = 0; r < 2; ++r) dX[r] = lds128(row_addr(Wc.y, r, cur));            \
+        _Pragma("unroll") for (int r = 0; r < 2; ++r) fma_row(acc[2 + r], wc, dY[r]);                    \
+        _Pragma("unroll") for (int r = 0; r < 2; ++r) dY[r] = lds128(row_addr(Wc.y, 2 + r, cur));        \
         if (PREFETCH) { Wc = ldg64(ibase + x0); ibase += pitch; }                                        \
-        _Pragma("unroll") for (int r = 0; r < 4; ++r) fma_row(acc[r], wc, dA[r]);                        \
+        _Pragma("unroll") for (int r = 0; r < 2; ++r) fma_row(acc[4 + r], wc, dX[r]);                    \
         const uint32_t ebar = fbar + 8 * kVS;                                                            \
-        TRIAD_DQ_REFILL()                                                                                \
         if (HAS_NEXT) {                                                                                  \
             advance();                                                                                   \
             wait_guarded(fbar, par, p.abort_flag, 11);                                                   \
-            _Pragma("unroll") for (int r = 0; r < 4; ++r) dA[r] = lds128(row_addr<kDp4a>(Wn.x, r, cur)); \
+            _Pragma("unroll") for (int r = 0; r < 2; ++r) dX[r] = lds128(row_addr(Wn.x, r, cur));        \
         }                                                                                                \
-        _Pragma("unroll") for (int r = 0; r < 4; ++r) fma_row(acc[4 + r], wc, dB[r]);                    \
+        _Pragma("unroll") for (int r = 0; r < 2; ++r) fma_row(acc[6 + r], wc, dY[r]);                    \
         __syncwarp();                                                                                    \
         if (lane0) mbar_arrive_local(ebar);                                                              \
         if (PREFETCH) { wc = ldg32f(gbase + goff); ++gbase; }                                            \
     }
-        for (; j + 3 <= last; j += 2) {                    // both images of the pair have a successor two ahead
-            TRIAD_DQ_IMAGE(W0, w0, W1, true, true)
-            TRIAD_DQ_IMAGE(W1, w1, W0, true, true)
-        }
-        for (; j <= last; ++j) {                           // the last two or three images
-            if (j & 1) TRIAD_DQ_IMAGE(W1, w1, W0, j < last, j + 2 <= last)
-            else TRIAD_DQ_IMAGE(W0, w0, W1, j < last, j + 2 <= last)
-        }
-#undef TRIAD_DQ_IMAGE
-    } else {
-        // ---- quarter-image pipelining: two 2-row buffers (16 registers): rows 2k..2k+1 are accumulated while rows
-        //      2k+2..2k+3 are in flight; the first pair of image j+1 is requested before the last pair of image j
-        //      is consumed.  16 registers less than the half-image form: no spills at 112 registers. ----
-        uint4 dX[2], dY[2];
-#pragma unroll
-        for (int r = 0; r < 2; ++r) dX[r] = lds128(row_addr<kDp4a>(W0.x, r, lane_base));
-#define TRIAD_DQ_IMAGE(Wc, wc, Wn, HAS_NEXT, PREFETCH)                                                       \
-    {                                                                                                        \
-        _Pragma("unroll") for (int r = 0; r < 2; ++r) dY[r] = lds128(row_addr<kDp4a>(Wc.x, 2 + r, cur));     \
-        _Pragma("unroll") for (int r = 0; r < 2; ++r) fma_row(acc[r], wc, dX[r]);                            \
-        _Pragma("unroll") for (int r = 0; r < 2; ++r) dX[r] = lds128(row_addr<kDp4a>(Wc.y, r, cur));         \
-        _Pragma("unroll") for (int r = 0; r < 2; ++r) fma_row(acc[2 + r], wc, dY[r]);                        \
-        _Pragma("unroll") for (int r = 0; r < 2; ++r) dY[r] = lds128(row_addr<kDp4a>(Wc.y, 2 + r, cur));     \
-        if (PREFETCH) { Wc = ldg64(ibase + x0); ibase += pitch; }                                            \
-        _Pragma("unroll") for (int r = 0; r < 2; ++r) fma_row(acc[4 + r], wc, dX[r]);                        \
-        const uint32_t ebar = fbar + 8 * kVS;                                                                \
-        TRIAD_DQ_REFILL()                                                                                    \
-        if (HAS_NEXT) {                                                                                      \
-            advance();                                                                                       \
-            wait_guarded(fbar, par, p.abort_flag, 11);                                                       \
-            _Pragma("unroll") for (int r = 0; r < 2; ++r) dX[r] = lds128(row_addr<kDp4a>(Wn.x, r, cur));     \
-        }                                                                                                    \
-        _Pragma("unroll") for (int r = 0; r < 2; ++r) fma_row(acc[6 + r], wc, dY[r]);                        \
-        __syncwarp();                                                                                        \
-        if (lane0) mbar_arrive_local(ebar);                                                                  \
-        if (PREFETCH) { wc = ldg32f(gbase + goff); ++gbase; }                                                \
+    int j = 0;
+    for (; j + 3 <= last; j += 2) {                        // both images of the pair have a successor two ahead
+        TRIAD_DQ_IMAGE(W0, w0, W1, true, true)
+        TRIAD_DQ_IMAGE(W1, w1, W0, true, true)
     }
-        for (; j + 3 <= last; j += 2) {
-            TRIAD_DQ_IMAGE(W0, w0, W1, true, true)
-            TRIAD_DQ_IMAGE(W1, w1, W0, true, true)
-        }
-        for (; j <= last; ++j) {
-            if (j & 1) TRIAD_DQ_IMAGE(W1, w1, W0, j < last, j + 2 <= last)
-            else TRIAD_DQ_IMAGE(W0, w0, W1, j < last, j + 2 <= last)
-        }
-#undef TRIAD_DQ_IMAGE
+    for (; j <= last; ++j) {                               // the last two or three images
+        if (j & 1) TRIAD_DQ_IMAGE(W1, w1, W0, j < last, j + 2 <= last)
+        else TRIAD_DQ_IMAGE(W0, w0, W1, j < last, j + 2 <= last)
     }
-#undef TRIAD_DQ_REFILL
+#undef TRIAD_DQ_IMAGE
 
     // ---- epilogue: scale, round to bf16, one 16-byte store per row and lane (128 B per row and group) ----
     const bool poisoned = *(volatile int*)p.abort_flag != 0;   // a timed-out wait anywhere in the grid: make it loud
@@ -325,17 +255,6 @@ dq_pipe_kernel(const __grid_constant__ CUtensorMap tmap_v, const Params p) {
     }
 }
 
-template <int kVS, bool kDp4a, int kLag, int kRowsPerStep>
-static int launch_t(const CUtensorMap& mv, const Params& p, int max_groups, cudaStream_t st) {
-    auto kern = dq_pipe_kernel<kVS, kDp4a, kLag, kRowsPerStep>;
-    constexpr int kThreads = kLag == 0 ? kThreadsWG : kThreadsIn;
-    TRIAD_SET_MAX_SMEM(kern, smem_bytes<kVS>());
-    const dim3 grid((unsigned)(p.D / kSlice), (unsigned)ceil_div(max_groups, kGroupsPerTile));
-    kern<<<grid, kThreads, smem_bytes<kVS>(), st>>>(mv, p);
-    TRIAD_LAUNCH_CHECK("dq_pipe_kernel");
-    return TRIAD_OK;
-}
-
 }  // namespace dq4
 
 bool dq_pipe_supported(int Nv, int D, int dtype) {
@@ -345,7 +264,7 @@ bool dq_pipe_supported(int Nv, int D, int dtype) {
 // glist / n_groups_dev: active 8-row groups (device), or null for "all rows of all queries".
 int launch_dq_pipe(const void* v, const void* idx, const float* g, const float* row_scale, const float* Tp,
                    int Bq, int Bv, int Nq, int Nv, int D, void* dq, int* abort_flag,
-                   const int* glist, const int* n_groups_dev, int variant, cudaStream_t st) {
+                   const int* glist, const int* n_groups_dev, cudaStream_t st) {
     using namespace dq4;
     CUtensorMap mv;
     cuuint64_t dims[3] = {(cuuint64_t)D, (cuuint64_t)Nv, (cuuint64_t)Bv};
@@ -361,14 +280,11 @@ int launch_dq_pipe(const void* v, const void* idx, const float* g, const float* 
     if (glist) TRIAD_CUDA_CHECK(cudaMemsetAsync(dq, 0, (size_t)Bq * Nq * D * 2, st));   // rows of inactive groups: zero gradient
     if ((long long)Bq * p.nq_pad > 0x7fffffffLL || (long long)Bq * Bv > 0x7fffffffLL)
         return fail_msg(TRIAD_ERR_BAD_SHAPE, "dq_pipe: Bq*nq_pad and Bq*Bv must fit in 31 bits");
-    switch (variant) {
-        // measured at cfg 2 (B=256, 250x256, D=512; round-1 staged kernel 1.045 ms): see DESIGN.md K3a
-        case 1: return launch_t<7, true, 2, 4>(mv, p, max_groups, st);     // in-warp refill two images behind, 128 registers
-        case 2: return launch_t<7, true, 0, 4>(mv, p, max_groups, st);     // producer warpgroup, half-image pipelining (spills at 112)
-        case 3: return launch_t<6, true, 0, 2>(mv, p, max_groups, st);     // 6-deep ring
-        case 4: return launch_t<7, true, 2, 2>(mv, p, max_groups, st);     // in-warp refill, quarter-image pipelining
-        default: return launch_t<7, true, 0, 2>(mv, p, max_groups, st);    // producer warpgroup, quarter-image pipelining
-    }
+    TRIAD_SET_MAX_SMEM(dq_pipe_kernel, kSmemBytes);
+    const dim3 grid((unsigned)(D / kSlice), (unsigned)ceil_div(max_groups, kGroupsPerTile));
+    dq_pipe_kernel<<<grid, kThreads, kSmemBytes, st>>>(mv, p);
+    TRIAD_LAUNCH_CHECK("dq_pipe_kernel");
+    return TRIAD_OK;
 }
 
 }  // namespace triad

@@ -1,4 +1,5 @@
-// dQ of the max-mean backward, bf16, tiled for on-chip reuse (SURVEY.md §8 a5):
+// dQ of the max-mean backward, bf16, Nv > 256 (uint16 winners), tiled for on-chip reuse (SURVEY.md §8 a5;
+// Nv <= 256 is served by the shared-memory pipeline of bwd_dq_pipe.cu):
 //
 //   dq[r, :] = T * row_scale[r] * sum_j g[i(r), j] * v[j, idx[j][r], :]
 //
@@ -23,7 +24,6 @@
 // weights g[i(r), j] of 8 images at a time are staged through shared memory (thread t stages
 // tile row t), double buffered, one __syncthreads per 8 images.
 #include "common.cuh"
-#include "ptx.cuh"
 
 namespace triad {
 namespace dq2 {
@@ -54,27 +54,14 @@ __device__ __forceinline__ void fma8(float (&a)[8], float w, const uint4& u) {
 
 constexpr int kStages = 3;      // staging ring: group G computes, G+1 is the prefetch target, G+2 is being loaded
 
-// Two fp32 FMAs per issue slot (Blackwell FFMA2): acc (lo,hi) += w * (bf16 pair of one 32-bit word).
-// These kernels are issue-bound, so halving the FMA instruction count is a direct win.
-__device__ __forceinline__ void ffma2(float2& acc, float w, uint32_t pair) {
-    float2 wv = make_float2(w, w);
-    float2 vv = make_float2(__uint_as_float(pair << 16), __uint_as_float(pair & 0xffff0000u));
-    unsigned long long a = *reinterpret_cast<unsigned long long*>(&acc);
-    const unsigned long long b = *reinterpret_cast<unsigned long long*>(&wv);
-    const unsigned long long c = *reinterpret_cast<unsigned long long*>(&vv);
-    asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(a) : "l"(b), "l"(c));
-    acc = *reinterpret_cast<float2*>(&a);
-}
-__device__ __forceinline__ void fma8p(float2 (&a)[4], float w, const uint4& u) {
-    ffma2(a[0], w, u.x); ffma2(a[1], w, u.y); ffma2(a[2], w, u.z); ffma2(a[3], w, u.w);
-}
+using IdxT = uint16_t;           // winners: this kernel serves Nv > 256
+constexpr size_t kSmemBytes = (size_t)kStages * kJG * kRows * (sizeof(IdxT) + sizeof(float));
 
-template <typename IdxT> constexpr size_t smem_bytes() { return (size_t)kStages * kJG * kRows * (sizeof(IdxT) + sizeof(float)); }
+// kPF = prefetch distance in images: before the rows of image j are gathered, every lane asks for
+// the line ONE of its group's rows will need at image j+kPF (prefetch.global.L1), so that by the
+// time the LDG.128s are issued they hit L1 instead of waiting ~700 cycles on L2.
+constexpr int kPF = 2;
 
-// kPF = prefetch distance in images (0 = none): before the rows of image j are gathered, every
-// lane asks for the line ONE of its group's rows will need at image j+kPF (prefetch.global.L1),
-// so that by the time the LDG.128s are issued they hit L1 instead of waiting ~700 cycles on L2.
-template <typename IdxT, int kPF>
 __global__ void __launch_bounds__(kThreads, 1)
 dq_tile_kernel(const __nv_bfloat16* __restrict__ v, const IdxT* __restrict__ idx, const float* __restrict__ g,
                const float* __restrict__ row_scale, const float* __restrict__ Tptr,
@@ -134,11 +121,9 @@ dq_tile_kernel(const __nv_bfloat16* __restrict__ v, const IdxT* __restrict__ idx
     stage(0, 0);
     if (kJG < Bv) stage(kJG, 1);
     __syncthreads();
-    if (kPF > 0) {                                            // warm-up: the first kPF images
 #pragma unroll
-        for (int jp = 0; jp < kPF; ++jp)
-            if (jp < Bv) prefetch_l1(vslice + (size_t)jp * img_bytes + (uint32_t)idx_s[0][jp][rb + c] * row_bytes);
-    }
+    for (int jp = 0; jp < kPF; ++jp)                          // warm-up: the first kPF images
+        if (jp < Bv) prefetch_l1(vslice + (size_t)jp * img_bytes + (uint32_t)idx_s[0][jp][rb + c] * row_bytes);
     int st = 0;
     for (int j0 = 0; j0 < Bv; j0 += kJG) {
         const int jn = min(kJG, Bv - j0);
@@ -147,24 +132,15 @@ dq_tile_kernel(const __nv_bfloat16* __restrict__ v, const IdxT* __restrict__ idx
 #pragma unroll
         for (int jj = 0; jj < kJG; ++jj) {
             if (jj < jn) {
-                if (kPF > 0) {
-                    const int jp = jj + kPF;                               // compile-time after unrolling
-                    if (j0 + jp < Bv) {
-                        const uint32_t pp = (jp < kJG) ? idx_s[st][jp % kJG][rb + c] : idx_s[st1][jp % kJG][rb + c];
-                        prefetch_l1(vslice + (size_t)(j0 + jp) * img_bytes + pp * row_bytes);
-                    }
+                const int jp = jj + kPF;                                   // compile-time after unrolling
+                if (j0 + jp < Bv) {
+                    const uint32_t pp = (jp < kJG) ? idx_s[st][jp % kJG][rb + c] : idx_s[st1][jp % kJG][rb + c];
+                    prefetch_l1(vslice + (size_t)(j0 + jp) * img_bytes + pp * row_bytes);
                 }
                 const char* vj = vbase + (size_t)(j0 + jj) * img_bytes;
-                uint32_t p[8];
-                if (sizeof(IdxT) == 1) {
-                    const uint2 pk = *reinterpret_cast<const uint2*>(&idx_s[st][jj][rb]);
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) { p[k] = (pk.x >> (8 * k)) & 0xffu; p[4 + k] = (pk.y >> (8 * k)) & 0xffu; }
-                } else {
-                    const uint4 pk = *reinterpret_cast<const uint4*>(&idx_s[st][jj][rb]);
-                    p[0] = pk.x & 0xffffu; p[1] = pk.x >> 16; p[2] = pk.y & 0xffffu; p[3] = pk.y >> 16;
-                    p[4] = pk.z & 0xffffu; p[5] = pk.z >> 16; p[6] = pk.w & 0xffffu; p[7] = pk.w >> 16;
-                }
+                const uint4 pk = *reinterpret_cast<const uint4*>(&idx_s[st][jj][rb]);
+                const uint32_t p[8] = {pk.x & 0xffffu, pk.x >> 16, pk.y & 0xffffu, pk.y >> 16,
+                                       pk.z & 0xffffu, pk.z >> 16, pk.w & 0xffffu, pk.w >> 16};
                 const float4 wa = *reinterpret_cast<const float4*>(&w_s[st][jj][rb]);
                 const float4 wb = *reinterpret_cast<const float4*>(&w_s[st][jj][rb + 4]);
                 const float w[8] = {wa.x, wa.y, wa.z, wa.w, wb.x, wb.y, wb.z, wb.w};
@@ -202,234 +178,16 @@ dq_tile_kernel(const __nv_bfloat16* __restrict__ v, const IdxT* __restrict__ idx
 
 bool dq_tile_supported(int D, int dtype) { return dtype == TRIAD_DTYPE_BF16 && D % dq2::kSlice == 0; }
 
-// ---------------------------------------------------------------------------------------------
-// Same tiling, but the gather is served from SHARED memory: one elected thread streams the
-// 64-element slice of every image (Nv x 128 bytes, <= 32 KB) through a 5-deep TMA ring, so the
-// consumers never wait on L2 — an LDS.128 per lane reads one 128-byte row per 8-lane group
-// (conflict-free), with a fixed ~30-cycle latency that 16 warps hide.  Used when Nv <= 256.
-// ---------------------------------------------------------------------------------------------
-namespace dq3 {
-using namespace ptx;
-
-__device__ __forceinline__ uint4 lds128(uint32_t addr) {
-    uint4 u;
-    asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(u.x), "=r"(u.y), "=r"(u.z), "=r"(u.w) : "r"(addr));
-    return u;
-}
-
-constexpr int kRows = 512;
-constexpr int kThreads = 512;
-constexpr int kSlice = 64;
-constexpr int kJG = 8;           // images per idx/weight staging group (one __syncthreads per group)
-constexpr int kStages = 2;       // idx/weight staging: double buffered
-constexpr int kVS = 5;           // V-slice ring depth (4 images of look-ahead)
-constexpr int kMaxNv = 256;
-constexpr uint32_t kVStageBytes = kMaxNv * kSlice * 2;                                   // 32 KB
-constexpr uint32_t kWBytes = kStages * kJG * kRows * 4;      // weights g[i(r), j]
-constexpr uint32_t kIdxBytes = kStages * kJG * kRows * 4;    // winners as byte offsets p*128 into the V stage
-constexpr uint32_t kSmemBytes = kVS * kVStageBytes + kWBytes + kIdxBytes + 2 * 8 * kVS + 128;  // + alignment slack
-
-__global__ void __launch_bounds__(kThreads, 1)
-dq_smem_kernel(const __grid_constant__ CUtensorMap tmap_v, const uint8_t* __restrict__ idx, const float* __restrict__ g,
-               const float* __restrict__ row_scale, const float* __restrict__ Tptr,
-               int M, int Bv, int Nq, int Nv, int D, int nq_pad, int g_vec, __nv_bfloat16* __restrict__ dq, int* abort_flag,
-               const int* __restrict__ pack_off, const int* __restrict__ rowmap) {
-    // packed rows (pack.cu): the tile rows are the KEPT rows; rows with zero weight were zeroed by the launcher
-    const int M_eff = pack_off ? pack_off[M / Nq] : M;
-    if ((int)blockIdx.y * kRows >= M_eff) return;
-    extern __shared__ unsigned char dq3_smem[];
-    const uint32_t s0 = smem_u32(dq3_smem);
-    const uint32_t sbase = (s0 + 127u) & ~127u;
-    unsigned char* base = dq3_smem + (sbase - s0);
-    unsigned char* v_s = base;
-    float (*w_s)[kJG][kRows] = reinterpret_cast<float (*)[kJG][kRows]>(base + kVS * kVStageBytes);
-    uint32_t (*off_s)[kJG][kRows] = reinterpret_cast<uint32_t (*)[kJG][kRows]>(base + kVS * kVStageBytes + kWBytes);
-    const uint32_t bar_full = sbase + kVS * kVStageBytes + kWBytes + kIdxBytes;
-    const uint32_t bar_empty = bar_full + 8 * kVS;
-
-    const int t = threadIdx.x;
-    const int slice = blockIdx.x;
-    const int row0 = blockIdx.y * kRows;
-
-    // ---- staging role: thread t = tile row t.  A warp stages exactly the 32 rows it later gathers
-    //      for, so the staging buffers are warp-private: __syncwarp is all the ordering they need and
-    //      the warps of a CTA only meet at the V ring's mbarriers (they may drift up to kVS-1 images).
-    const bool rs_valid = row0 + t < M_eff;
-    const int rs = rs_valid ? (rowmap ? rowmap[row0 + t] : row0 + t) : 0;      // original row
-    const int qi = rs_valid ? rs / Nq : 0;
-    const size_t pitch = (size_t)(M / Nq) * nq_pad;
-    const uint8_t* idx_row = idx + (size_t)qi * nq_pad + (rs_valid ? rs - qi * Nq : 0);
-    const float* g_row = g + (size_t)qi * Bv;
-
-    // ---- compute role -------------------------------------------------------------------------
-    const int warp = t >> 5, lane = t & 31, grp = lane >> 3, c = lane & 7;
-    const int rb = warp * 32 + grp * 8;
-
-    float2 acc[8][4];                             // 8 rows x 4 packed (lo,hi) fp32 pairs
-#pragma unroll
-    for (int k = 0; k < 8; ++k)
-#pragma unroll
-        for (int e = 0; e < 4; ++e) acc[k][e] = make_float2(0.f, 0.f);
-    const uint32_t vs_base = sbase + (uint32_t)c * 16u;
-
-    // staging is split in two so the global loads of group G+1 are in flight while group G computes
-    uint8_t pi[kJG];
-    float pw[kJG];
-    auto stage_load = [&](int j0) {
-        if (rs_valid && g_vec && j0 + kJG <= Bv) {
-            const float4 a = __ldg(reinterpret_cast<const float4*>(g_row + j0));
-            const float4 b = __ldg(reinterpret_cast<const float4*>(g_row + j0 + 4));
-            pw[0] = a.x; pw[1] = a.y; pw[2] = a.z; pw[3] = a.w; pw[4] = b.x; pw[5] = b.y; pw[6] = b.z; pw[7] = b.w;
-#pragma unroll
-            for (int jj = 0; jj < kJG; ++jj) pi[jj] = __ldcs(idx_row + (size_t)(j0 + jj) * pitch);
-        } else {
-#pragma unroll
-            for (int jj = 0; jj < kJG; ++jj) {
-                const int j = j0 + jj;
-                const bool ok = rs_valid && j < Bv;
-                pi[jj] = ok ? __ldcs(idx_row + (size_t)j * pitch) : (uint8_t)0;
-                pw[jj] = ok ? __ldg(g_row + j) : 0.f;
-            }
-        }
-    };
-    auto stage_store = [&](int st) {
-#pragma unroll
-        for (int jj = 0; jj < kJG; ++jj) { off_s[st][jj][t] = (uint32_t)pi[jj] * (kSlice * 2); w_s[st][jj][t] = pw[jj]; }
-    };
-
-    const uint32_t stage_tx = (uint32_t)Nv * (kSlice * 2);
-    if (t == 0) {
-        prefetch_tmap(&tmap_v);
-        for (int s = 0; s < kVS; ++s) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, kThreads / 32); }
-        fence_barrier_init();
-    }
-    stage_load(0);
-    stage_store(0);
-    __syncthreads();                 // barrier init visible to all warps (the only CTA-wide barrier)
-    if (t == 0) {
-        for (int jn = 0; jn < kVS - 1 && jn < Bv; ++jn) {
-            mbar_expect_tx(bar_full + 8 * jn, stage_tx);
-            tma_load_3d<1>(sbase + jn * kVStageBytes, &tmap_v, bar_full + 8 * jn, slice * kSlice, 0, jn);
-        }
-    }
-
-    int st = 0, vslot = 0;
-    uint32_t vphase = 0;
-    bool ok = true;
-    for (int j0 = 0; j0 < Bv; j0 += kJG) {
-        const int jn = min(kJG, Bv - j0);
-        const bool more = j0 + kJG < Bv;
-        if (more) stage_load(j0 + kJG);
-#pragma unroll
-        for (int jj = 0; jj < kJG; ++jj) {
-            if (jj < jn) {
-                const int j = j0 + jj;
-                if (ok) ok = mbar_wait(bar_full + 8 * vslot, vphase, abort_flag, 11);
-                ok = __all_sync(0xffffffffu, ok);
-                if (ok) {
-                    const uint4 oa = *reinterpret_cast<const uint4*>(&off_s[st][jj][rb]);
-                    const uint4 ob = *reinterpret_cast<const uint4*>(&off_s[st][jj][rb + 4]);
-                    const uint32_t off[8] = {oa.x, oa.y, oa.z, oa.w, ob.x, ob.y, ob.z, ob.w};
-                    const float4 wa = *reinterpret_cast<const float4*>(&w_s[st][jj][rb]);
-                    const float4 wb = *reinterpret_cast<const float4*>(&w_s[st][jj][rb + 4]);
-                    const float w[8] = {wa.x, wa.y, wa.z, wa.w, wb.x, wb.y, wb.z, wb.w};
-                    // shared-space addresses (32-bit) computed from a base hoisted out of the loop: a generic-pointer
-                    // dereference made ptxas rebuild the shared window base (S2R/LEA/LOP chain) for every image
-                    const uint32_t vs = vs_base + (uint32_t)vslot * kVStageBytes;
-                    uint4 d[8];
-#pragma unroll
-                    for (int k = 0; k < 8; ++k) d[k] = lds128(vs + off[k]);
-#pragma unroll
-                    for (int k = 0; k < 8; ++k) dq2::fma8p(acc[k], w[k], d[k]);
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive_local(bar_empty + 8 * vslot);
-                    if (t == 0) {
-                        const int jnext = j + kVS - 1;                       // refills the slot image j-1 used
-                        if (jnext < Bv) {
-                            const int s2 = (vslot == 0) ? kVS - 1 : vslot - 1;
-                            bool pok = true;
-                            if (j >= 1) pok = mbar_wait(bar_empty + 8 * s2, (uint32_t)(((j - 1) / kVS) & 1), abort_flag, 12);
-                            if (pok) {
-                                mbar_expect_tx(bar_full + 8 * s2, stage_tx);
-                                tma_load_3d<1>(sbase + s2 * kVStageBytes, &tmap_v, bar_full + 8 * s2, slice * kSlice, 0, jnext);
-                            }
-                        }
-                    }
-                }
-                if (++vslot == kVS) { vslot = 0; vphase ^= 1; }
-            }
-        }
-        if (more) stage_store(st ^ 1);
-        __syncwarp();
-        st ^= 1;
-    }
-
-    const float Tval = *Tptr;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        const int rk = row0 + rb + k;
-        if (rk < M_eff) {
-            const int r = rowmap ? rowmap[rk] : rk;
-            const float s = Tval * row_scale[r];
-            uint4 o;
-            uint32_t* w32 = reinterpret_cast<uint32_t*>(&o);
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                const float2 f = acc[k][e];
-                __nv_bfloat162 h = __floats2bfloat162_rn(f.x * s, f.y * s);
-                w32[e] = *reinterpret_cast<uint32_t*>(&h);
-            }
-            *reinterpret_cast<uint4*>(dq + (size_t)r * D + slice * kSlice + c * 8) = o;
-        }
-    }
-}
-
-}  // namespace dq3
-
-bool dq_smem_supported(int Nv, int D, int dtype) { return dtype == TRIAD_DTYPE_BF16 && D % dq3::kSlice == 0 && Nv <= dq3::kMaxNv; }
-
-int launch_dq_smem(const void* v, const void* idx, const float* g, const float* row_scale, const float* Tp,
-                   int M, int Bv, int Nq, int Nv, int D, void* dq, int* abort_flag, const int* pack_maps, cudaStream_t st) {
-    using namespace dq3;
-    TRIAD_SET_MAX_SMEM(dq_smem_kernel, kSmemBytes);
-    CUtensorMap mv;
-    cuuint64_t dims[3] = {(cuuint64_t)D, (cuuint64_t)Nv, (cuuint64_t)Bv};
-    cuuint64_t strides[2] = {(cuuint64_t)D * 2, (cuuint64_t)Nv * D * 2};
-    cuuint32_t box[3] = {(cuuint32_t)kSlice, (cuuint32_t)Nv, 1};
-    int rc = encode_tmap_bf16(&mv, v, 3, dims, strides, box, false);
-    if (rc) return rc;
-    const dim3 grid((unsigned)(D / kSlice), (unsigned)ceil_div(M, kRows));
-    const int g_vec = (Bv % 4 == 0) && (((uintptr_t)g & 15) == 0);
-    if (pack_maps) TRIAD_CUDA_CHECK(cudaMemsetAsync(dq, 0, (size_t)M * D * 2, st));      // rows that were dropped: zero gradient
-    dq_smem_kernel<<<grid, kThreads, kSmemBytes, st>>>(mv, (const uint8_t*)idx, g, row_scale, Tp, M, Bv, Nq, Nv, D,
-                                                      nq_padded(Nq), g_vec, (__nv_bfloat16*)dq, abort_flag,
-                                                      pack_maps, pack_maps ? pack_maps + M / Nq + 1 : nullptr);
-    TRIAD_LAUNCH_CHECK("dq_smem_kernel");
-    return TRIAD_OK;
-}
-
-template <typename IdxT, int kPF>
-static int launch_dq_t(const void* v, const void* idx, const float* g, const float* row_scale, const float* Tp,
-                       int M, int Bv, int Nq, int Nv, int D, void* dq, cudaStream_t st) {
+int launch_dq_tile(const void* v, const void* idx, const float* g, const float* row_scale, const float* Tp,
+                   int M, int Bv, int Nq, int Nv, int D, void* dq, cudaStream_t st) {
     using namespace dq2;
-    auto kern = dq_tile_kernel<IdxT, kPF>;
-    TRIAD_SET_MAX_SMEM(kern, smem_bytes<IdxT>());
+    TRIAD_SET_MAX_SMEM(dq_tile_kernel, kSmemBytes);
     const dim3 grid((unsigned)(D / kSlice), (unsigned)ceil_div(M, kRows));
     const int g_vec = (Bv % 4 == 0) && (((uintptr_t)g & 15) == 0);
-    kern<<<grid, kThreads, smem_bytes<IdxT>(), st>>>((const __nv_bfloat16*)v, (const IdxT*)idx, g, row_scale, Tp, M, Bv, Nq, Nv, D,
-                                                     nq_padded(Nq), g_vec, (__nv_bfloat16*)dq);
+    dq_tile_kernel<<<grid, kThreads, kSmemBytes, st>>>((const __nv_bfloat16*)v, (const uint16_t*)idx, g, row_scale, Tp,
+                                                      M, Bv, Nq, Nv, D, nq_padded(Nq), g_vec, (__nv_bfloat16*)dq);
     TRIAD_LAUNCH_CHECK("dq_tile_kernel");
     return TRIAD_OK;
-}
-
-int launch_dq_tile(const void* v, const void* idx, int idx_bytes, const float* g, const float* row_scale,
-                   const float* Tp, int M, int Bv, int Nq, int Nv, int D, int prefetch, void* dq, cudaStream_t st) {
-    if (idx_bytes == 1) {
-        return prefetch ? launch_dq_t<uint8_t, 2>(v, idx, g, row_scale, Tp, M, Bv, Nq, Nv, D, dq, st)
-                        : launch_dq_t<uint8_t, 0>(v, idx, g, row_scale, Tp, M, Bv, Nq, Nv, D, dq, st);
-    }
-    return prefetch ? launch_dq_t<uint16_t, 2>(v, idx, g, row_scale, Tp, M, Bv, Nq, Nv, D, dq, st)
-                    : launch_dq_t<uint16_t, 0>(v, idx, g, row_scale, Tp, M, Bv, Nq, Nv, D, dq, st);
 }
 
 }  // namespace triad

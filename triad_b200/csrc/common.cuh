@@ -109,18 +109,15 @@ int launch_finalize_clip_packed(const float* part, const int* pack_off, int Bq, 
 // - (group of the query's first packed row); a query of <= Nq kept rows spans at most (Nq+30)/32 + 1 groups
 static inline int packed_pieces(int Nq) { return (Nq + 30) / 32 + 1; }
 bool tc_supported(int Nv, int D);
-// tiled dQ of the backward, bf16 only — bwd_dq_tile.cu (TMA/shared-memory gather, and the L1-resident variant)
-bool dq_smem_supported(int Nv, int D, int dtype);
-int launch_dq_smem(const void* v, const void* idx, const float* g, const float* row_scale, const float* Tp,
-                   int M, int Bv, int Nq, int Nv, int D, void* dq, int* abort_flag, const int* pack_maps, cudaStream_t st);
-// software-pipelined variant (bwd_dq_pipe.cu): rows addressed in the padded index space, register prefetch of winners
+// tiled dQ of the backward, bf16 only.  Nv <= 256 (uint8 winners): the software-pipelined shared-memory gather
+// (bwd_dq_pipe.cu); Nv > 256 (uint16 winners): the L1-resident gather (bwd_dq_tile.cu)
 bool dq_pipe_supported(int Nv, int D, int dtype);
 int launch_dq_pipe(const void* v, const void* idx, const float* g, const float* row_scale, const float* Tp,
                    int Bq, int Bv, int Nq, int Nv, int D, void* dq, int* abort_flag,
-                   const int* glist, const int* n_groups_dev, int variant, cudaStream_t st);
+                   const int* glist, const int* n_groups_dev, cudaStream_t st);
 bool dq_tile_supported(int D, int dtype);
-int launch_dq_tile(const void* v, const void* idx, int idx_bytes, const float* g, const float* row_scale,
-                   const float* Tp, int M, int Bv, int Nq, int Nv, int D, int prefetch, void* dq, cudaStream_t st);
+int launch_dq_tile(const void* v, const void* idx, const float* g, const float* row_scale, const float* Tp,
+                   int M, int Bv, int Nq, int Nv, int D, void* dq, cudaStream_t st);
 
 // ---- device helpers -----------------------------------------------------------------------
 #if defined(__CUDACC__)

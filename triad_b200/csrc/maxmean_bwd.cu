@@ -18,9 +18,11 @@
 //                                            -> dv_gather_grouped_kernel (packed rows, FFMA2, 64 registers);
 //   bf16, Nv  > 1024:                        dv_count / dv_offsets / dv_scatter_sort (global sort) -> dv_gather_bf16_kernel;
 //   fp32 inputs or TRIAD_BWD_GENERIC_DV:     the global sort -> dv_gather_kernel (generic, the cross-check).
-// dq lives in bwd_dq_tile.cu (TMA / shared-memory tiles) with dq_gather_kernel here as the generic path.
+// dq code paths:
+//   bf16, Nv <= 256, D % 64 == 0:            dq_pipe_kernel (bwd_dq_pipe.cu, shared-memory gather);
+//   bf16, Nv  > 256, D % 64 == 0:            dq_tile_kernel (bwd_dq_tile.cu, L1-resident gather);
+//   otherwise or TRIAD_BWD_GENERIC_DQ:       dq_gather_kernel here (generic, the cross-check: same summation order).
 #include "common.cuh"
-#include <stdlib.h>
 
 #include <type_traits>
 
@@ -833,13 +835,6 @@ static DvPlan dv_plan(int Bq, int Bv, int Nq, int Nv, int D, int elt_bytes, bool
     return pl;
 }
 
-// experiment knob: TRIAD_DQ_VARIANT selects the ring depth / address form of dq_pipe_kernel (0 = shipped default)
-static int dq_pipe_variant() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("TRIAD_DQ_VARIANT"); v = e ? atoi(e) : 0; }
-    return v;
-}
-
 template <typename T, typename IdxT>
 static int bwd_typed(const void* q, const void* v, const void* idx, const float* g,
                      const float* clip, const float* row_scale, const float* Tp,
@@ -850,37 +845,27 @@ static int bwd_typed(const void* q, const void* v, const void* idx, const float*
     constexpr int E = Vec16<T>::kElems;
     const int kch = ceil_div(D / E, 32);
     if (dq && (kch < 1 || kch > 4)) return fail_msg(TRIAD_ERR_UNSUPPORTED, "maxmean_bwd: D too large (max 1024 bf16 / 512 fp32)");
-    if (dq && sizeof(T) == 2 && sizeof(IdxT) == 1 && dq_pipe_supported(Nv, D, TRIAD_DTYPE_BF16) &&
-        !(bwd_flags & (TRIAD_BWD_GENERIC_DQ | TRIAD_BWD_DQ_L1 | TRIAD_BWD_DQ_STAGED))) {
-        // the software-pipelined shared-memory gather (bwd_dq_pipe.cu); TRIAD_BWD_PACK_ROWS (masked text queries): only
-        // the 8-row groups that hold a row with a non-zero weight are swept
-        const int* glist = nullptr;
-        const int* n_groups = nullptr;
-        if (bwd_flags & TRIAD_BWD_PACK_ROWS) {
-            void* maps = (char*)ws + pack_maps_offset;
-            const int rcm = launch_pack_groups(row_scale, Bq, Nq, maps, st);
-            if (rcm) return rcm;
-            n_groups = (const int*)maps + Bq;
-            glist = (const int*)maps + Bq + 1;
+    if (dq && sizeof(T) == 2 && !(bwd_flags & TRIAD_BWD_GENERIC_DQ) &&
+        (sizeof(IdxT) == 1 ? dq_pipe_supported(Nv, D, TRIAD_DTYPE_BF16) : dq_tile_supported(D, TRIAD_DTYPE_BF16))) {
+        if constexpr (sizeof(IdxT) == 1) {
+            // the software-pipelined shared-memory gather (bwd_dq_pipe.cu); TRIAD_BWD_PACK_ROWS (masked text queries):
+            // only the 8-row groups that hold a row with a non-zero weight are swept
+            const int* glist = nullptr;
+            const int* n_groups = nullptr;
+            if (bwd_flags & TRIAD_BWD_PACK_ROWS) {
+                void* maps = (char*)ws + pack_maps_offset;
+                const int rcm = launch_pack_groups(row_scale, Bq, Nq, maps, st);
+                if (rcm) return rcm;
+                n_groups = (const int*)maps + Bq;
+                glist = (const int*)maps + Bq + 1;
+            }
+            const int rc = launch_dq_pipe(v, idx, g, row_scale, Tp, Bq, Bv, Nq, Nv, D, dq, (int*)ws, glist, n_groups, st);
+            if (rc) return rc;
+        } else {
+            // the L1-resident gather (bwd_dq_tile.cu) sweeps every row, TRIAD_BWD_PACK_ROWS or not
+            const int rc = launch_dq_tile(v, idx, g, row_scale, Tp, M, Bv, Nq, Nv, D, dq, st);
+            if (rc) return rc;
         }
-        const int rc = launch_dq_pipe(v, idx, g, row_scale, Tp, Bq, Bv, Nq, Nv, D, dq, (int*)ws, glist, n_groups, dq_pipe_variant(), st);
-        if (rc) return rc;
-    } else if (dq && sizeof(T) == 2 && sizeof(IdxT) == 1 && dq_smem_supported(Nv, D, TRIAD_DTYPE_BF16) &&
-        !(bwd_flags & (TRIAD_BWD_GENERIC_DQ | TRIAD_BWD_DQ_L1))) {
-        // TRIAD_BWD_PACK_ROWS (masked text queries): only the rows with a non-zero weight are swept
-        const int* pack_maps = nullptr;
-        if (bwd_flags & TRIAD_BWD_PACK_ROWS) {
-            void* maps = (char*)ws + pack_maps_offset;
-            const int rcm = launch_pack_map(row_scale, Bq, Nq, maps, st);
-            if (rcm) return rcm;
-            pack_maps = (const int*)maps;
-        }
-        const int rc = launch_dq_smem(v, idx, g, row_scale, Tp, M, Bv, Nq, Nv, D, dq, (int*)ws, pack_maps, st);
-        if (rc) return rc;
-    } else if (dq && sizeof(T) == 2 && dq_tile_supported(D, TRIAD_DTYPE_BF16) && !(bwd_flags & TRIAD_BWD_GENERIC_DQ)) {
-        const int rc = launch_dq_tile(v, idx, (int)sizeof(IdxT), g, row_scale, Tp, M, Bv, Nq, Nv, D,
-                                      (bwd_flags & TRIAD_BWD_NO_PREFETCH) ? 0 : 1, dq, st);
-        if (rc) return rc;
     } else if (dq) {
         const int grid = ceil_div(M, kDqRows);
 #define TRIAD_DQ(K) dq_gather_kernel<T, IdxT, K><<<grid, 256, 0, st>>>( \
@@ -1011,6 +996,10 @@ static int bwd_typed(const void* q, const void* v, const void* idx, const float*
 
 using namespace triad;
 
+// every TRIAD_BWD_* bit; any other bit is an error rather than silently ignored
+static constexpr int kBwdFlags = TRIAD_BWD_GENERIC_DQ | TRIAD_BWD_GENERIC_DV | TRIAD_BWD_SMALL_BLOCKS | TRIAD_BWD_PACK_ROWS |
+                                 TRIAD_BWD_UNIFORM_SCALE | TRIAD_BWD_TEST_TRIP_WATCHDOG;
+
 extern "C" size_t triad_maxmean_bwd_workspace_bytes(int Bq, int Bv, int Nq, int Nv, int D, int dtype) {
     if (Bq <= 0 || Bv <= 0 || Nq <= 0 || Nv <= 0 || D <= 0) return 0;
     // the caller may ask for dv in `dtype` (fp32 scratch when several query blocks) or as an fp32 partial
@@ -1034,6 +1023,7 @@ extern "C" int triad_maxmean_bwd(const void* q, const void* v, const void* idx, 
     if (Bq <= 0 || Bv <= 0 || Nq <= 0 || Nv <= 0 || D <= 0 || D % 8 != 0 || Nv > 65535)
         return fail_msg(TRIAD_ERR_BAD_SHAPE, "maxmean_bwd: bad shape");
     if (dtype != TRIAD_DTYPE_F32 && dtype != TRIAD_DTYPE_BF16) return fail_msg(TRIAD_ERR_BAD_ARG, "maxmean_bwd: dtype");
+    if (flags & ~kBwdFlags) return fail_msg(TRIAD_ERR_BAD_ARG, "maxmean_bwd: unknown flag bit");
     if (((uintptr_t)q | (uintptr_t)v | (uintptr_t)dq | (uintptr_t)dv | (uintptr_t)ws) & 15) return fail_msg(TRIAD_ERR_ALIGNMENT, "maxmean_bwd: 16-byte alignment");
     if (!ws || ws_bytes < ((dv || (flags & TRIAD_BWD_PACK_ROWS)) ? triad_maxmean_bwd_workspace_bytes(Bq, Bv, Nq, Nv, D, dtype) : kCtrlBytes))
         return fail_msg(TRIAD_ERR_WORKSPACE, "maxmean_bwd: workspace too small");
