@@ -230,13 +230,16 @@ size_t triad_retrieve_workspace_bytes(int Nq, int n_img, int Nv, int D, int dtyp
 int triad_retrieve_scores(const void* q, int Nq, const void* gallery, int n_img, int Nv, int D,
                           int dtype, const float* temperature, int divide_by_T, int direction,
                           float* scores, void* ws, size_t ws_bytes, void* stream);
-/* top-k of scores (descending, ties -> lower id first, like a stable argsort of -scores):
- * out_scores fp32 [k], out_ids int32 [k].  ws: triad_topk_workspace_bytes(n). */
+/* top-k of scores (descending, ties -> lower id first, like a stable argsort of -scores;
+ * -0.0 and +0.0 are equal scores): out_scores fp32 [k] = scores[out_ids], bit for bit,
+ * out_ids int32 [k].  NaN scores have no defined place.  ws: triad_topk_workspace_bytes(n). */
 size_t triad_topk_workspace_bytes(int n, int k);
 int triad_topk(const float* scores, int n, int k, float* out_scores, int32_t* out_ids,
                void* ws, size_t ws_bytes, void* stream);
 /* rank of the diagonal in each row of an N x N similarity matrix (retrieval.py:125-133):
- * ranks int32 [N] = #{j : sim[i,j] > sim[i,i]} + #{j < i : sim[i,j] == sim[i,i]}. */
+ * ranks int32 [N] = #{j : sim[i,j] > sim[i,i]} + #{j < i : sim[i,j] == sim[i,i]}, the position
+ * of i in a stable argsort of -sim[i].  NaN sorts last: a NaN entry ranks below every number, and
+ * a NaN diagonal gets #{j : sim[i,j] is not NaN} + #{j < i : sim[i,j] is NaN}. */
 int triad_diag_ranks(const float* sim, int N, int32_t* ranks, void* stream);
 
 /* ---- per-pair normalised similarity (viz / forward()) -------------------------------- */

@@ -6,9 +6,11 @@
 namespace triad {
 
 // order-preserving key: larger score -> larger key; among equal scores the LOWER id is larger,
-// i.e. a descending sort of keys is a stable descending argsort of the scores.
+// i.e. a descending sort of keys is a stable descending argsort of the scores.  -0.0 and +0.0 are
+// equal scores, so both get the key of +0.0 (f32_key alone would rank every +0.0 above every -0.0).
 __device__ __forceinline__ unsigned long long make_key(float s, uint32_t id) {
-    return ((unsigned long long)f32_key(s) << 32) | (unsigned long long)(0xffffffffu - id);
+    const uint32_t k = s == 0.f ? f32_key(0.f) : f32_key(s);
+    return ((unsigned long long)k << 32) | (unsigned long long)(0xffffffffu - id);
 }
 
 constexpr int kTopkChunk = 4096;
@@ -42,24 +44,28 @@ topk_chunk_kernel(const unsigned long long* __restrict__ in, int n, int keep, un
     for (int t = threadIdx.x; t < keep; t += 1024) out[(size_t)blockIdx.x * keep + t] = s[t];
 }
 
-__global__ void topk_emit_kernel(const unsigned long long* __restrict__ keys, int k, float* __restrict__ out_scores,
-                                 int32_t* __restrict__ out_ids) {
+// the score is read back from the input rather than decoded from the key: a -0.0 keeps its sign bit
+__global__ void topk_emit_kernel(const unsigned long long* __restrict__ keys, const float* __restrict__ scores, int k,
+                                 float* __restrict__ out_scores, int32_t* __restrict__ out_ids) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= k) return;
-    const unsigned long long key = keys[i];
-    out_scores[i] = f32_unkey((uint32_t)(key >> 32));
-    out_ids[i] = (int32_t)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
+    const uint32_t id = 0xffffffffu - (uint32_t)(keys[i] & 0xffffffffull);
+    out_scores[i] = scores[id];
+    out_ids[i] = (int32_t)id;
 }
 
 // ranks[i] = #{j: sim[i,j] > sim[i,i]} + #{j < i: sim[i,j] == sim[i,i]}  (position of i in a
-// stable descending argsort of row i, retrieval.py:129-131)
+// stable descending argsort of row i, retrieval.py:129-131).  NaN sorts last there, so a NaN
+// diagonal ranks after every non-NaN entry and after the NaNs to its left: a forward whose
+// watchdog fired (NaN scores) must not count as a hit.
 __global__ void diag_ranks_kernel(const float* __restrict__ sim, int N, int32_t* __restrict__ ranks) {
     const int i = blockIdx.x;
     const float d = sim[(size_t)i * N + i];
+    const bool d_nan = d != d;
     int cnt = 0;
     for (int j = threadIdx.x; j < N; j += blockDim.x) {
         const float x = sim[(size_t)i * N + j];
-        cnt += (x > d) || (x == d && j < i);
+        cnt += d_nan ? (x == x || j < i) : (x > d || (x == d && j < i));
     }
     __shared__ int red[32];
 #pragma unroll
@@ -129,7 +135,7 @@ extern "C" int triad_topk(const float* scores, int n, int k, float* out_scores, 
         cur = nchunk * keep;
         if (nchunk == 1) break;
     }
-    topk_emit_kernel<<<ceil_div(k, 256), 256, 0, st>>>(a, k, out_scores, out_ids);
+    topk_emit_kernel<<<ceil_div(k, 256), 256, 0, st>>>(a, scores, k, out_scores, out_ids);
     TRIAD_LAUNCH_CHECK("topk_emit_kernel");
     return TRIAD_OK;
 }
