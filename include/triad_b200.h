@@ -142,7 +142,8 @@ int triad_contrastive_head(const float* clip, int B, const float* temperature,
  *   dT        = sum_ij g[i,j]*clip[i,j] / T
  * g fp32 [Bq,Bv] is dLoss/dclip.  dq is written in `dtype` ([Bq,Nq,D]); dv is written as
  * fp32 [Bv,Nv,D] when dv_f32 != 0 (partial to be reduce-scattered across ranks) else in
- * `dtype`; dT fp32 [1].  Any of dq / dv / dT may be NULL to skip it.  `flags` is an OR of the
+ * `dtype`; dT fp32 [1].  Any of dq / dv / dT may be NULL to skip it.  dv needs Nv <= 3072: beyond,
+ * the call fails with TRIAD_ERR_UNSUPPORTED before queueing any work.  `flags` is an OR of the
  * TRIAD_BWD_* bits below; any other bit (4, 8 and 64 are retired) fails with TRIAD_ERR_BAD_ARG. */
 #define TRIAD_BWD_DEFAULT      0
 #define TRIAD_BWD_GENERIC_DQ   1   /* L2-served gather kernel for dq (always used for fp32 / D % 64 != 0) */

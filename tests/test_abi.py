@@ -60,7 +60,7 @@ def test_status_strings_and_version(lib):
 
 def test_argument_validation_without_gpu(lib):
     """Every entry point rejects bad arguments before any CUDA call (so this runs on CPU)."""
-    E = {"arg": -1, "shape": -2, "align": -3, "ws": -4}
+    E = {"arg": -1, "shape": -2, "align": -3, "ws": -4, "unsupported": -7}
     null = None
     one = ctypes.c_void_p(16)     # a non-null, 16-byte aligned fake pointer: never dereferenced on these paths
     odd = ctypes.c_void_p(24)
@@ -84,6 +84,10 @@ def test_argument_validation_without_gpu(lib):
     assert b(one, one, one, one, one, one, one, 2, 2, 4, 8, 64, 1, one, one, 0, one, one, 256, 32, null) == E["ws"]
     for bad in (4, 8, 64, 512, 32 | 64):
         assert b(one, one, one, one, one, one, one, 2, 2, 4, 8, 64, 1, one, one, 0, one, one, 256, bad, null) == E["arg"], bad
+    # dv beyond the largest patch count the dv sorts handle: rejected before any work is queued
+    for dtype in (0, 1):
+        ws = lib.triad_maxmean_bwd_workspace_bytes(2, 2, 4, 3073, 64, dtype)
+        assert b(one, one, one, one, one, one, one, 2, 2, 4, 3073, 64, dtype, one, one, 0, one, one, ws, 0, null) == E["unsupported"], dtype
     assert lib.triad_topk(one, 10, 11, one, one, one, 1 << 20, null) == E["shape"]
     assert lib.triad_diag_ranks(null, 4, one, null) == E["arg"]
     assert lib.triad_similarity_matrix(one, one, one, 0, 1, 1, 8, one, null) == E["shape"]

@@ -297,11 +297,12 @@ def test_full_size_properties_cfg2():
 
 
 @pytest.mark.parametrize("masked", [False, True])
-@pytest.mark.parametrize("Nv", [200, 600])
+@pytest.mark.parametrize("Nv", [200, 600, 2048, 3072])
 def test_backward_variants_agree(Nv, masked):
     """Every backward kernel variant (dq: shared-memory pipeline for Nv <= 256, L1-resident tile for Nv > 256,
     generic L2 gather; single-block and multi-block dv, fp32-partial and bf16 dv) against the oracle's closed
-    form and against each other."""
+    form and against each other.  Nv = 2048 and 3072 take the global dv sort with the packed bf16 gather; 3072 is
+    the largest Nv the dv pass handles."""
     from triad_b200 import _lib, ops
     B, Nq, D = 20, 77, 256
     q, v, mask = O.make_inputs(B, Nq, Nv, D, torch.bfloat16, seed=41, masked=masked, min_len=3)

@@ -1,7 +1,9 @@
 #!/usr/bin/env python
 """Times the pieces of one step at a BASELINE shape and cross-checks the backward variants.
 
-    python tools/bwd_bench.py [cfg2|cfg3|...] [iters]
+    python tools/bwd_bench.py [cfg2|cfg3|...] [iters] [Bq] [Bv] [Nv]
+
+Bq defaults to the config's batch, Bv to Bq, and Nv (patches per image) to the config's.
 
 Prints CUDA-event times of: forward, InfoNCE, dq (tiled / generic), dv (default / generic), and
 the max relative difference between the variants' outputs (they must agree to bf16 rounding).
@@ -40,6 +42,8 @@ def main():
     iters = int(sys.argv[2]) if len(sys.argv) > 2 else 5
     Bq = int(sys.argv[3]) if len(sys.argv) > 3 else cfg["B"]       # local query rows (a rank's shard)
     Bv = int(sys.argv[4]) if len(sys.argv) > 4 else Bq             # images (the all-gathered batch)
+    if len(sys.argv) > 5:
+        cfg["Nv"] = int(sys.argv[5])
     dev = torch.device("cuda", 0)
     (q, _, mask), = bench.make_device_inputs(cfg, Bq, 1234, dev, 1)
     (_, v, _), = bench.make_device_inputs(cfg, Bv, 4321, dev, 1)

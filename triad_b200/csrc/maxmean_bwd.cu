@@ -13,10 +13,12 @@
 // (row, weight) pairs, and a warp then accumulates that list in registers — no atomics, fixed
 // summation order, bit-reproducible.
 //
-// dv code paths (all produce the same lists in the same order, hence bit-identical results; the tests compare them):
-//   bf16, Nv <= 1024 (the training shapes): dv_group_sort_kernel (shared-memory sort per image x 8192-row group)
+// dv code paths, for Nv <= kDvMaxNv (all produce the same lists in the same order, hence bit-identical results; the
+// tests compare them):
+//   bf16, Nv <= kGroupMaxNv (the training shapes): dv_group_sort_kernel (shared-memory sort per image x 8192-row group)
 //                                            -> dv_gather_grouped_kernel (packed rows, FFMA2, 64 registers);
-//   bf16, Nv  > 1024:                        dv_count / dv_offsets / dv_scatter_sort (global sort) -> dv_gather_bf16_kernel;
+//   bf16, Nv  > kGroupMaxNv:                 dv_count / dv_offsets / dv_scatter_sort (global sort)
+//                                            -> dv_gather_grouped_kernel over the image's one list;
 //   fp32 inputs or TRIAD_BWD_GENERIC_DV:     the global sort -> dv_gather_kernel (generic, the cross-check).
 // dq code paths:
 //   bf16, Nv <= 256, D % 64 == 0:            dq_pipe_kernel (bwd_dq_pipe.cu, shared-memory gather);
@@ -197,6 +199,10 @@ dq_gather_kernel(const T* __restrict__ v, const IdxT* __restrict__ idx, const fl
 // ---------------------------------------------------------------------------------------
 constexpr int kSortGroups = 8;
 constexpr int kSortWarps = 4;
+// The largest patch count the dv pass handles: the global sort keeps kSortWarps counters of Nv words in (at most the
+// default 48 KB of) dynamic shared memory.
+constexpr int kDvMaxNv = 3072;
+static_assert((size_t)kSortWarps * kDvMaxNv * 4 <= 48 * 1024, "dv global sort: per-warp counters exceed 48 KB");
 
 struct __align__(8) DvEntry { uint32_t row; float w; };
 
@@ -318,14 +324,19 @@ dv_scatter_sort_kernel(const IdxT* __restrict__ idx, const float* __restrict__ g
 //   and writes the group's list as ONE contiguous, fully coalesced run into the group's own region of the
 //   entry buffer.  The per-(image, group) segment table replaces the global offsets; the gather walks a
 //   patch's list group by group.  Order inside a patch is still "rows ascending", so dv is bit-identical to
-//   the ungrouped path.
+//   the global sort's.
 // ---------------------------------------------------------------------------------------
 constexpr int kGroupRows = 8192;
 constexpr int kGroupWarps = 8;
 constexpr int kGroupPerLane = kGroupRows / (kGroupWarps * 32);      // 32 rows per lane
+constexpr int kGroupMaxQueries = kGroupRows / 16 + 2;               // queries one group touches (nq_pad >= 16)
+// Above kGroupMaxNv patches bf16 takes the global sort: the dv pass measured slower with the grouped sort at Nv = 2048
+// and 3072, where its tables leave room for one CTA per SM (DESIGN.md, K3b).
 constexpr int kGroupMaxNv = 1024;
 
-static size_t group_sort_smem(int Nv) { return (size_t)kGroupRows * 2 + (size_t)(kGroupWarps + 2) * Nv * 4 + 16; }
+static constexpr size_t group_sort_smem(int Nv) { return (size_t)kGroupRows * 2 + (size_t)(kGroupWarps + 2) * Nv * 4 + 16; }
+static_assert(group_sort_smem(kGroupMaxNv) + kGroupMaxQueries * sizeof(float) <= 227 * 1024,
+              "dv grouped sort: shared memory exceeds 227 KB per block");
 
 // Rows are walked in the PADDED index space of the argmax buffer (x = i*nq_pad + a): one image's winners are then
 // one contiguous byte string, fetched 16 bytes (16 rows) per lane and load instead of a byte at a time, and the
@@ -357,9 +368,9 @@ dv_group_sort_kernel(const IdxT* __restrict__ idx, const float* __restrict__ g, 
     const IdxT* base = idx + (size_t)j * img_pitch;
 
     for (int k = tid; k < kGroupWarps * Nv; k += blockDim.x) hist[k] = 0;
-    // g[i][j] of the queries this group touches (<= kGroupRows/16 + 2 of them): step 4 looks its weights up here
+    // g[i][j] of the queries this group touches (<= kGroupMaxQueries of them): step 4 looks its weights up here
     // instead of issuing one scattered global load per entry (32 sectors per warp instruction)
-    __shared__ float gq_s[kGroupRows / 16 + 2];
+    __shared__ float gq_s[kGroupMaxQueries];
     const uint32_t i_first = fast_div((uint32_t)x_group, div_pad);
     {
         const int x_last = min(x_group + kGroupRows, Mpad) - 1;
@@ -535,9 +546,9 @@ dv_gather_kernel(const T* __restrict__ q, const DvEntry* __restrict__ entries, c
     }
 }
 
-// bf16 specialisation of the gather above, shaped for the two things ncu shows it short of — bytes in
-// flight (the generic kernel's 102 registers allow 16 warps/SM; L2 throughput sits at 44 %) and issue
-// slots (54 % busy, mostly bf16 unpacking and scalar FMAs):
+// dv step 2, bf16: the gather above over the GROUPED lists of dv_group_sort_kernel, shaped for the two things ncu
+// shows the generic kernel short of — bytes in flight (its 102 registers allow 16 warps/SM; L2 throughput sits at
+// 44 %) and issue slots (54 % busy, mostly bf16 unpacking and scalar FMAs):
 //   * rows stay PACKED (one uint4 per lane and row) until they are consumed, so kU rows in flight cost
 //     4*kU registers instead of 8*kU and kMinBlocks CTAs fit per SM;
 //   * FFMA2 (two fp32 FMAs per issue slot) on the (lo,hi) halves of every 32-bit word;
@@ -554,22 +565,24 @@ __device__ __forceinline__ void ffma2_pair(float2& acc, float w, uint32_t pair) 
     acc = *reinterpret_cast<float2*>(&a);
 }
 
+// The (row, weight) list of (image, patch) is the concatenation, over the groups c, of
+// entries[jl][c][segc[jl][c][p] .. segc[jl][c][p+1]), with Mrows entry slots per image: n_groups * kGroupRows for
+// the lists of dv_group_sort_kernel; the global sort's list is one group of the block's rows.  The first batch of
+// the next group is requested before the current group's rows are consumed.
 // kW = 16-byte chunks per lane and row: kW = 1 -> a warp covers 512 bytes of the row (D = 512: two warps per
 // segment, each walking the entry list); kW = 2 -> one warp covers 1 KB with two loads per row, halving the
 // list/shuffle overhead per byte.
 template <typename OutT, int kU, int kW, int kMinBlocks>
 __global__ void __launch_bounds__(256, kMinBlocks)
-dv_gather_bf16_kernel(const __nv_bfloat16* __restrict__ q, const DvEntry* __restrict__ entries,
-                      const uint32_t* __restrict__ seg, const float* __restrict__ Tptr, int j0, int nj, int Nv, int D,
-                      int wps, size_t Mrows, int accumulate, OutT* __restrict__ dv) {
+dv_gather_grouped_kernel(const __nv_bfloat16* __restrict__ q, const DvEntry* __restrict__ entries,
+                         const uint32_t* __restrict__ segc, const float* __restrict__ Tptr, int j0, int nj, int n_groups,
+                         size_t Mrows, int Nv, int D, int wps, int accumulate, OutT* __restrict__ dv) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const long long wid = (long long)blockIdx.x * 8 + warp;
     const long long sid = wid / wps;
-    const int ch0 = (int)(wid - sid * wps) * 32 * kW + lane;    // this lane's first 16-byte chunk; the others follow at +32
+    const int ch0 = (int)(wid - sid * wps) * 32 * kW + lane;
     if (sid >= (long long)nj * Nv) return;
     const int jl = (int)(sid / Nv), p = (int)(sid % Nv);
-    const uint32_t e0 = seg[(size_t)jl * (Nv + 1) + p], e1 = seg[(size_t)jl * (Nv + 1) + p + 1];
-    const DvEntry* list = entries + (size_t)jl * Mrows;
     // 32-bit byte offsets from the (uniform) block base: a query block is <= 64 MB (dv_plan), so the
     // address is one register per row in flight instead of two
     const char* qbase = reinterpret_cast<const char*>(q);
@@ -585,87 +598,8 @@ dv_gather_bf16_kernel(const __nv_bfloat16* __restrict__ q, const DvEntry* __rest
 #pragma unroll
         for (int c = 0; c < 4; ++c) acc[k][c] = make_float2(0.f, 0.f);
 
-    DvEntry next; next.row = 0; next.w = 0.f;
-    if (e0 + lane < e1) next = list[e0 + lane];
-    for (uint32_t base = e0; base < e1; base += 32) {
-        const uint32_t my_row = next.row;
-        const float my_w = next.w;
-        next.row = 0; next.w = 0.f;
-        if (base + 32 + lane < e1) next = list[base + 32 + lane];
-        const int n = min(32u, e1 - base);
-        for (int l = 0; l < n; l += kU) {
-            uint4 d[kU][kW];
-            float w[kU];
-#pragma unroll
-            for (int u = 0; u < kU; ++u) {
-                // slots past n re-read the segment's last entry with weight 0: no branch in the batch
-                const int src = min(l + u, n - 1);
-                const uint32_t row = __shfl_sync(0xffffffffu, my_row, src);
-                const float ww = __shfl_sync(0xffffffffu, my_w, src);
-                w[u] = (l + u < n) ? ww : 0.f;
-#pragma unroll
-                for (int k = 0; k < kW; ++k)
-                    d[u][k] = __ldg(reinterpret_cast<const uint4*>(qbase + (row * row_bytes + lane_off[k])));
-            }
-#pragma unroll
-            for (int u = 0; u < kU; ++u)
-#pragma unroll
-                for (int k = 0; k < kW; ++k) {
-                    ffma2_pair(acc[k][0], w[u], d[u][k].x); ffma2_pair(acc[k][1], w[u], d[u][k].y);
-                    ffma2_pair(acc[k][2], w[u], d[u][k].z); ffma2_pair(acc[k][3], w[u], d[u][k].w);
-                }
-        }
-    }
-    const float Tval = *Tptr;
-#pragma unroll
-    for (int k = 0; k < kW; ++k) {
-        if (!act[k]) continue;
-        float o[8];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) { o[2 * c] = acc[k][c].x * Tval; o[2 * c + 1] = acc[k][c].y * Tval; }
-        OutT* dst = dv + ((size_t)(j0 + jl) * Nv + p) * D + (ch0 + 32 * k) * 8;
-        if (accumulate) {                       // later query blocks add to the fp32 partial of the earlier ones
-            float prev[8];
-            LoadAs<OutT, 8>::get(dst, prev);
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-                o[2 * c] = __fmaf_rn(acc[k][c].x, Tval, prev[2 * c]);
-                o[2 * c + 1] = __fmaf_rn(acc[k][c].y, Tval, prev[2 * c + 1]);
-            }
-        }
-        StoreAs<OutT, 8>::put(dst, o);
-    }
-}
-
-// The same gather over the GROUPED lists of dv_group_sort_kernel: the (row, weight) list of (image, patch) is
-// the concatenation, over the groups c, of entries[jl][c][segc[jl][c][p] .. segc[jl][c][p+1]).  The first
-// batch of the next group is requested before the current group's rows are consumed.
-template <typename OutT, int kU, int kW, int kMinBlocks>
-__global__ void __launch_bounds__(256, kMinBlocks)
-dv_gather_grouped_kernel(const __nv_bfloat16* __restrict__ q, const DvEntry* __restrict__ entries,
-                         const uint32_t* __restrict__ segc, const float* __restrict__ Tptr, int j0, int nj, int n_groups,
-                         int Nv, int D, int wps, int accumulate, OutT* __restrict__ dv) {
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const long long wid = (long long)blockIdx.x * 8 + warp;
-    const long long sid = wid / wps;
-    const int ch0 = (int)(wid - sid * wps) * 32 * kW + lane;
-    if (sid >= (long long)nj * Nv) return;
-    const int jl = (int)(sid / Nv), p = (int)(sid % Nv);
-    const char* qbase = reinterpret_cast<const char*>(q);
-    const uint32_t row_bytes = (uint32_t)D * 2u;
-    bool act[kW];
-    uint32_t lane_off[kW];
-#pragma unroll
-    for (int k = 0; k < kW; ++k) { act[k] = (ch0 + 32 * k) * 8 < D; lane_off[k] = act[k] ? (uint32_t)(ch0 + 32 * k) * 16u : 0u; }
-
-    float2 acc[kW][4];
-#pragma unroll
-    for (int k = 0; k < kW; ++k)
-#pragma unroll
-        for (int c = 0; c < 4; ++c) acc[k][c] = make_float2(0.f, 0.f);
-
     const uint32_t* sg = segc + (size_t)jl * n_groups * (Nv + 1) + p;
-    const DvEntry* lists = entries + (size_t)jl * n_groups * kGroupRows;
+    const DvEntry* lists = entries + (size_t)jl * Mrows;
     // segment bounds of 32 groups at a time live in lane registers (lane c <-> group c0 + c): no dependent
     // table load per group
     uint32_t myE0 = 0, myE1 = 0;
@@ -887,10 +821,14 @@ static int bwd_typed(const void* q, const void* v, const void* idx, const float*
         uint32_t* cnt = (uint32_t*)((char*)ws + pl.off_cnt);
         uint32_t* start = (uint32_t*)((char*)ws + pl.off_start);
         uint32_t* seg = (uint32_t*)((char*)ws + pl.off_seg);
+        uint32_t* segc = (uint32_t*)((char*)ws + pl.off_segc);
         DvEntry* entries = (DvEntry*)((char*)ws + pl.off_entries);
         float* scratch = (float*)((char*)ws + pl.off_scratch);
-        const size_t smem = (size_t)kSortWarps * Nv * 4;
-        if (smem > 48 * 1024) return fail_msg(TRIAD_ERR_UNSUPPORTED, "maxmean_bwd: Nv too large for the dv sort");
+        const size_t smem = (size_t)kSortWarps * Nv * 4;                          // <= 48 KB: Nv <= kDvMaxNv
+        // bf16: the packed FFMA2 gather, over the grouped sort's lists up to kGroupMaxNv patches and over the global
+        // sort's list beyond; fp32 and TRIAD_BWD_GENERIC_DV: the global sort and the generic gather
+        const bool packed = sizeof(T) == 2 && !(bwd_flags & TRIAD_BWD_GENERIC_DV);
+        const bool grouped = packed && Nv <= kGroupMaxNv;
         const size_t img_pitch = (size_t)Bq * nq_pad;
         const int wps = ceil_div(D / E, 32);                                       // warps per segment
         for (int j0 = 0; j0 < Bv; j0 += pl.jb) {
@@ -906,72 +844,58 @@ static int bwd_typed(const void* q, const void* v, const void* idx, const float*
                 const float* rs_b = row_scale + (size_t)q0 * Nq;
                 const float* g_b = g + (size_t)q0 * Bv;
                 const T* q_b = (const T*)q + (size_t)q0 * Nq * D;
-                if constexpr (sizeof(T) == 2) {
-                    if (Nv <= kGroupMaxNv && !(bwd_flags & TRIAD_BWD_GENERIC_DV)) {
-                        // grouped path: shared-memory sort per (image, row group) + gather over the grouped lists
-                        const int Mpad = nq * nq_pad;
-                        const int n_groups = ceil_div(Mpad, kGroupRows);
-                        uint32_t* segc = (uint32_t*)((char*)ws + pl.off_segc);
-                        auto skern = dv_group_sort_kernel<IdxT>;
-                        TRIAD_SET_MAX_SMEM(skern, group_sort_smem(kGroupMaxNv));
-                        skern<<<nj * n_groups, kGroupWarps * 32, group_sort_smem(Nv), st>>>(
-                            idx_b, g_b, rs_b, (bwd_flags & TRIAD_BWD_UNIFORM_SCALE) ? 0 : 1, img_pitch, j0, n_groups, Mpad, Bv, Nq, Nv,
-                            nq_pad, make_fastdiv((uint32_t)nq_pad), segc, entries);
-                        TRIAD_LAUNCH_CHECK("dv_group_sort_kernel");
-                        const __nv_bfloat16* qb16 = (const __nv_bfloat16*)q_b;
-                        const bool wide_rows = D > 256;
+                // the sort leaves n_groups lists per image (Mrows entry slots per image) and their segment table in segs
+                const uint32_t* segs = seg;
+                int n_groups = 1;
+                size_t Mrows = Mb;
+                if (grouped) {                                     // shared-memory sort per (image, row group)
+                    const int Mpad = nq * nq_pad;
+                    n_groups = ceil_div(Mpad, kGroupRows);
+                    Mrows = (size_t)n_groups * kGroupRows;
+                    segs = segc;
+                    auto skern = dv_group_sort_kernel<IdxT>;
+                    TRIAD_SET_MAX_SMEM(skern, group_sort_smem(kGroupMaxNv));
+                    skern<<<nj * n_groups, kGroupWarps * 32, group_sort_smem(Nv), st>>>(
+                        idx_b, g_b, rs_b, (bwd_flags & TRIAD_BWD_UNIFORM_SCALE) ? 0 : 1, img_pitch, j0, n_groups, Mpad, Bv, Nq, Nv,
+                        nq_pad, make_fastdiv((uint32_t)nq_pad), segc, entries);
+                    TRIAD_LAUNCH_CHECK("dv_group_sort_kernel");
+                } else {                                           // global sort: one list per image
+                    dv_count_kernel<IdxT><<<sort_grid, kSortWarps * 32, smem, st>>>(idx_b, rs_b, img_pitch, j0, nj, nq, Nq, Nv, nq_pad, cnt);
+                    TRIAD_LAUNCH_CHECK("dv_count_kernel");
+                    dv_offsets_kernel<<<nj, 1024, 0, st>>>(cnt, nj, Nv, start, seg);
+                    TRIAD_LAUNCH_CHECK("dv_offsets_kernel");
+                    dv_scatter_sort_kernel<IdxT><<<sort_grid, kSortWarps * 32, smem, st>>>(
+                        idx_b, g_b, rs_b, start, img_pitch, j0, nj, nq, Bv, Nq, Nv, nq_pad, Mb, entries);
+                    TRIAD_LAUNCH_CHECK("dv_scatter_sort_kernel");
+                }
+                // the gather
+                if (packed) {
+                    const __nv_bfloat16* qb16 = (const __nv_bfloat16*)q_b;
+                    // rows of more than 512 bytes: one warp per segment, two 16-byte loads per lane and row
+                    // (measured at cfg 2: 1.46 -> 1.36 ms for the whole dv pass); otherwise one load per lane
+                    const bool wide_rows = D > 256;
 #define TRIAD_DVG_K(OUT, DST, J0, U, W, MB) do { \
-                            const int wps_ = ceil_div(D / 8, 32 * W); \
-                            const unsigned grid_ = (unsigned)(((long long)nj * Nv * wps_ + 7) / 8); \
-                            dv_gather_grouped_kernel<OUT, U, W, MB><<<grid_, 256, 0, st>>>(qb16, entries, segc, Tp, J0, nj, n_groups, Nv, D, wps_, b > 0, DST); \
-                        } while (0)
+                        const int wps_ = ceil_div(D / 8, 32 * W); \
+                        const unsigned grid_ = (unsigned)(((long long)nj * Nv * wps_ + 7) / 8); \
+                        dv_gather_grouped_kernel<OUT, U, W, MB><<<grid_, 256, 0, st>>>(qb16, entries, segs, Tp, J0, nj, n_groups, Mrows, Nv, D, wps_, b > 0, DST); \
+                    } while (0)
 #define TRIAD_DVG(OUT, DST, J0) \
-                        if (wide_rows) TRIAD_DVG_K(OUT, DST, J0, 4, 2, 4); else TRIAD_DVG_K(OUT, DST, J0, 8, 1, 3);
-                        if (pl.scratch) { TRIAD_DVG(float, scratch, 0) }
-                        else if (out_f32) { TRIAD_DVG(float, (float*)dv, j0) }
-                        else { TRIAD_DVG(__nv_bfloat16, (__nv_bfloat16*)dv, j0) }
+                    if (wide_rows) TRIAD_DVG_K(OUT, DST, J0, 4, 2, 4); else TRIAD_DVG_K(OUT, DST, J0, 8, 1, 3);
+                    if (pl.scratch) { TRIAD_DVG(float, scratch, 0) }
+                    else if (out_f32) { TRIAD_DVG(float, (float*)dv, j0) }
+                    else { TRIAD_DVG(__nv_bfloat16, (__nv_bfloat16*)dv, j0) }
 #undef TRIAD_DVG
 #undef TRIAD_DVG_K
-                        TRIAD_LAUNCH_CHECK("dv_gather_grouped_kernel");
-                        continue;
-                    }
+                    TRIAD_LAUNCH_CHECK("dv_gather_grouped_kernel");
+                } else {
+                    if (pl.scratch)      // accumulate this image batch in fp32 scratch (local image index), convert at the end
+                        dv_gather_kernel<T, float><<<ggrid, 256, 0, st>>>(q_b, entries, seg, Tp, 0, nj, Nv, D, wps, Mb, b > 0, scratch);
+                    else if (out_f32)
+                        dv_gather_kernel<T, float><<<ggrid, 256, 0, st>>>(q_b, entries, seg, Tp, j0, nj, Nv, D, wps, Mb, b > 0, (float*)dv);
+                    else
+                        dv_gather_kernel<T, T><<<ggrid, 256, 0, st>>>(q_b, entries, seg, Tp, j0, nj, Nv, D, wps, Mb, b > 0, (T*)dv);
+                    TRIAD_LAUNCH_CHECK("dv_gather_kernel");
                 }
-                dv_count_kernel<IdxT><<<sort_grid, kSortWarps * 32, smem, st>>>(idx_b, rs_b, img_pitch, j0, nj, nq, Nq, Nv, nq_pad, cnt);
-                TRIAD_LAUNCH_CHECK("dv_count_kernel");
-                dv_offsets_kernel<<<nj, 1024, 0, st>>>(cnt, nj, Nv, start, seg);
-                TRIAD_LAUNCH_CHECK("dv_offsets_kernel");
-                dv_scatter_sort_kernel<IdxT><<<sort_grid, kSortWarps * 32, smem, st>>>(
-                    idx_b, g_b, rs_b, start, img_pitch, j0, nj, nq, Bv, Nq, Nv, nq_pad, Mb, entries);
-                TRIAD_LAUNCH_CHECK("dv_scatter_sort_kernel");
-                if constexpr (sizeof(T) == 2) {
-                    if (!(bwd_flags & TRIAD_BWD_GENERIC_DV)) {
-                        const __nv_bfloat16* qb16 = (const __nv_bfloat16*)q_b;
-                        // rows of more than 512 bytes: one warp per segment, two 16-byte loads per lane and row
-                        // (measured at cfg 2: 1.46 -> 1.36 ms for the whole dv pass); otherwise one load per lane
-                        const bool wide_rows = D > 256;
-#define TRIAD_DVG_K(OUT, DST, J0, U, W, MB) do { \
-                            const int wps_ = ceil_div(D / 8, 32 * W); \
-                            const unsigned grid_ = (unsigned)(((long long)nj * Nv * wps_ + 7) / 8); \
-                            dv_gather_bf16_kernel<OUT, U, W, MB><<<grid_, 256, 0, st>>>(qb16, entries, seg, Tp, J0, nj, Nv, D, wps_, Mb, b > 0, DST); \
-                        } while (0)
-#define TRIAD_DVG(OUT, DST, J0) \
-                        if (wide_rows) TRIAD_DVG_K(OUT, DST, J0, 4, 2, 4); else TRIAD_DVG_K(OUT, DST, J0, 8, 1, 3);
-                        if (pl.scratch) { TRIAD_DVG(float, scratch, 0) }
-                        else if (out_f32) { TRIAD_DVG(float, (float*)dv, j0) }
-                        else { TRIAD_DVG(__nv_bfloat16, (__nv_bfloat16*)dv, j0) }
-#undef TRIAD_DVG
-#undef TRIAD_DVG_K
-                        TRIAD_LAUNCH_CHECK("dv_gather_bf16_kernel");
-                        continue;
-                    }
-                }
-                if (pl.scratch)          // accumulate this image batch in fp32 scratch (local image index), convert at the end
-                    dv_gather_kernel<T, float><<<ggrid, 256, 0, st>>>(q_b, entries, seg, Tp, 0, nj, Nv, D, wps, Mb, b > 0, scratch);
-                else if (out_f32)
-                    dv_gather_kernel<T, float><<<ggrid, 256, 0, st>>>(q_b, entries, seg, Tp, j0, nj, Nv, D, wps, Mb, b > 0, (float*)dv);
-                else
-                    dv_gather_kernel<T, T><<<ggrid, 256, 0, st>>>(q_b, entries, seg, Tp, j0, nj, Nv, D, wps, Mb, b > 0, (T*)dv);
-                TRIAD_LAUNCH_CHECK("dv_gather_kernel");
             }
             if (pl.scratch) {
                 const size_t n = (size_t)nj * Nv * D;
@@ -1024,6 +948,7 @@ extern "C" int triad_maxmean_bwd(const void* q, const void* v, const void* idx, 
         return fail_msg(TRIAD_ERR_BAD_SHAPE, "maxmean_bwd: bad shape");
     if (dtype != TRIAD_DTYPE_F32 && dtype != TRIAD_DTYPE_BF16) return fail_msg(TRIAD_ERR_BAD_ARG, "maxmean_bwd: dtype");
     if (flags & ~kBwdFlags) return fail_msg(TRIAD_ERR_BAD_ARG, "maxmean_bwd: unknown flag bit");
+    if (dv && Nv > kDvMaxNv) return fail_msg(TRIAD_ERR_UNSUPPORTED, "maxmean_bwd: dv needs Nv <= 3072");
     if (((uintptr_t)q | (uintptr_t)v | (uintptr_t)dq | (uintptr_t)dv | (uintptr_t)ws) & 15) return fail_msg(TRIAD_ERR_ALIGNMENT, "maxmean_bwd: 16-byte alignment");
     if (!ws || ws_bytes < ((dv || (flags & TRIAD_BWD_PACK_ROWS)) ? triad_maxmean_bwd_workspace_bytes(Bq, Bv, Nq, Nv, D, dtype) : kCtrlBytes))
         return fail_msg(TRIAD_ERR_WORKSPACE, "maxmean_bwd: workspace too small");
