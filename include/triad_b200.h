@@ -57,8 +57,6 @@ extern "C" {
 #define TRIAD_FWD_PACK_ROWS   16   /* bf16 tensor-core path: rows whose row_scale is 0 (padded text tokens,
                                       model.py:509-512) are dropped before the GEMM; their idx entries read 0 */
 
-#define TRIAD_FWD_PROBE_NO_N_STORES 64 /* timing probe (tools/emit_probe.py): triad_maxmean_fwd_nonneg does all its arithmetic
-                                          but stores no N */
 #define TRIAD_FWD_TEST_TRIP_WATCHDOG 32 /* test aid: raise the pipeline-watchdog flag after the kernel, as a timed-out
                                          barrier wait would: clip must come back NaN (never a silent garbage matrix) */
 

@@ -56,9 +56,12 @@ def test_merged_forward_equals_its_parts(shape, flags):
     assert torch.equal(clip0, clip1)
     assert torch.equal(idx0.view(Bv, Bq, -1)[:, :, :Nq], idx1.view(Bv, Bq, -1)[:, :, :Nq])
     assert torch.equal(N0, N1)
-    # the same squares; the merged pass sums a row's 256 columns in one warp, the regulariser-only pass in two halves:
-    # fp32 association of the per-tile sums differs, nothing else
-    assert ((sums0 - sums1).abs() <= 1e-6 * sums0.abs()).all()
+    # both passes sum in the same emission warps; the regulariser-only pass always runs CTA pairs in the default tile
+    # order, so with other flags the per-tile sums are added in a different order: fp32 association, nothing else
+    if flags == 0:
+        assert torch.equal(sums0, sums1)
+    else:
+        assert ((sums0 - sums1).abs() <= 1e-6 * sums0.abs()).all()
     Nref, s2, sT = _dense_reference(q, v, 1.5, lo, coef)
     err = ((N1.double() - Nref).norm() / Nref.norm()).item()
     assert err < 4e-3, err                                                          # one bf16 rounding of N
@@ -84,7 +87,7 @@ def test_merged_forward_at_the_clamp_floor():
     clip1, idx1, N1, sums1 = ops.maxmean_fwd_nonneg(q, v, scale, T, lo, coef)
     assert torch.equal(clip0, clip1)
     assert torch.equal(idx0.view(Bv, Bq, -1)[:, :, :Nq], idx1.view(Bv, Bq, -1)[:, :, :Nq])     # (beyond Nq: padding)
-    assert torch.equal(N0, N1) and ((sums0 - sums1).abs() <= 1e-6 * sums0.abs()).all()
+    assert torch.equal(N0, N1) and torch.equal(sums0, sums1)
     # gate: nothing flows where the bf16-rounded similarity is below the floor
     S_ref = (raw.bfloat16().float() * 1.5).bfloat16().float()
     assert (N1[S_ref < lo] == 0).all()

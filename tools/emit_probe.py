@@ -37,8 +37,6 @@ def main():
     print("regulariser, no stores ", timed(lambda: R.nonneg_fused_chunk(q, v, T, -60.0, coef, False, sums)))
     print("regulariser, stores    ", timed(lambda: R.nonneg_fused_chunk(q, v, T, -60.0, coef, True, sums)))
     print("merged                 ", timed(lambda: ops.maxmean_fwd_nonneg(q, v, scale, T, -60.0, coef)))
-    from triad_b200 import _lib
-    print("merged, no stores      ", timed(lambda: ops.maxmean_fwd_nonneg(q, v, scale, T, -60.0, coef, flags=_lib.FWD_PROBE_NO_N_STORES)))
     print("zero_ of N (%.1f GB)    " % (N.numel() * 2 / 1e9), timed(lambda: N.zero_()))
     print("fill_ of N             ", timed(lambda: N.fill_(1.0)))
     M = torch.empty_like(N)

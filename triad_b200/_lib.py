@@ -17,7 +17,6 @@ DTYPE_F32, DTYPE_BF16 = 0, 1
 FWD_DEFAULT, FWD_FORCE_SIMT, FWD_FORCE_1CTA, FWD_DIVIDE_BY_T, FWD_SYNC_CHUNKS, FWD_PACK_ROWS = 0, 1, 2, 4, 8, 16
 BWD_DEFAULT, BWD_GENERIC_DQ, BWD_GENERIC_DV, BWD_SMALL_BLOCKS, BWD_PACK_ROWS = 0, 1, 2, 16, 32
 FWD_TEST_TRIP_WATCHDOG = 32
-FWD_PROBE_NO_N_STORES = 64
 BWD_TEST_TRIP_WATCHDOG = 256
 BWD_UNIFORM_SCALE = 128
 

@@ -175,7 +175,7 @@ extern "C" int triad_maxmean_fwd_nonneg(const void* q, const void* v, const floa
     float* part = (float*)((char*)ws + 256);
     double* npart = (double*)((char*)ws + 256 + fwd_part_bytes(M, Bv, Nq));
     TRIAD_CUDA_CHECK(cudaMemsetAsync(abort_flag, 0, 256, st));
-    EmitNArgs e{n_out, ldn, lo, coef, (flags & TRIAD_FWD_PROBE_NO_N_STORES) ? 0 : 1, npart, 1};
+    EmitNArgs e{n_out, ldn, lo, coef, 1, npart, 1};
     const int cta_group = (flags & TRIAD_FWD_FORCE_1CTA) ? 1 : 2;
     int rc = launch_maxmean_tc(q, v, row_scale, temperature, 0, M, Bv, Nq, Nv, D, part, idx, abort_flag, cta_group, flags,
                                nullptr, &e, st);

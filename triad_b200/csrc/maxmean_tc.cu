@@ -80,7 +80,8 @@ struct Params {
     long long ldn;
     float lo, coef;          // clamp floor (< 0), 2*weight/numel
     int write_n;             // 0: value only
-    double* n_partials;      // [gridDim.x*4][2]: sum clamp^2, sum dS*<q,v> per epilogue warp
+    double* n_partials;      // [gridDim.x*8][2]: sum clamp^2, sum dS*<q,v>; slot blockIdx.x*8 + (warp - 4), written by the
+                             // emission warps 8-11 (slots of the other epilogue warps stay as cleared)
 };
 
 __device__ __forceinline__ float fmax3(float a, float b, float c) { return fmaxf(fmaxf(a, b), c); }
@@ -121,17 +122,18 @@ __device__ __forceinline__ void first_ge32(const uint32_t (&r)[32], int col0, in
 
 // ---- dense-regulariser epilogue (kMode 1: instead of the max-mean reduction; kMode 2: next to it) -----------------
 // N = coef*T*min(T*acc, 0) = (coef*T^2) * min(acc, 0) for T > 0, written as bf16.  A thread owns a ROW of the
-// accumulator, so storing straight from registers would hit 32 different rows per store instruction.  Each epilogue
+// accumulator, so storing straight from registers would hit 32 different rows per store instruction.  Each emission
 // warp instead stages a 32-row x 64-column box (4 KB, the SWIZZLE_128B layout of a TMA box: 16-byte piece c of row
 // r sits at piece c ^ (r & 7), so the 32 lanes' st.shared.v4 are conflict-free) and ONE lane hands it to the TMA
 // unit (cp.async.bulk.tensor store): no per-lane global stores, no address arithmetic, and rows >= M / columns >= Nv
 // are clipped by the tensor map {Nv, images, M}.  Round 1's version (per-lane 16-byte stores out of a transposing
 // staging buffer) spent 4 dependent STS -> LDS -> STG round trips per chunk: 3.8 ms per pass against 2.45 ms for
 // the plain forward.
-constexpr int kEmitEpiWarps = 8;                                    // two per scheduler: columns [0,128) and [128,256)
+constexpr int kEmitEpiWarps = 8;                                    // epilogue warps 4-11; one n_partials slot each
 constexpr int kEmitThreads = (kEpiWarp0 + kEmitEpiWarps) * 32;      // 384
 constexpr uint32_t kStgBytesPerWarp = 32 * 128;                     // one 32 x 64 bf16 box
-constexpr uint32_t kStgBytes = kEmitEpiWarps * kStgBytesPerWarp;    // 32 KB, carved from the end of the V ring
+constexpr uint32_t kStgBytes = 4 * 2 * kStgBytesPerWarp;            // four emission warps x two boxes: 32 KB, carved
+                                                                    // from the end of the V ring
 constexpr uint16_t kNoCol = 0xffffu;                                // "no column of my half reaches the threshold"
 
 __device__ __forceinline__ void sts128(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
@@ -296,18 +298,19 @@ struct TileIter {
 // ---------------------------------------------------------------------------------------------
 // kSub = false: one accumulator tile per image (Nv <= 256), the training shapes' hot path;
 // kSub = true : n_sub 256-patch sub-tiles per image.
-// kMode 0: max-mean reduction (the contrastive forward / retrieval); 1: dense-regulariser pass only (the epilogue
-// writes N = dL/d<q,v> of the non-negative pressure term); 2: BOTH in one pass over the similarities — the training
-// step with the reference's full loss needs the max-mean reduction and N of the very same tiles.
+// kMode 0: max-mean reduction (the contrastive forward / retrieval); 2: BOTH the max-mean reduction (warps 4-7) and
+// the dense regulariser (emission warps 8-11 write N = dL/d<q,v> of the non-negative pressure term) in one pass over
+// the similarities — the training step with the reference's full loss needs both of the very same tiles; 1: kMode 2
+// without the max-mean warps (the regulariser-only pass).
 template <int kCtaGroup, bool kSub, int kMode = 0>
 __global__ void __launch_bounds__(kEmitThreads, 1)
 maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_v,
                   const __grid_constant__ CUtensorMap tmap_n, const Params p) {
     constexpr bool kEmitN = kMode != 0;
     constexpr int kVStageBytes = (kMaxN / kCtaGroup) * kBlockK * 2;       // 32 KB / 16 KB
-    // the dense-regulariser modes give the last 32 KB of the ring to the epilogue's store staging: kMode 1 eight warps x
-    // one 4 KB box (32 rows x 64 columns), kMode 2 four emission warps x two such boxes.  (Two 2 KB boxes of 32 columns
-    // per emission warp, i.e. 5 ring stages instead of 4, were measured: no faster, twice the bulk stores.)
+    // the dense-regulariser modes give the last 32 KB of the ring to the epilogue's store staging: four emission warps x
+    // two 4 KB boxes (32 rows x 64 columns).  (Two 2 KB boxes of 32 columns per emission warp, i.e. 5 ring stages
+    // instead of 4, were measured: no faster, twice the bulk stores.)
     constexpr uint32_t kStgTotal = kMode != 0 ? kStgBytes : 0u;
     constexpr int kStages = (kVRingBytes - kStgTotal) / kVStageBytes;                  // 3 / 6  (2 / 4)
     constexpr int kTileRows = kBlockM * kCtaGroup;
@@ -352,7 +355,10 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
         for (int i = 0; i < kMaxKB; ++i) mbar_init(bar_q_full + 8 * i, 1);
         mbar_init(bar_q_empty, 1);
         for (int i = 0; i < kStages; ++i) { mbar_init(bar_v_full + 8 * i, 1); mbar_init(bar_v_empty + 8 * i, 1); }
-        for (int i = 0; i < 2; ++i) { mbar_init(bar_t_full + 8 * i, 1); mbar_init(bar_t_empty + 8 * i, ((kEmitN || p.idx != nullptr) ? kEmitEpiWarps : 4) * kCtaGroup); }
+        // arrivals that free an accumulator: kMode 2 its four max-mean and four emission warps, kMode 1 the four
+        // emission warps, kMode 0 the eight max-mean warps (four when no idx is wanted: the upper halves sit out)
+        const int t_empty_warps = kMode == 2 ? 8 : kMode == 1 ? 4 : (p.idx != nullptr ? 8 : 4);
+        for (int i = 0; i < 2; ++i) { mbar_init(bar_t_full + 8 * i, 1); mbar_init(bar_t_empty + 8 * i, t_empty_warps * kCtaGroup); }
         fence_barrier_init();
     }
     if (warp == 2) tmem_alloc<kCtaGroup>(tmem_ptr_smem, kTmemCols);
@@ -457,105 +463,17 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
                 prev_m = t.m;
             }
         }
-    } else if (warp >= kEpiWarp0 && kMode == 1) {
-        // ============ epilogue, dense-regulariser mode: N = coef*T*min(S,0) for every pair =============
+    } else if (kEmitN && warp >= kEpiWarp0 + 4) {
+        // ============ emission warps: N = coef*T*min(S,0) for every pair (one warp per TMEM lane quarter) =============
         // One pass over the accumulator: n = min(acc, 0); the tile's sum of n^2 (times T^2) feeds the value and,
         // because n*s == n^2, also dL/dT (sum dS*<q,v> = sum n^2 / T).  The clamp floor `lo` (-60 / -20) is far
         // outside the data range; a tile that does come near it (row minimum within two bf16 ulps of lo) is redone
         // with the reference's bf16 rounding of S, clamp and gradient gate before its accumulator is released.
         // Padded text tokens take part, as in the reference (model.py:525).
-        const int quarter = warp & 3;
-        const uint32_t t_empty_sig = (kCtaGroup == 2) ? mapa(bar_t_empty, 0) : bar_t_empty;
-        const float Tval = *p.T;
-        const float coefT = p.coef * Tval;
-        const float2 cT2 = make_float2(coefT * Tval, coefT * Tval);
-        const float T2f = Tval * Tval;
-        const int half = (warp - kEpiWarp0) >> 2;                  // 0: columns [0,128), 1: [128,256)
-        const uint32_t stg = v_smem + (uint32_t)kStages * (uint32_t)kVStageBytes + (uint32_t)(warp - kEpiWarp0) * kStgBytesPerWarp;
-        const uint32_t stg_row = stg + (uint32_t)lane * 128u;
-        const bool wn = p.write_n != 0;
-        double s2 = 0.0, sT = 0.0;
-        uint32_t t_cnt = 0;
-        bool alive = true;
-        Tile t;
-        const int own = half * 4;                                   // this warp's 32-column chunks: [own, own + 4)
-        while (alive && it.next(t)) {
-            const int wrow0 = t.m * kTileRows + (int)cta_rank * kBlockM + quarter * 32;      // the warp's first row
-            const bool vrow = wrow0 + lane < p.M;
-            const uint32_t acc = t_cnt & 1u, acc_phase = (t_cnt >> 1) & 1u;
-            ++t_cnt;
-            bool ok = mbar_wait(bar_t_full + 8 * acc, acc_phase, p.abort_flag, 6);
-            ok = __all_sync(0xffffffffu, ok);
-            if (!ok) { alive = false; break; }
-            tc_fence_after();
-            const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * kMaxN;
-            // ---- fast pass: pipelined 32-column loads (chunk c+1 in flight while chunk c is processed); two chunks
-            //      fill one staged box, which leaves through the TMA unit while the next two are processed ----
-            float2 a2[2] = {make_float2(0.f, 0.f), make_float2(0.f, 0.f)};
-            float mn[2] = {0.f, 0.f};
-            {
-                uint32_t bufA[32], bufB[32], w[16];
-                tmem_ld32_raw(taddr + own * 32, bufA);
-                tmem_wait_ld();
-#pragma unroll
-                for (int b = 0; b < 2; ++b) {
-                    const int c = own + 2 * b;
-                    tmem_ld32_raw(taddr + (c + 1) * 32, bufB);
-                    emit_chunk(bufA, c * 32, p.Nv, cT2, a2, mn, w);
-                    if (wn) { emit_box_reusable(lane); stage_chunk(w, stg_row, lane, 0); }   // (the previous box has been read)
-                    tmem_wait_ld();
-                    if (b == 0) tmem_ld32_raw(taddr + (c + 2) * 32, bufA);               // compile-time condition
-                    emit_chunk(bufB, (c + 1) * 32, p.Nv, cT2, a2, mn, w);
-                    if (wn) { stage_chunk(w, stg_row, lane, 1); if (c * 32 < p.Nv) emit_box_store(&tmap_n, stg, c * 32, t.j, wrow0, lane); }
-                    tmem_wait_ld();
-                }
-            }
-            const float a2s = (a2[0].x + a2[0].y) + (a2[1].x + a2[1].y);
-            const float mns = fminf(mn[0], mn[1]) * Tval;
-            // (margin of two bf16 ulps: the reference clamps the bf16-ROUNDED similarity, so a value a hair above
-            //  the floor in fp32 can sit on it after rounding)
-            if (!__any_sync(0xffffffffu, vrow && mns < p.lo * (1.0f - 1.0f / 64.0f))) {
-                if (vrow) { s2 += (double)(a2s * T2f); sT += (double)(a2s * Tval); }
-            } else {
-                // ---- exact pass (some similarity of this warp's rows is below the clamp floor): redo the tile with
-                //      the clamp and its gradient gate applied, overwriting what the fast pass stored ----
-                float e2 = 0.f, eT = 0.f;
-                if (wn) emit_box_drain(lane);                               // the fast pass's stores have landed
-                for (int b = 0; b < 2; ++b) {
-                    const int c = own + 2 * b;
-                    if (c * 32 >= p.Nv) break;                              // warp-uniform
-                    uint32_t buf[32], w[16];
-                    tmem_ld32_raw(taddr + c * 32, buf);
-                    tmem_wait_ld();
-                    emit_chunk_exact(buf, c * 32, p.Nv, Tval, coefT, p.lo, e2, eT, w);
-                    if (wn) { emit_box_reusable(lane); stage_chunk(w, stg_row, lane, 0); }
-                    tmem_ld32_raw(taddr + (c + 1) * 32, buf);
-                    tmem_wait_ld();
-                    emit_chunk_exact(buf, (c + 1) * 32, p.Nv, Tval, coefT, p.lo, e2, eT, w);
-                    if (wn) { stage_chunk(w, stg_row, lane, 1); emit_box_store(&tmap_n, stg, c * 32, t.j, wrow0, lane); }
-                }
-                if (vrow) { s2 += (double)e2; sT += (double)eT; }
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) {
-                if constexpr (kCtaGroup == 2) mbar_arrive_cluster(t_empty_sig + 8 * acc);
-                else mbar_arrive_local(bar_t_empty + 8 * acc);
-            }
-        }
-        emit_box_reusable(lane);                                    // the staging box must outlive the last bulk read
-        s2 = warp_sum_d(s2);
-        sT = warp_sum_d(sT);
-        if (lane == 0) {
-            p.n_partials[(size_t)(blockIdx.x * kEmitEpiWarps + (warp - kEpiWarp0)) * 2] = s2;
-            p.n_partials[(size_t)(blockIdx.x * kEmitEpiWarps + (warp - kEpiWarp0)) * 2 + 1] = sT * (double)p.coef;
-        }
-    } else if (kMode == 2 && warp >= kEpiWarp0 + 4) {
-        // ============ kMode 2, emission warps (one per TMEM lane quarter, all 256 columns) =============
-        // Same arithmetic as the kMode 1 branch.  The max-mean epilogue runs beside it in warps 4-7 (one warp per
-        // quarter, the round-1 arrangement): two independent ~1 000-instruction chains per scheduler instead of two
-        // ~1 500-instruction ones doing both jobs.  The 8 KB of staging per warp are two 32 x 64 boxes: a box leaves
-        // through the TMA unit while the next one is filled (cp.async.bulk.wait_group.read 1).
+        // In kMode 2 the max-mean epilogue runs beside these warps in warps 4-7 (one warp per quarter, the round-1
+        // arrangement): two independent ~1 000-instruction chains per scheduler instead of two ~1 500-instruction ones
+        // doing both jobs; in kMode 1 warps 4-7 have no work.  The 8 KB of staging per warp are two 32 x 64 boxes: a
+        // box leaves through the TMA unit while the next one is filled (cp.async.bulk.wait_group.read 1).
         const int quarter = warp & 3;
         const uint32_t t_empty_sig = (kCtaGroup == 2) ? mapa(bar_t_empty, 0) : bar_t_empty;
         const float Tval = *p.T;
@@ -606,10 +524,13 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             }
             const float a2s = (a2[0].x + a2[0].y) + (a2[1].x + a2[1].y);
             const float mns = fminf(mn[0], mn[1]) * Tval;
+            // (margin of two bf16 ulps: the reference clamps the bf16-ROUNDED similarity, so a value a hair above
+            //  the floor in fp32 can sit on it after rounding)
             if (!__any_sync(0xffffffffu, vrow && mns < p.lo * (1.0f - 1.0f / 64.0f))) {
                 if (vrow) { kahan_add(s2, s2c, a2s * T2f); kahan_add(sT, sTc, a2s * Tval); }
             } else {
-                // exact pass (a similarity of this warp's rows is at the clamp floor): see the kMode 1 branch
+                // exact pass (some similarity of this warp's rows is below the clamp floor): redo the tile with the
+                // clamp and its gradient gate applied, overwriting what the fast pass stored
                 float e2 = 0.f, eT = 0.f;
                 if (wn) emit_box_drain(lane);
                 for (int b = 0; b < 4; ++b) {
@@ -643,7 +564,7 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             p.n_partials[(size_t)(blockIdx.x * kEmitEpiWarps + (warp - kEpiWarp0)) * 2] = s2d;
             p.n_partials[(size_t)(blockIdx.x * kEmitEpiWarps + (warp - kEpiWarp0)) * 2 + 1] = sTd * (double)p.coef;
         }
-    } else if (warp >= kEpiWarp0 && (p.idx != nullptr || warp < kEpiWarp0 + 4)) {
+    } else if (kMode != 1 && warp >= kEpiWarp0 && (p.idx != nullptr || warp < kEpiWarp0 + 4)) {
         // =============================== epilogue =======================================
         // Two warps per TMEM lane quarter (one per scheduler pair): both take the row maximum over all columns
         // (cheap: FMNMX3), then each searches ITS half of the columns for the first one that reaches the
@@ -953,7 +874,7 @@ int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, cons
     if ((long long)n_clusters > total) n_clusters = (int)total;
     if (n_clusters < 1) n_clusters = 1;
     if (emit) {
-        // every CTA's eight epilogue warps write a partial: clear the slots of CTAs that get no work
+        // one slot per epilogue warp of every CTA, written only by the emission warps of CTAs that get work: clear all
         TRIAD_CUDA_CHECK(cudaMemsetAsync(emit->partials, 0, (size_t)sms * kEmitEpiWarps * 2 * sizeof(double), st));
         if (emit->with_maxmean)
             return cta_group == 2 ? launch_t<2, false, 2>(mq, mv, mn, p, n_clusters, st) : launch_t<1, false, 2>(mq, mv, mn, p, n_clusters, st);
