@@ -152,6 +152,10 @@ int triad_contrastive_head(const float* clip, int B, const float* temperature,
 #define TRIAD_BWD_UNIFORM_SCALE 128  /* the caller guarantees row_scale has no zeros (no attention mask): the dv sort then
                                       does not read it per row to decide which rows to list                            */
 #define TRIAD_BWD_TEST_TRIP_WATCHDOG 256 /* test aid: raise the watchdog flag before the kernels run: dq must come back NaN */
+#define TRIAD_BWD_ACCUMULATE_DV 1024 /* dv += the gradient instead of dv = (every query block adds to the caller's
+                                        values, the first one included), so a row-sharded step can land one rank's
+                                        contrastive dv on its dense-regulariser dV in one fp32 buffer; needs fp32 dv
+                                        (dv_f32 != 0 or fp32 inputs), TRIAD_ERR_BAD_ARG otherwise */
 size_t triad_maxmean_bwd_workspace_bytes(int Bq, int Bv, int Nq, int Nv, int D, int dtype);
 int triad_maxmean_bwd(const void* q, const void* v, const void* idx, const float* g,
                       const float* clip, const float* row_scale, const float* temperature,
@@ -203,6 +207,13 @@ int triad_maxmean_fwd_nonneg(const void* q, const void* v, const float* row_scal
 size_t triad_dense_grad_gemm_workspace_bytes(int M, int Kc, int D, int mode);
 int triad_dense_grad_gemm(const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode,
                           void* out, void* ws, size_t ws_bytes, void* stream);
+/* The same product with an fp32 output (same workspace query).  accumulate = 0: out = sum of the K splits in order
+ * (bf16(out) is bit for bit what triad_dense_grad_gemm writes); accumulate = 1: out = out + (sum of the splits in
+ * order), added once per element, so a zero `out` ends up equal to accumulate = 0.  Deterministic, no atomics.  Lets a
+ * caller carry dQ across image chunks in fp32, or write a chunk's dV straight into its rows of a larger fp32 buffer.
+ * Any other `accumulate` fails with TRIAD_ERR_BAD_ARG. */
+int triad_dense_grad_gemm_f32(const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode,
+                              float* out, int accumulate, void* ws, size_t ws_bytes, void* stream);
 
 /* Regularisers on the B POSITIVE pairs only (token_sims[i,i]): temporal smoothness (mode 0, model.py:394-408:
  * mean over (i, a < Nq-1, p) of (S[i,a+1,p] - S[i,a,p])^2) and patch-usage sparsity (mode 1, model.py:528-541:

@@ -19,6 +19,7 @@ BWD_DEFAULT, BWD_GENERIC_DQ, BWD_GENERIC_DV, BWD_SMALL_BLOCKS, BWD_PACK_ROWS = 0
 FWD_TEST_TRIP_WATCHDOG = 32
 BWD_TEST_TRIP_WATCHDOG = 256
 BWD_UNIFORM_SCALE = 128
+BWD_ACCUMULATE_DV = 1024
 
 # name -> (restype, argtypes); must list every symbol of include/triad_b200.h
 SIGNATURES = {
@@ -59,6 +60,8 @@ SIGNATURES = {
     "triad_dense_grad_gemm_workspace_bytes": (c_size_t, [c_int] * 4),
     "triad_dense_grad_gemm": (c_int, [c_void_p, ctypes.c_longlong, c_int, c_int, c_void_p, c_int, c_int, c_void_p,
                                       c_void_p, c_size_t, c_void_p]),
+    "triad_dense_grad_gemm_f32": (c_int, [c_void_p, ctypes.c_longlong, c_int, c_int, c_void_p, c_int, c_int, c_void_p,
+                                          c_int, c_void_p, c_size_t, c_void_p]),
     "triad_pospair_workspace_bytes": (c_size_t, [c_int]),
     "triad_pospair_terms": (c_int, [c_void_p, c_int, c_void_p, c_int, c_float, c_int, c_int, c_int, c_void_p, c_void_p,
                                     c_void_p, c_size_t, c_void_p]),

@@ -20,7 +20,9 @@
 // count (cfg 2: 250 row tiles x 2 = 500 items on 74 pairs).  Every item writes an fp32 partial tile (TMA bulk-tensor
 // stores of swizzled 32 x 32 boxes, as the forward's N emission); a second launch adds the splits in order and rounds
 // to bf16 once — deterministic, no atomics.  Out-of-range rows / columns / K are zero-filled by the loads and clipped
-// by the stores (the tensor maps carry the true extents).
+// by the stores (the tensor maps carry the true extents).  triad_dense_grad_gemm_f32 differs in that second launch
+// only: it writes the fp32 sum, or adds it to the caller's fp32 output (an accumulator carried across image chunks, or
+// one chunk's rows of a per-rank dV partial).
 #include "common.cuh"
 #include "ptx.cuh"
 
@@ -222,9 +224,14 @@ dgemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
     if (warp == 2) tmem_dealloc<2>(tmem0, 512);
 }
 
-// out[r][d] = bf16( sum over splits, in order, of part[s][r][d] ); NaN everywhere if the GEMM's watchdog fired
+// What the split reduction writes: bf16(sum), the fp32 sum, or out + sum in fp32 (the splits are added in order
+// first, then to out once, so accumulating onto zeros gives the bits of kOutF32)
+enum { kOutBf16 = 0, kOutF32 = 1, kOutF32Add = 2 };
+
+// out[r][d] = sum over splits, in order, of part[s][r][d]; NaN everywhere if the GEMM's watchdog fired
+template <int kOut>
 __global__ void __launch_bounds__(256)
-reduce_kernel(const float4* __restrict__ part, size_t n4, int splits, uint2* __restrict__ out, const int* __restrict__ abort_flag) {
+reduce_kernel(const float4* __restrict__ part, size_t n4, int splits, void* __restrict__ out, const int* __restrict__ abort_flag) {
     const bool poisoned = *abort_flag != 0;
     for (size_t k = (size_t)blockIdx.x * 256 + threadIdx.x; k < n4; k += (size_t)gridDim.x * 256) {
         float4 a = part[k];
@@ -232,9 +239,17 @@ reduce_kernel(const float4* __restrict__ part, size_t n4, int splits, uint2* __r
             const float4 b = part[(size_t)s * n4 + k];
             a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w;
         }
+        if constexpr (kOut == kOutF32Add) {
+            const float4 o = reinterpret_cast<const float4*>(out)[k];
+            a.x = o.x + a.x; a.y = o.y + a.y; a.z = o.z + a.z; a.w = o.w + a.w;
+        }
         if (poisoned) a.x = a.y = a.z = a.w = __int_as_float(0x7fc00000);
-        __nv_bfloat162 lo = __floats2bfloat162_rn(a.x, a.y), hi = __floats2bfloat162_rn(a.z, a.w);
-        out[k] = make_uint2(*reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi));
+        if constexpr (kOut == kOutBf16) {
+            __nv_bfloat162 lo = __floats2bfloat162_rn(a.x, a.y), hi = __floats2bfloat162_rn(a.z, a.w);
+            reinterpret_cast<uint2*>(out)[k] = make_uint2(*reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi));
+        } else {
+            reinterpret_cast<float4*>(out)[k] = a;
+        }
     }
 }
 
@@ -279,8 +294,8 @@ extern "C" size_t triad_dense_grad_gemm_workspace_bytes(int M, int Kc, int D, in
     return 256 + (size_t)splits * (size_t)(mode == 0 ? M : Kc) * (size_t)D * sizeof(float);
 }
 
-extern "C" int triad_dense_grad_gemm(const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode,
-                                     void* out, void* ws, size_t ws_bytes, void* stream) {
+static int dense_grad_gemm_run(const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode,
+                               void* out, int out_kind, void* ws, size_t ws_bytes, void* stream) {
     using namespace dgemm;
     if (!n_mat || !x || !out || !ws) return fail_msg(TRIAD_ERR_BAD_ARG, "dense_grad_gemm: null pointer");
     if (mode != 0 && mode != 1) return fail_msg(TRIAD_ERR_BAD_ARG, "dense_grad_gemm: mode");
@@ -358,7 +373,21 @@ extern "C" int triad_dense_grad_gemm(const void* n_mat, long long ldn, int M, in
     const size_t n4 = (size_t)rows_out * D / 4;
     size_t want = (n4 + 255) / 256;
     const int blocks = (int)(want > (size_t)(148 * 16) ? (size_t)(148 * 16) : (want < 1 ? 1 : want));
-    reduce_kernel<<<blocks, 256, 0, st>>>((const float4*)part, n4, p.splits, (uint2*)out, (const int*)ws);
+    if (out_kind == kOutBf16)     reduce_kernel<kOutBf16><<<blocks, 256, 0, st>>>((const float4*)part, n4, p.splits, out, (const int*)ws);
+    else if (out_kind == kOutF32) reduce_kernel<kOutF32><<<blocks, 256, 0, st>>>((const float4*)part, n4, p.splits, out, (const int*)ws);
+    else                          reduce_kernel<kOutF32Add><<<blocks, 256, 0, st>>>((const float4*)part, n4, p.splits, out, (const int*)ws);
     TRIAD_LAUNCH_CHECK("dense_grad_gemm reduce_kernel");
     return TRIAD_OK;
+}
+
+extern "C" int triad_dense_grad_gemm(const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode,
+                                     void* out, void* ws, size_t ws_bytes, void* stream) {
+    return dense_grad_gemm_run(n_mat, ldn, M, Kc, x, D, mode, out, dgemm::kOutBf16, ws, ws_bytes, stream);
+}
+
+extern "C" int triad_dense_grad_gemm_f32(const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode,
+                                         float* out, int accumulate, void* ws, size_t ws_bytes, void* stream) {
+    if (accumulate != 0 && accumulate != 1) return fail_msg(TRIAD_ERR_BAD_ARG, "dense_grad_gemm_f32: accumulate must be 0 or 1");
+    return dense_grad_gemm_run(n_mat, ldn, M, Kc, x, D, mode, out, accumulate ? dgemm::kOutF32Add : dgemm::kOutF32,
+                               ws, ws_bytes, stream);
 }

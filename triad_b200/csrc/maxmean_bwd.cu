@@ -831,6 +831,7 @@ static int bwd_typed(const void* q, const void* v, const void* idx, const float*
         const bool grouped = packed && Nv <= kGroupMaxNv;
         const size_t img_pitch = (size_t)Bq * nq_pad;
         const int wps = ceil_div(D / E, 32);                                       // warps per segment
+        const bool add_first = (bwd_flags & TRIAD_BWD_ACCUMULATE_DV) != 0;        // fp32 out (checked): no scratch
         for (int j0 = 0; j0 < Bv; j0 += pl.jb) {
             const int nj = (Bv - j0 < pl.jb) ? (Bv - j0) : pl.jb;
             const int sort_grid = ceil_div(nj * kSortGroups, kSortWarps);
@@ -877,7 +878,7 @@ static int bwd_typed(const void* q, const void* v, const void* idx, const float*
 #define TRIAD_DVG_K(OUT, DST, J0, U, W, MB) do { \
                         const int wps_ = ceil_div(D / 8, 32 * W); \
                         const unsigned grid_ = (unsigned)(((long long)nj * Nv * wps_ + 7) / 8); \
-                        dv_gather_grouped_kernel<OUT, U, W, MB><<<grid_, 256, 0, st>>>(qb16, entries, segs, Tp, J0, nj, n_groups, Mrows, Nv, D, wps_, b > 0, DST); \
+                        dv_gather_grouped_kernel<OUT, U, W, MB><<<grid_, 256, 0, st>>>(qb16, entries, segs, Tp, J0, nj, n_groups, Mrows, Nv, D, wps_, b > 0 || add_first, DST); \
                     } while (0)
 #define TRIAD_DVG(OUT, DST, J0) \
                     if (wide_rows) TRIAD_DVG_K(OUT, DST, J0, 4, 2, 4); else TRIAD_DVG_K(OUT, DST, J0, 8, 1, 3);
@@ -891,7 +892,7 @@ static int bwd_typed(const void* q, const void* v, const void* idx, const float*
                     if (pl.scratch)      // accumulate this image batch in fp32 scratch (local image index), convert at the end
                         dv_gather_kernel<T, float><<<ggrid, 256, 0, st>>>(q_b, entries, seg, Tp, 0, nj, Nv, D, wps, Mb, b > 0, scratch);
                     else if (out_f32)
-                        dv_gather_kernel<T, float><<<ggrid, 256, 0, st>>>(q_b, entries, seg, Tp, j0, nj, Nv, D, wps, Mb, b > 0, (float*)dv);
+                        dv_gather_kernel<T, float><<<ggrid, 256, 0, st>>>(q_b, entries, seg, Tp, j0, nj, Nv, D, wps, Mb, b > 0 || add_first, (float*)dv);
                     else
                         dv_gather_kernel<T, T><<<ggrid, 256, 0, st>>>(q_b, entries, seg, Tp, j0, nj, Nv, D, wps, Mb, b > 0, (T*)dv);
                     TRIAD_LAUNCH_CHECK("dv_gather_kernel");
@@ -922,7 +923,7 @@ using namespace triad;
 
 // every TRIAD_BWD_* bit; any other bit is an error rather than silently ignored
 static constexpr int kBwdFlags = TRIAD_BWD_GENERIC_DQ | TRIAD_BWD_GENERIC_DV | TRIAD_BWD_SMALL_BLOCKS | TRIAD_BWD_PACK_ROWS |
-                                 TRIAD_BWD_UNIFORM_SCALE | TRIAD_BWD_TEST_TRIP_WATCHDOG;
+                                 TRIAD_BWD_UNIFORM_SCALE | TRIAD_BWD_TEST_TRIP_WATCHDOG | TRIAD_BWD_ACCUMULATE_DV;
 
 extern "C" size_t triad_maxmean_bwd_workspace_bytes(int Bq, int Bv, int Nq, int Nv, int D, int dtype) {
     if (Bq <= 0 || Bv <= 0 || Nq <= 0 || Nv <= 0 || D <= 0) return 0;
@@ -948,6 +949,8 @@ extern "C" int triad_maxmean_bwd(const void* q, const void* v, const void* idx, 
         return fail_msg(TRIAD_ERR_BAD_SHAPE, "maxmean_bwd: bad shape");
     if (dtype != TRIAD_DTYPE_F32 && dtype != TRIAD_DTYPE_BF16) return fail_msg(TRIAD_ERR_BAD_ARG, "maxmean_bwd: dtype");
     if (flags & ~kBwdFlags) return fail_msg(TRIAD_ERR_BAD_ARG, "maxmean_bwd: unknown flag bit");
+    if ((flags & TRIAD_BWD_ACCUMULATE_DV) && !dv_f32 && dtype != TRIAD_DTYPE_F32)
+        return fail_msg(TRIAD_ERR_BAD_ARG, "maxmean_bwd: TRIAD_BWD_ACCUMULATE_DV needs an fp32 dv");
     if (dv && Nv > kDvMaxNv) return fail_msg(TRIAD_ERR_UNSUPPORTED, "maxmean_bwd: dv needs Nv <= 3072");
     if (((uintptr_t)q | (uintptr_t)v | (uintptr_t)dq | (uintptr_t)dv | (uintptr_t)ws) & 15) return fail_msg(TRIAD_ERR_ALIGNMENT, "maxmean_bwd: 16-byte alignment");
     if (!ws || ws_bytes < ((dv || (flags & TRIAD_BWD_PACK_ROWS)) ? triad_maxmean_bwd_workspace_bytes(Bq, Bv, Nq, Nv, D, dtype) : kCtrlBytes))

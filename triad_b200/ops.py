@@ -142,11 +142,21 @@ def maxmean_fwd(q: torch.Tensor, v: torch.Tensor, scale: torch.Tensor, T: torch.
     return clip, idx
 
 
+def _check_out(t: torch.Tensor, shape, dtype, name: str) -> None:
+    if t.dtype != dtype or tuple(t.shape) != tuple(shape) or not t.is_contiguous() or t.device.type != "cuda":
+        raise ValueError(f"{name} must be a contiguous {dtype} CUDA tensor of shape {tuple(shape)}")
+
+
 def maxmean_fwd_nonneg(q: torch.Tensor, v: torch.Tensor, scale: torch.Tensor, T: torch.Tensor, lo: float, coef: float,
-                       flags: int = 0):
+                       flags: int = 0, idx: Optional[torch.Tensor] = None, N: Optional[torch.Tensor] = None,
+                       sums: Optional[torch.Tensor] = None):
     """The max-mean forward AND N = dL/d<q,v> of the dense non-negative-pressure regulariser (coef * T * clamp'(S) * S
     for every token pair, bf16 [Bq*Nq, Bv*Nv]) from one pass over the similarities (triad_maxmean_fwd_nonneg).
-    Returns clip fp32 [Bq,Bv], idx, N, sums fp64 [2] = {sum clamp(S,lo,0)^2, sum dS*<q,v>}."""
+    Returns clip fp32 [Bq,Bv], idx, N, sums fp64 [2] = {sum clamp(S,lo,0)^2, sum dS*<q,v>}.
+
+    A caller that sweeps the images in chunks passes its own outputs: `idx` ([Bv, Bq*nq_padded(Nq)], e.g. the chunk's
+    rows of a whole-batch index buffer), `N` (a row-major [Bq*Nq, >= Bv*Nv] bf16 buffer reused across chunks: the
+    first Bv*Nv columns are written, the row pitch is N.stride(0)) and `sums` (fp64 [2], ADDED to)."""
     lib = _lib.load()
     _require_cuda(q, v, scale, T)
     if q.dtype != torch.bfloat16 or v.dtype != torch.bfloat16:
@@ -157,14 +167,22 @@ def maxmean_fwd_nonneg(q: torch.Tensor, v: torch.Tensor, scale: torch.Tensor, T:
     if D != D2:
         raise ValueError("embedding dims differ")
     clip = torch.empty(Bq, Bv, dtype=torch.float32, device=q.device)
-    idx = torch.empty(Bv, Bq * nq_padded(Nq), dtype=idx_dtype(Nv), device=q.device)
-    N = torch.empty(Bq * Nq, Bv * Nv, dtype=torch.bfloat16, device=q.device)
-    sums = torch.zeros(2, dtype=torch.float64, device=q.device)
+    if idx is None:
+        idx = torch.empty(Bv, Bq * nq_padded(Nq), dtype=idx_dtype(Nv), device=q.device)
+    _check_out(idx, (Bv, Bq * nq_padded(Nq)), idx_dtype(Nv), "idx")
+    if N is None:
+        N = torch.empty(Bq * Nq, Bv * Nv, dtype=torch.bfloat16, device=q.device)
+    if (N.dtype != torch.bfloat16 or N.dim() != 2 or N.shape[0] != Bq * Nq or N.shape[1] < Bv * Nv or N.stride(1) != 1
+            or N.device != q.device):
+        raise ValueError(f"N must be a row-major bf16 [{Bq * Nq}, >= {Bv * Nv}] tensor on {q.device}")
+    if sums is None:
+        sums = torch.zeros(2, dtype=torch.float64, device=q.device)
+    _check_out(sums, (2,), torch.float64, "sums")
     nws = lib.triad_maxmean_fwd_nonneg_workspace_bytes(Bq, Bv, Nq, Nv, D)
     with _on(q):
         ws = _Workspace.get(nws, q.device, "fwd")
         check(lib.triad_maxmean_fwd_nonneg(q.data_ptr(), v.data_ptr(), scale.data_ptr(), T.data_ptr(), Bq, Bv, Nq, Nv, D,
-                                           clip.data_ptr(), idx.data_ptr(), float(lo), float(coef), N.data_ptr(), Bv * Nv,
+                                           clip.data_ptr(), idx.data_ptr(), float(lo), float(coef), N.data_ptr(), N.stride(0),
                                            sums.data_ptr(), ws.data_ptr(), ws.numel(), int(flags), _stream(q.device)),
               "triad_maxmean_fwd_nonneg")
     return clip, idx, N, sums
@@ -193,8 +211,33 @@ def dense_grad_gemm(N: torch.Tensor, x: torch.Tensor, mode: int) -> torch.Tensor
     return out
 
 
+def dense_grad_gemm_f32(N: torch.Tensor, x: torch.Tensor, mode: int, out: torch.Tensor, accumulate: bool) -> torch.Tensor:
+    """dense_grad_gemm with an fp32 result written into `out` ([M, D] for mode 0, [Kc, D] for mode 1, contiguous —
+    a row slice of a larger buffer will do), or added to it when `accumulate` (triad_dense_grad_gemm_f32)."""
+    lib = _lib.load()
+    _require_cuda(N, x, out)
+    if N.dtype != torch.bfloat16 or x.dtype != torch.bfloat16 or N.dim() != 2 or x.dim() != 2:
+        raise TypeError("dense_grad_gemm_f32 takes 2-D bfloat16 matrices")
+    if N.stride(1) != 1:
+        raise ValueError("N must be row-major")
+    x = x.contiguous()
+    M, Kc = N.shape
+    D = x.shape[1]
+    if x.shape[0] != (Kc if mode == 0 else M):
+        raise ValueError("dense_grad_gemm_f32: inner dimensions differ")
+    _check_out(out, (M if mode == 0 else Kc, D), torch.float32, "out")
+    nws = lib.triad_dense_grad_gemm_workspace_bytes(M, Kc, D, int(mode))
+    with _on(N):
+        ws = _Workspace.get(nws, N.device, "dgemm")
+        check(lib.triad_dense_grad_gemm_f32(N.data_ptr(), N.stride(0), M, Kc, x.data_ptr(), D, int(mode), out.data_ptr(),
+                                            1 if accumulate else 0, ws.data_ptr(), ws.numel(), _stream(N.device)),
+              "triad_dense_grad_gemm_f32")
+    return out
+
+
 def maxmean_bwd(q, v, idx, g, clip, scale, T, need_dq=True, need_dv=True, need_dT=True, dv_f32=False,
-                flags: int = 0):
+                flags: int = 0, dv_out: Optional[torch.Tensor] = None):
+    """dv_out: write dv there (fp32 [Bv,Nv,D]) instead of a new tensor; with flags BWD_ACCUMULATE_DV it is added to."""
     lib = _lib.load()
     q, v, g = q.contiguous(), v.contiguous(), g.contiguous()
     if g.dtype != torch.float32:
@@ -203,8 +246,11 @@ def maxmean_bwd(q, v, idx, g, clip, scale, T, need_dq=True, need_dv=True, need_d
     Bv, Nv, _ = v.shape
     dt = _dtype_code(q)
     dq = torch.empty_like(q) if need_dq else None
-    dv = (torch.empty(Bv, Nv, D, dtype=torch.float32 if dv_f32 else v.dtype, device=v.device)
-          if need_dv else None)
+    if dv_out is not None:
+        _check_out(dv_out, (Bv, Nv, D), torch.float32, "dv_out")
+        need_dv, dv_f32 = True, True
+    dv = dv_out if dv_out is not None else (
+        torch.empty(Bv, Nv, D, dtype=torch.float32 if dv_f32 else v.dtype, device=v.device) if need_dv else None)
     dT = torch.empty((), dtype=torch.float32, device=q.device) if need_dT else None
     nws = lib.triad_maxmean_bwd_workspace_bytes(Bq, Bv, Nq, Nv, D, dt)
     with _on(q):
