@@ -278,6 +278,28 @@ int triad_project_tokens(const void* x, const void* w1, const float* b1, const f
 int triad_patch_compact(const void* x, const uint8_t* keep, int B, int N, int D, int elt_bytes, int max_len,
                         void* out, void* stream);
 
+/* Backward of triad_project_tokens (l2_normalize = 0) for gy = dLoss/dout, bf16 [M, Dout] (e.g. the dq / dv that
+ * triad_maxmean_bwd writes).  x, w1, b1, ln_g, ln_b, ln_eps and w2 are the forward's arguments (b2 is not needed).
+ * The hidden activations are recomputed from x with the forward's arithmetic (bit-identical LayerNorm statistics).
+ * Outputs, each optional (NULL skips it; dx / dw1 / dw2 skip their GEMM):
+ *   dx  bf16 [M, Din]      dw1 fp32 [512, Din]     db1 fp32 [512]
+ *   dln_g, dln_b fp32 [512]                        dw2 fp32 [Dout, 512]    db2 fp32 [Dout]
+ * Weight gradients are fp32 sums of fp32 products of bf16 operands (not rounded to bf16).  Deterministic: every
+ * reduction over tokens adds fixed partial sums in a fixed order, no float atomics.  Shapes as the forward:
+ * Din % 64 == 0, Dout % 16 == 0, Dout <= 512, any M >= 1.  x, w1, w2, gy, dx, dw1, dw2 and ws 16-byte aligned, the
+ * fp32 vectors 4-byte aligned.  ws: triad_project_tokens_bwd_workspace_bytes(M, Din, Dout) (it holds the bf16
+ * [M, 512] hidden gradient and LayerNorm output, about 2 KB per token). */
+size_t triad_project_tokens_bwd_workspace_bytes(int M, int Din, int Dout);
+int triad_project_tokens_bwd(const void* x, const void* w1, const float* b1, const float* ln_g, const float* ln_b,
+                             float ln_eps, const void* w2, const void* gy, int M, int Din, int Dout,
+                             void* dx, float* dw1, float* db1, float* dln_g, float* dln_b, float* dw2, float* db2,
+                             void* ws, size_t ws_bytes, void* stream);
+/* Backward of triad_patch_compact (same keep, B, N, D, elt_bytes, max_len): gx[b][n] = keep[b][n] ? gy[b][slot] : 0,
+ * where slot is patch n's position among image b's kept patches; gy [B, max_len, D], gx [B, N, D], one launch, no
+ * host synchronisation.  A pure copy: bit-identical to indexing gy. */
+int triad_patch_expand(const void* gy, const uint8_t* keep, int B, int N, int D, int elt_bytes, int max_len,
+                       void* gx, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

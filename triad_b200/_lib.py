@@ -78,6 +78,11 @@ SIGNATURES = {
     "triad_project_tokens": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_void_p,
                                      c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "triad_patch_compact": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "triad_project_tokens_bwd_workspace_bytes": (c_size_t, [c_int] * 3),
+    "triad_project_tokens_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_void_p,
+                                         c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                         c_void_p, c_void_p, c_size_t, c_void_p]),
+    "triad_patch_expand": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
 }
 
 _lib = None

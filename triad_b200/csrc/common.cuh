@@ -115,6 +115,11 @@ bool dq_pipe_supported(int Nv, int D, int dtype);
 int launch_dq_pipe(const void* v, const void* idx, const float* g, const float* row_scale, const float* Tp,
                    int Bq, int Bv, int Nq, int Nv, int D, void* dq, int* abort_flag,
                    const int* glist, const int* n_groups_dev, cudaStream_t st);
+// the projection head backward's products on the dense-gradient GEMM (dense_gemm.cu): mode 0 out[M][D] = N . x,
+// mode 1 out[Kc][D] = N^T . x, any D % 64 == 0 (512-column output slices), fp32 (out_f32) or bf16 out
+size_t head_gemm_workspace_bytes(int M, int Kc, int D, int mode);
+int launch_head_gemm(const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode, void* out,
+                     int out_f32, void* ws, size_t ws_bytes, cudaStream_t st);
 bool dq_tile_supported(int D, int dtype);
 int launch_dq_tile(const void* v, const void* idx, const float* g, const float* row_scale, const float* Tp,
                    int M, int Bv, int Nq, int Nv, int D, void* dq, cudaStream_t st);

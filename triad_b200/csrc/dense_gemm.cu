@@ -23,6 +23,11 @@
 // by the stores (the tensor maps carry the true extents).  triad_dense_grad_gemm_f32 differs in that second launch
 // only: it writes the fp32 sum, or adds it to the caller's fp32 output (an accumulator carried across image chunks, or
 // one chunk's rows of a per-rank dV partial).
+//
+// The projection head's backward (proj_head.cu) runs its three products on the same kernel through
+// launch_head_gemm: outputs wider than 512 columns are cut into 512-column slices (work item = row tile x slice x
+// K split), and the K splits are planned for few output tiles over a long K (the weight gradients: 1-4 tiles, K = the
+// token count).  A call with D <= 512 is one slice, so the public entry points run exactly as before.
 #include "common.cuh"
 #include "ptx.cuh"
 
@@ -52,7 +57,8 @@ struct Params {
     int kb_per_split;     // k-blocks per split (the last one may be shorter)
     int nkb;              // k-blocks in all
     int n_halves;         // 1 when D <= 256
-    int D;
+    int D;                // output columns in all
+    int n_slices;         // 512-column output slices (1 when D <= 512)
     int* abort_flag;
 };
 
@@ -85,7 +91,7 @@ dgemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
     const uint32_t cta_rank = cluster_ctarank();
     const bool is_leader = cta_rank == 0;
     const int cluster_id = blockIdx.x >> 1, n_clusters = gridDim.x >> 1;
-    const int n_items = p.n_tiles * p.splits;
+    const int n_items = p.n_tiles * p.n_slices * p.splits;
     constexpr uint32_t b_bytes = (uint32_t)kHalves * kBHalfBytes;
 
     if (warp == 0 && lane == 0) { prefetch_tmap(&tmap_a); prefetch_tmap(&tmap_b); prefetch_tmap(&tmap_c); }
@@ -107,7 +113,8 @@ dgemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
         const uint32_t full_sig = mapa(bar_full, 0);                  // every load signals the LEADER's barrier
         int s = 0; uint32_t ph = 0; bool ok = true;
         for (int it = cluster_id; it < n_items && ok; it += n_clusters) {
-            const int tile = it / p.splits, sp = it - tile * p.splits;
+            const int unit = it / p.splits, sp = it - unit * p.splits;
+            const int tile = unit / p.n_slices, col0 = (unit - tile * p.n_slices) * (2 * kHalfN);
             const int kb0 = sp * p.kb_per_split, kb1 = min(p.nkb, kb0 + p.kb_per_split);
             const int m0 = tile * kTileM + (int)cta_rank * kCtaM;
             for (int kb = kb0; kb < kb1; ++kb) {
@@ -124,7 +131,7 @@ dgemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
                     }
 #pragma unroll
                     for (int h = 0; h < kHalves; ++h) {
-                        const int n0 = h * kHalfN + (int)cta_rank * (kHalfN / 2);
+                        const int n0 = col0 + h * kHalfN + (int)cta_rank * (kHalfN / 2);
                         const uint32_t bs = st + kABytes + h * kBHalfBytes;
                         tma_load_2d<2>(bs, &tmap_b, full_sig + 8 * s, n0, kb * kBlockK);
                         tma_load_2d<2>(bs + kBoxBytes, &tmap_b, full_sig + 8 * s, n0 + 64, kb * kBlockK);
@@ -184,13 +191,15 @@ dgemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
         const uint32_t taddr = tmem0 + ((uint32_t)(quarter * 32) << 16);
         uint32_t tph = 0, nbox = 0; bool ok = true;
         for (int it = cluster_id; it < n_items && ok; it += n_clusters) {
-            const int tile = it / p.splits, sp = it - tile * p.splits;
+            const int unit = it / p.splits, sp = it - unit * p.splits;
+            const int tile = unit / p.n_slices, col0 = (unit - tile * p.n_slices) * (2 * kHalfN);
+            const int width = min(2 * kHalfN, p.D - col0);
             const int row0 = tile * kTileM + (int)cta_rank * kCtaM + quarter * 32;
             ok = mbar_wait(bar_t_full, tph, p.abort_flag, 34);
             ok = __all_sync(0xffffffffu, ok);
             if (!ok) break;
             tc_fence_after();
-            for (int c = 0; c * 32 < p.D; ++c, ++nbox) {
+            for (int c = 0; c * 32 < width; ++c, ++nbox) {
                 const uint32_t stg = stg_w + (nbox & 1u) * kStgPerWarp;
                 const uint32_t stg_row = stg + (uint32_t)lane * 128u;
                 uint32_t buf[32];
@@ -206,7 +215,7 @@ dgemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
                 __syncwarp();
                 if (lane == 0) {
                     asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-                                 ::"l"(reinterpret_cast<uint64_t>(&tmap_c)), "r"(stg), "r"(c * 32), "r"(row0), "r"(sp) : "memory");
+                                 ::"l"(reinterpret_cast<uint64_t>(&tmap_c)), "r"(stg), "r"(col0 + c * 32), "r"(row0), "r"(sp) : "memory");
                     asm volatile("cp.async.bulk.commit_group;" ::: "memory");
                 }
             }
@@ -275,16 +284,35 @@ int encode_tmap_f32_3d(CUtensorMap* map, const void* base, const cuuint64_t* dim
 
 using namespace triad;
 
-static int plan_splits(int M, int Kc, int mode, int* n_tiles, int* nkb, int* kb_per_split) {
+static int device_sms() {
     int dev = 0, sms = 148;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (sms < 2) sms = 2;
+    return sms < 2 ? 2 : sms;
+}
+
+static int plan_splits(int M, int Kc, int mode, int* n_tiles, int* nkb, int* kb_per_split) {
+    const int sms = device_sms();
     const int rows_out = mode == 0 ? M : Kc, K = mode == 0 ? Kc : M;
     *n_tiles = ceil_div(rows_out, dgemm::kTileM);
     *nkb = ceil_div(K, dgemm::kBlockK);
     int splits = dgemm::pick_splits(*n_tiles, *nkb, sms / 2);
     *kb_per_split = ceil_div(*nkb, splits);
     return ceil_div(*nkb, *kb_per_split);             // no empty split
+}
+
+// The head backward's plan: with fewer (row tile, column slice) units than CTA pairs (the weight gradients: K = the
+// token count, 1-4 units) the K range is cut so that every pair gets one item; otherwise the shared heuristic.
+static int plan_head_splits(int M, int Kc, int D, int mode, int* n_tiles, int* n_slices, int* nkb, int* kb_per_split) {
+    const int clusters = device_sms() / 2;
+    const int rows_out = mode == 0 ? M : Kc, K = mode == 0 ? Kc : M;
+    *n_tiles = ceil_div(rows_out, dgemm::kTileM);
+    *n_slices = ceil_div(D, 2 * dgemm::kHalfN);
+    *nkb = ceil_div(K, dgemm::kBlockK);
+    const int units = *n_tiles * *n_slices;
+    int splits = units >= clusters ? dgemm::pick_splits(units, *nkb, clusters) : clusters / units;
+    splits = max(1, min(splits, *nkb));
+    *kb_per_split = ceil_div(*nkb, splits);
+    return ceil_div(*nkb, *kb_per_split);
 }
 
 extern "C" size_t triad_dense_grad_gemm_workspace_bytes(int M, int Kc, int D, int mode) {
@@ -294,23 +322,24 @@ extern "C" size_t triad_dense_grad_gemm_workspace_bytes(int M, int Kc, int D, in
     return 256 + (size_t)splits * (size_t)(mode == 0 ? M : Kc) * (size_t)D * sizeof(float);
 }
 
-static int dense_grad_gemm_run(const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode,
-                               void* out, int out_kind, void* ws, size_t ws_bytes, void* stream) {
+namespace triad {
+size_t head_gemm_workspace_bytes(int M, int Kc, int D, int mode) {
+    int n_tiles, n_slices, nkb, kbs;
+    const int splits = plan_head_splits(M, Kc, D, mode, &n_tiles, &n_slices, &nkb, &kbs);
+    return 256 + (size_t)splits * (size_t)(mode == 0 ? M : Kc) * (size_t)D * sizeof(float);
+}
+}  // namespace triad
+
+// Launches the GEMM and the split reduction for a validated call and a plan in p (n_tiles, n_slices, splits,
+// kb_per_split, nkb).
+static int dgemm_launch(dgemm::Params p, const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode,
+                        void* out, int out_kind, void* ws, size_t ws_bytes, cudaStream_t st) {
     using namespace dgemm;
-    if (!n_mat || !x || !out || !ws) return fail_msg(TRIAD_ERR_BAD_ARG, "dense_grad_gemm: null pointer");
-    if (mode != 0 && mode != 1) return fail_msg(TRIAD_ERR_BAD_ARG, "dense_grad_gemm: mode");
-    if (M <= 0 || Kc <= 0 || D <= 0) return fail_msg(TRIAD_ERR_BAD_SHAPE, "dense_grad_gemm: bad shape");
-    if (D % 8 != 0 || D > 512 || ldn % 8 != 0 || ldn < Kc || (long long)ldn * 2 >= (1ll << 40))
-        return fail_msg(TRIAD_ERR_UNSUPPORTED, "dense_grad_gemm: needs D % 8 == 0, D <= 512, ldn % 8 == 0");
-    if (((uintptr_t)n_mat | (uintptr_t)x | (uintptr_t)out | (uintptr_t)ws) & 15) return fail_msg(TRIAD_ERR_ALIGNMENT, "dense_grad_gemm: 16-byte alignment");
-    cudaStream_t st = (cudaStream_t)stream;
     int dev = 0, sms = 0;
     TRIAD_CUDA_CHECK(cudaGetDevice(&dev));
     TRIAD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     const int rows_out = mode == 0 ? M : Kc;          // rows of the product
     const int K = mode == 0 ? Kc : M;                 // contraction length
-    Params p;
-    p.splits = plan_splits(M, Kc, mode, &p.n_tiles, &p.nkb, &p.kb_per_split);
     int n_clusters = sms / 2;
     p.n_halves = D > kHalfN ? 2 : 1;
     p.D = D;
@@ -348,7 +377,7 @@ static int dense_grad_gemm_run(const void* n_mat, long long ldn, int M, int Kc, 
         rc = encode_tmap_f32_3d(&mc, part, dims, strides, box);
         if (rc) return rc;
     }
-    const int n_items = p.n_tiles * p.splits;
+    const int n_items = p.n_tiles * p.n_slices * p.splits;
     if (n_clusters > n_items) n_clusters = n_items;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(n_clusters * 2));
@@ -379,6 +408,31 @@ static int dense_grad_gemm_run(const void* n_mat, long long ldn, int M, int Kc, 
     TRIAD_LAUNCH_CHECK("dense_grad_gemm reduce_kernel");
     return TRIAD_OK;
 }
+
+static int dense_grad_gemm_run(const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode,
+                               void* out, int out_kind, void* ws, size_t ws_bytes, void* stream) {
+    using namespace dgemm;
+    if (!n_mat || !x || !out || !ws) return fail_msg(TRIAD_ERR_BAD_ARG, "dense_grad_gemm: null pointer");
+    if (mode != 0 && mode != 1) return fail_msg(TRIAD_ERR_BAD_ARG, "dense_grad_gemm: mode");
+    if (M <= 0 || Kc <= 0 || D <= 0) return fail_msg(TRIAD_ERR_BAD_SHAPE, "dense_grad_gemm: bad shape");
+    if (D % 8 != 0 || D > 512 || ldn % 8 != 0 || ldn < Kc || (long long)ldn * 2 >= (1ll << 40))
+        return fail_msg(TRIAD_ERR_UNSUPPORTED, "dense_grad_gemm: needs D % 8 == 0, D <= 512, ldn % 8 == 0");
+    if (((uintptr_t)n_mat | (uintptr_t)x | (uintptr_t)out | (uintptr_t)ws) & 15) return fail_msg(TRIAD_ERR_ALIGNMENT, "dense_grad_gemm: 16-byte alignment");
+    Params p;
+    p.splits = plan_splits(M, Kc, mode, &p.n_tiles, &p.nkb, &p.kb_per_split);
+    p.n_slices = 1;
+    return dgemm_launch(p, n_mat, ldn, M, Kc, x, D, mode, out, out_kind, ws, ws_bytes, (cudaStream_t)stream);
+}
+
+namespace triad {
+// The projection head's products (arguments validated by triad_project_tokens_bwd): D % 64 == 0, any width
+int launch_head_gemm(const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode, void* out,
+                     int out_f32, void* ws, size_t ws_bytes, cudaStream_t st) {
+    dgemm::Params p;
+    p.splits = plan_head_splits(M, Kc, D, mode, &p.n_tiles, &p.n_slices, &p.nkb, &p.kb_per_split);
+    return dgemm_launch(p, n_mat, ldn, M, Kc, x, D, mode, out, out_f32 ? dgemm::kOutF32 : dgemm::kOutBf16, ws, ws_bytes, st);
+}
+}  // namespace triad
 
 extern "C" int triad_dense_grad_gemm(const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode,
                                      void* out, void* ws, size_t ws_bytes, void* stream) {

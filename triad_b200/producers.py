@@ -7,13 +7,15 @@ embedders and its patch dropout, each as one kernel.
     the forward is ONE launch of ``triad_project_tokens`` (tcgen05 GEMM -> LayerNorm epilogue -> tcgen05 GEMM ->
     bias / optional L2 normalisation), emitting the bf16 ``[B, N, D]`` K-major tensor the similarity kernel reads.
     The arithmetic follows the reference under autocast (bf16 GEMMs with fp32 accumulation, LayerNorm in fp32).
-    Backward (training): closed-form through the three layers with library GEMMs (plain matmuls; the hidden
-    activations are recomputed, not stored).
+    Backward (training): ``triad_project_tokens_bwd``: one tcgen05 row pass recomputes the hidden activations
+    from x (they are not stored) and writes the hidden gradient and the LayerNorm output, then the hand-written
+    dense-gradient GEMMs form dx and the fp32 weight gradients; only the gradients autograd asks for are computed.
 
 ``patch_dropout``  src/model.py:268-308 without its per-image Python loop: the same ``torch.bernoulli`` call (same
     random stream, so the same output for the same seed), then ``triad_patch_compact`` moves the kept patches to
     the front of every image and zero-fills the rest.  The one host synchronisation left is the one that sizes the
-    output (the batch's longest kept list), which the reference's ``max(...)`` needs too.
+    output (the batch's longest kept list), which the reference's ``max(...)`` needs too; the backward
+    (``triad_patch_expand``) has none.
 
 CUDA only, like the rest of the package: CPU tensors raise.
 """
@@ -52,42 +54,51 @@ def project_tokens(x: torch.Tensor, w1: torch.Tensor, b1: torch.Tensor, ln_g: to
     return out.view(*x.shape[:-1], Dout)
 
 
+def project_tokens_bwd(x, w1, b1, ln_g, ln_b, ln_eps, w2, gy, need):
+    """Raw call: gradients of ``project_tokens(..., normalize=False)`` for gy = dL/dout.  ``need`` is
+    (x, w1, b1, ln_g, ln_b, w2, b2) booleans; returns the seven gradients (None where not needed): dx bf16 shaped
+    like x, weight and bias gradients fp32."""
+    lib = _lib.load()
+    ops._require_cuda(x, w1, b1, ln_g, ln_b, w2, gy)
+    Din, Dout = x.shape[-1], w2.shape[0]
+    x2 = x.contiguous().view(-1, Din)
+    M = x2.shape[0]
+    gy2 = gy.to(torch.bfloat16).contiguous().view(M, Dout)
+    w1b, w2b = w1.detach().to(torch.bfloat16).contiguous(), w2.detach().to(torch.bfloat16).contiguous()
+    f32 = lambda t: t.detach().to(torch.float32).contiguous()                                         # noqa: E731
+    b1f, gf, bf = f32(b1), f32(ln_g), f32(ln_b)
+    dev = x.device
+    out = lambda want, *shape, dtype=torch.float32: torch.empty(*shape, dtype=dtype, device=dev) if want else None  # noqa: E731
+    dx = out(need[0], M, Din, dtype=torch.bfloat16)
+    dw1, db1, dg, db = out(need[1], HIDDEN, Din), out(need[2], HIDDEN), out(need[3], HIDDEN), out(need[4], HIDDEN)
+    dw2, db2 = out(need[5], Dout, HIDDEN), out(need[6], Dout)
+    ptr = lambda t: t.data_ptr() if t is not None else None                                          # noqa: E731
+    with ops._on(x):
+        ws = ops._Workspace.get(lib.triad_project_tokens_bwd_workspace_bytes(M, Din, Dout), dev, "project_bwd")
+        check(lib.triad_project_tokens_bwd(x2.data_ptr(), w1b.data_ptr(), b1f.data_ptr(), gf.data_ptr(), bf.data_ptr(),
+                                           float(ln_eps), w2b.data_ptr(), gy2.data_ptr(), M, Din, Dout,
+                                           ptr(dx), ptr(dw1), ptr(db1), ptr(dg), ptr(db), ptr(dw2), ptr(db2),
+                                           ws.data_ptr(), ws.numel(), ops._stream(dev)), "triad_project_tokens_bwd")
+    return (dx.view(x.shape) if dx is not None else None), dw1, db1, dg, db, dw2, db2
+
+
 class _ProjectFn(torch.autograd.Function):
-    """Forward: the fused kernel.  Backward: the chain rule through Linear -> LayerNorm -> Linear with library GEMMs
-    (the bf16 hidden activations are recomputed from x)."""
+    """Forward: the fused kernel.  Backward: ``triad_project_tokens_bwd`` (the hidden activations are recomputed
+    from x), computing only the gradients autograd asks for."""
 
     @staticmethod
     def forward(ctx, x, w1, b1, g, b, w2, b2, eps):
-        ctx.save_for_backward(x, w1, b1, g, b, w2)
+        ctx.save_for_backward(x, w1, b1, g, b, w2, b2)
         ctx.eps = eps
-        ctx.b2_dtype = b2.dtype
         return project_tokens(x, w1, b1, g, b, eps, w2, b2, normalize=False)
 
     @staticmethod
     def backward(ctx, gy):
-        x, w1, b1, g, b, w2 = ctx.saved_tensors
-        Din = x.shape[-1]
-        x2 = x.reshape(-1, Din)
-        gy2 = gy.reshape(-1, gy.shape[-1]).to(torch.bfloat16)
-        w1b, w2b = w1.to(torch.bfloat16), w2.to(torch.bfloat16)
-        h = (x2 @ w1b.t() + b1.to(torch.bfloat16)).float()                    # Linear 1 output (bf16-rounded), as fp32
-        mu = h.mean(dim=1, keepdim=True)
-        rstd = torch.rsqrt(h.var(dim=1, unbiased=False, keepdim=True) + ctx.eps)
-        xh = (h - mu) * rstd
-        ln = (xh * g.float() + b.float()).to(torch.bfloat16)
-        gw2 = gy2.t() @ ln                                                    # (Dout, 512)
-        gb2 = gy2.float().sum(dim=0)
-        gln = (gy2 @ w2b).float()                                             # (M, 512)
-        gg = (gln * xh).sum(dim=0)
-        gb = gln.sum(dim=0)
-        gxh = gln * g.float()
-        gh = (gxh - gxh.mean(dim=1, keepdim=True) - xh * (gxh * xh).mean(dim=1, keepdim=True)) * rstd
-        ghb = gh.to(torch.bfloat16)
-        gw1 = ghb.t() @ x2
-        gb1 = gh.sum(dim=0)
-        gx = (ghb @ w1b).view_as(x)
-        return (gx, gw1.to(w1.dtype), gb1.to(b1.dtype), gg.to(g.dtype), gb.to(b.dtype), gw2.to(w2.dtype),
-                gb2.to(ctx.b2_dtype), None)
+        x, w1, b1, g, b, w2, b2 = ctx.saved_tensors
+        need = ctx.needs_input_grad[:7]
+        grads = project_tokens_bwd(x, w1, b1, g, b, ctx.eps, w2, gy, need)
+        like = (x, w1, b1, g, b, w2, b2)
+        return tuple(d.to(t.dtype) if d is not None else None for d, t in zip(grads, like)) + (None,)
 
 
 class ProjectionHead(torch.nn.Module):
@@ -129,19 +140,29 @@ class _PatchCompact(torch.autograd.Function):
         with ops._on(x):
             check(lib.triad_patch_compact(x.data_ptr(), keep8.data_ptr(), B, N, D, x.element_size(), max_len, out.data_ptr(),
                                           ops._stream(x.device)), "triad_patch_compact")
-        ctx.save_for_backward(keep)
+        ctx.save_for_backward(keep8)
         ctx.n = N
         return out
 
     @staticmethod
     def backward(ctx, gy):
-        (keep,) = ctx.saved_tensors
-        B, L, D = gy.shape
-        pos = keep.cumsum(dim=1) - 1
-        gx = gy.new_zeros(B, ctx.n, D)
-        bi, ni = keep.nonzero(as_tuple=True)
-        gx[bi, ni] = gy[bi, pos[bi, ni]]
-        return gx, None, None
+        (keep8,) = ctx.saved_tensors
+        return patch_expand(gy, keep8, ctx.n), None, None
+
+
+def patch_expand(gy: torch.Tensor, keep: torch.Tensor, n: int) -> torch.Tensor:
+    """Backward of the compaction: (B, max_len, D) -> (B, n, D), row n of image b = gy[b, slot] where patch n is kept,
+    zero elsewhere.  One launch, no host synchronisation."""
+    lib = _lib.load()
+    ops._require_cuda(gy, keep)
+    B, L, D = gy.shape
+    gy = gy.contiguous()
+    keep8 = keep.to(torch.uint8).contiguous()
+    gx = torch.empty(B, n, D, dtype=gy.dtype, device=gy.device)
+    with ops._on(gy):
+        check(lib.triad_patch_expand(gy.data_ptr(), keep8.data_ptr(), B, n, D, gy.element_size(), L, gx.data_ptr(),
+                                     ops._stream(gy.device)), "triad_patch_expand")
+    return gx
 
 
 def patch_dropout(x: torch.Tensor, drop_rate: float, training: bool = True) -> torch.Tensor:
