@@ -10,7 +10,7 @@ import pytest
 import torch
 
 from triad_b200.producers import ProjectionHead, patch_dropout, patch_expand, project_tokens_bwd
-from tests.helpers import rel_err
+from tests.helpers import head_fp64_grads, rel_err
 
 NAMES = ("dx", "dw1", "db1", "dg", "db", "dw2", "db2")
 ALL = (True,) * 7
@@ -66,22 +66,6 @@ def _closed_form(x, w1, b1, g, b, w2, eps, gy):
     return gx, gw1.float(), gb1, gg, gb, gw2.float(), gb2
 
 
-def _round_bf16(t):
-    return t + (t.to(torch.bfloat16).double() - t).detach()
-
-
-def _fp64_reference(x, w1, b1, g, b, w2, b2, eps, gy):
-    """Autograd in fp64 of the autocast recipe: bf16 x / W1 / W2 / b1 / b2, h and ln rounded to bf16."""
-    leaves = [x.double(), w1.bfloat16().double(), b1.double(), g.double(), b.double(), w2.bfloat16().double(), b2.double()]
-    leaves = [t.detach().requires_grad_() for t in leaves]
-    xx, ww1, bb1, gg, bb, ww2, bb2 = leaves
-    h = _round_bf16(xx.reshape(-1, xx.shape[-1]) @ ww1.t() + _round_bf16(bb1))
-    ln = _round_bf16(torch.nn.functional.layer_norm(h, (h.shape[-1],), gg, bb, eps))
-    out = ln @ ww2.t() + _round_bf16(bb2)
-    out.backward(gy.reshape(out.shape).double())
-    return tuple(t.grad for t in leaves)
-
-
 SHAPES = [(4, 250, 768, 512), (3, 77, 768, 512), (2, 256, 384, 512), (1, 5, 64, 64), (2, 130, 1024, 256), (1, 1, 128, 16),
           (2, 300, 768, 320),
           (1, 1, 768, 512), (1, 127, 384, 64), (1, 129, 1536, 16), (3, 43, 1024, 320), (1, 129, 64, 512), (1, 127, 1536, 512)]
@@ -97,7 +81,7 @@ def test_head_backward_against_fp64(B, N, Din, Dout):
     eps = head.layer_norm.eps
     got = project_tokens_bwd(x, w1, b1, g, b, eps, w2, gy, ALL)
     cf = _closed_form(x, w1, b1, g, b, w2, eps, gy)
-    ref = _fp64_reference(x, w1, b1, g, b, w2, b2, eps, gy)
+    ref = head_fp64_grads(x, w1, b1, g, b, w2, b2, eps, gy)
     assert got[0].shape == x.shape and got[0].dtype == torch.bfloat16
     assert got[1].shape == (512, Din) and got[5].shape == (Dout, 512) and got[6].shape == (Dout,)
     for name, k, c, r in zip(NAMES, got, cf, ref):
