@@ -240,6 +240,21 @@ size_t triad_retrieve_workspace_bytes(int Nq, int n_img, int Nv, int D, int dtyp
 int triad_retrieve_scores(const void* q, int Nq, const void* gallery, int n_img, int Nv, int D,
                           int dtype, const float* temperature, int divide_by_T, int direction,
                           float* scores, void* ws, size_t ws_bytes, void* stream);
+/* ---- retrieval on an e4m3 gallery (opt-in compressed storage; direction 0 only) ------- */
+/* Per-row quantization: for each row x[0..D) of `x` ([rows][D], `dtype` fp32 or bf16)
+ *   s = fp32(max_k |x_k| / 448),  codes[k] = e4m3_rn_satfinite(fp32(x_k / s)) if s > 0, else 0;
+ * a row holding an inf or a NaN gets s = NaN.  codes [rows][D] (one e4m3 byte each), scales fp32 [rows].
+ * D % 16 == 0, D <= 512; x and codes 16-byte aligned. */
+int triad_quantize_e4m3(const void* x, int dtype, long long rows, int D, void* codes, float* scales, void* stream);
+/* scores[n] = sum_a fp32(m_a * t_a), m_a = max_p fp32(g_scales[n][p] * acc_ap), acc_ap = sum_k q_codes[a][k] *
+ * g_codes[n][p][k] (tensor cores, fp32 accumulation), t_a = fp32(fp32(q_scales[a] * (1/Nq)) * fp32(1/T)): the
+ * direction-0 retrieval score (mean over query tokens of max over patches, divided by T) of the quantized operands.
+ * q_codes [Nq][D], g_codes [n_img][Nv][D] as written by triad_quantize_e4m3; D in {128, 256, 384, 512}
+ * (TRIAD_ERR_UNSUPPORTED otherwise).  Deterministic; a watchdog timeout gives NaN scores. */
+size_t triad_retrieve_e4m3_workspace_bytes(int Nq, int n_img, int Nv, int D);
+int triad_retrieve_scores_e4m3(const void* q_codes, const float* q_scales, int Nq, const void* g_codes,
+                               const float* g_scales, int n_img, int Nv, int D, const float* temperature,
+                               float* scores, void* ws, size_t ws_bytes, void* stream);
 /* top-k of scores (descending, ties -> lower id first, like a stable argsort of -scores;
  * -0.0 and +0.0 are equal scores): out_scores fp32 [k] = scores[out_ids], bit for bit,
  * out_ids int32 [k].  NaN scores have no defined place.  ws: triad_topk_workspace_bytes(n). */

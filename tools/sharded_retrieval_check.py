@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """torchrun helper (>= 2 ranks, NCCL): gallery-sharded top-k (triad_b200.dist.sharded_retrieve_topk) against the
-single-GPU top-k over the whole gallery — ids bit-equal on every rank, uneven shards, ties across shards."""
+single-GPU top-k over the whole gallery — ids bit-equal on every rank, uneven shards, ties across shards.
+With --fp8 the gallery is an e4m3 Fp8Gallery and each rank scores its slice of it."""
 import os
 import sys
 
@@ -18,6 +19,7 @@ def main():
     dist.init_process_group("nccl", device_id=dev)
     from triad_b200 import retrieval as R
     from triad_b200.dist import sharded_retrieve_topk
+    fp8 = "--fp8" in sys.argv[1:]
     ok = True
     for n_img, Nv, Nq, k in ((1001, 256, 77, 10), (515, 1024, 250, 20), (3, 64, 5, 8)):
         g = torch.Generator(device=dev).manual_seed(17)                 # same gallery on every rank
@@ -27,11 +29,16 @@ def main():
         base, rem = n_img // world, n_img % world
         n_loc = base + (1 if rank < rem else 0)
         id0 = rank * base + min(rank, rem)
-        s, ids = sharded_retrieve_topk(q, gal[id0:id0 + n_loc].contiguous(), 1.5, k, id0)
+        if fp8:
+            gal = R.quantize_gallery(gal)
+            shard = gal[id0:id0 + n_loc]                                # a view: per-patch scales make slices exact
+        else:
+            shard = gal[id0:id0 + n_loc].contiguous()
+        s, ids = sharded_retrieve_topk(q, shard, 1.5, k, id0)
         kk = min(k, n_img)
         s0, i0 = R.retrieve_topk(q, gal, 1.5, kk)
         good = torch.equal(ids[:kk], i0.to(torch.int64)) and torch.equal(s[:kk], s0)
-        print(f"rank {rank}: n_img={n_img} Nv={Nv} Nq={Nq} k={k}: ids equal {good}", flush=True)
+        print(f"rank {rank}: {'fp8 ' if fp8 else ''}n_img={n_img} Nv={Nv} Nq={Nq} k={k}: ids equal {good}", flush=True)
         ok &= good
     flag = torch.tensor([1 if ok else 0], device=dev)
     dist.all_reduce(flag, op=dist.ReduceOp.MIN)

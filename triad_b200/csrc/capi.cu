@@ -234,3 +234,40 @@ extern "C" int triad_retrieve_scores(const void* q, int Nq, const void* gallery,
     if (rc) return rc;
     return fwd_impl(gallery, q, rs, temperature, divide_by_T, n_img, 1, Nv, Nq, D, dtype, scores, nullptr, fws, fws_bytes, 0, st);
 }
+
+// ---------------------------------------------------------------------------------------------
+// retrieval scores on an e4m3 gallery (direction 0, divides by T)
+// workspace: row weights [Nq] | [0,256) control | partial sums
+// ---------------------------------------------------------------------------------------------
+extern "C" size_t triad_retrieve_e4m3_workspace_bytes(int Nq, int n_img, int Nv, int D) {
+    (void)Nv; (void)D;
+    if (Nq <= 0 || n_img <= 0) return 0;
+    return align_up((size_t)Nq * 4, 256) + 256 + fwd_part_bytes(Nq, n_img, Nq);
+}
+
+extern "C" int triad_retrieve_scores_e4m3(const void* q_codes, const float* q_scales, int Nq, const void* g_codes,
+                                          const float* g_scales, int n_img, int Nv, int D, const float* temperature,
+                                          float* scores, void* ws, size_t ws_bytes, void* stream) {
+    if (!q_codes || !q_scales || !g_codes || !g_scales || !temperature || !scores || !ws)
+        return fail_msg(TRIAD_ERR_BAD_ARG, "retrieve_scores_e4m3: null pointer");
+    if (Nq <= 0 || n_img <= 0 || Nv <= 0 || D <= 0 || Nv > 65535)
+        return fail_msg(TRIAD_ERR_BAD_SHAPE, "retrieve_scores_e4m3: bad shape (need Nq, n_img >= 1, 1 <= Nv <= 65535)");
+    if (!tc_e4m3_supported(Nv, D)) return fail_msg(TRIAD_ERR_UNSUPPORTED, "retrieve_scores_e4m3: needs D % 128 == 0, D <= 512");
+    if ((((uintptr_t)q_codes | (uintptr_t)g_codes | (uintptr_t)ws) & 15) ||
+        (((uintptr_t)q_scales | (uintptr_t)g_scales | (uintptr_t)scores) & 3))
+        return fail_msg(TRIAD_ERR_ALIGNMENT, "retrieve_scores_e4m3: codes and ws 16-byte aligned, scales and scores 4-byte aligned");
+    if (ws_bytes < triad_retrieve_e4m3_workspace_bytes(Nq, n_img, Nv, D))
+        return fail_msg(TRIAD_ERR_WORKSPACE, "retrieve_scores_e4m3: workspace too small");
+    cudaStream_t st = (cudaStream_t)stream;
+    float* rs = (float*)ws;
+    char* fws = (char*)ws + align_up((size_t)Nq * 4, 256);
+    int* abort_flag = (int*)fws;
+    float* part = (float*)(fws + 256);
+    TRIAD_CUDA_CHECK(cudaMemsetAsync(abort_flag, 0, 256, st));
+    int rc = launch_row_scale(nullptr, 1, Nq, rs, st);
+    if (rc) return rc;
+    rc = launch_maxmean_tc_e4m3(q_codes, q_scales, g_codes, g_scales, rs, temperature, Nq, n_img, Nq, Nv, D, part,
+                                abort_flag, st);
+    if (rc) return rc;
+    return launch_finalize_clip(part, 1, n_img, Nq, scores, abort_flag, st);
+}

@@ -109,6 +109,14 @@ int launch_finalize_clip_packed(const float* part, const int* pack_off, int Bq, 
 // - (group of the query's first packed row); a query of <= Nq kept rows spans at most (Nq+30)/32 + 1 groups
 static inline int packed_pieces(int Nq) { return (Nq + 30) / 32 + 1; }
 bool tc_supported(int Nv, int D);
+// e4m3 retrieval forward (maxmean_tc.cu, kFp8): q_codes [M][D], g_codes [Bv][Nv][D] (e4m3 bytes), q_scale [M],
+// g_scale [Bv][Nv]; divides by T; no idx.  D in {128, 256, 384, 512}
+bool tc_e4m3_supported(int Nv, int D);
+int launch_maxmean_tc_e4m3(const void* q_codes, const float* q_scale, const void* g_codes, const float* g_scale,
+                           const float* row_scale, const float* T, int M, int Bv, int Nq, int Nv, int D,
+                           float* part, int* abort_flag, cudaStream_t st);
+// rows x D (fp32 or bf16) -> e4m3 codes [rows][D] + one fp32 scale per row (quant_e4m3.cu); D % 16 == 0, D <= 512
+int launch_quantize_e4m3(const void* x, int dtype, long long rows, int D, void* codes, float* scales, cudaStream_t st);
 // tiled dQ of the backward, bf16 only.  Nv <= 256 (uint8 winners): the software-pipelined shared-memory gather
 // (bwd_dq_pipe.cu); Nv > 256 (uint16 winners): the L1-resident gather (bwd_dq_tile.cu)
 bool dq_pipe_supported(int Nv, int D, int dtype);

@@ -32,6 +32,7 @@
 #include "ptx.cuh"
 
 #include <cuda.h>
+#include <string.h>
 
 namespace triad {
 namespace tc {
@@ -82,6 +83,9 @@ struct Params {
     int write_n;             // 0: value only
     double* n_partials;      // [gridDim.x*8][2]: sum clamp^2, sum dS*<q,v>; slot blockIdx.x*8 + (warp - 4), written by the
                              // emission warps 8-11 (slots of the other epilogue warps stay as cleared)
+    // kFp8 (e4m3 retrieval): per-patch scales [Bv][Nv] of the gallery codes, per-token scales [M] of the query codes
+    const float* col_scale;
+    const float* q_scale;
 };
 
 __device__ __forceinline__ float fmax3(float a, float b, float c) { return fmaxf(fmaxf(a, b), c); }
@@ -104,6 +108,35 @@ __device__ __forceinline__ float chunk_max32(const uint32_t (&r)[32], int col0, 
         m[k] = fmaxf(m[k], v[8 * k + 7]);
     }
     return fmaxf(fmax3(m[0], m[1], m[2]), m[3]);
+}
+
+// maximum that returns NaN when either operand is NaN (fmaxf drops it): a NaN patch scale must reach the score
+__device__ __forceinline__ float fmax_nan(float a, float b) {
+    float r;
+    asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+    return r;
+}
+// e4m3 epilogue: maximum over one 32-column chunk of sg[c] * acc[c], the patch scales sg of the chunk's columns read
+// from shared memory (the same address in every lane: a broadcast); columns >= Nv do not take part, a NaN product does.
+// Scaled and reduced four columns at a time, so the products never occupy a second 32-register buffer.
+__device__ __forceinline__ float chunk_max32_scaled(const uint32_t (&r)[32], const float4* sg, int col0, int Nv) {
+    const bool part = col0 + 32 > Nv;
+    float m[4];
+#pragma unroll
+    for (int g = 0; g < 8; ++g) {
+        const float4 s = sg[g];
+        float v0 = __uint_as_float(r[4 * g]) * s.x, v1 = __uint_as_float(r[4 * g + 1]) * s.y;
+        float v2 = __uint_as_float(r[4 * g + 2]) * s.z, v3 = __uint_as_float(r[4 * g + 3]) * s.w;
+        if (part) {
+            if (col0 + 4 * g >= Nv) v0 = -INFINITY;
+            if (col0 + 4 * g + 1 >= Nv) v1 = -INFINITY;
+            if (col0 + 4 * g + 2 >= Nv) v2 = -INFINITY;
+            if (col0 + 4 * g + 3 >= Nv) v3 = -INFINITY;
+        }
+        const float a = fmax_nan(fmax_nan(v0, v1), fmax_nan(v2, v3));
+        m[g & 3] = g < 4 ? a : fmax_nan(m[g & 3], a);                // four independent chains
+    }
+    return fmax_nan(fmax_nan(m[0], m[1]), fmax_nan(m[2], m[3]));
 }
 
 // best = lowest column of this chunk with value >= theta, if any (columns >= Nv never qualify)
@@ -302,11 +335,19 @@ struct TileIter {
 // the dense regulariser (emission warps 8-11 write N = dL/d<q,v> of the non-negative pressure term) in one pass over
 // the similarities — the training step with the reference's full loss needs both of the very same tiles; 1: kMode 2
 // without the max-mean warps (the regulariser-only pass).
-template <int kCtaGroup, bool kSub, int kMode = 0>
+// kFp8: e4m3 operands (kMode 0, no idx: the retrieval forward on a quantized gallery).  A 128-byte swizzle row then
+// holds 128 elements, so a k-block is 128 wide (num_kb = D/128 <= 4) and one kind::f8f6f4 MMA step covers K = 32;
+// the ring, the descriptors and the issue loops are those of bf16.  The epilogue multiplies every column by its
+// patch scale before the max and the row by t_a = fp32(fp32(q_scale * row_scale) * (1/T)) after it.  The scales of
+// the current 256-patch sub-tile are staged per epilogue warp in the upper half of the query region (num_kb <= 4
+// leaves it unused).
+template <int kCtaGroup, bool kSub, int kMode = 0, bool kFp8 = false>
 __global__ void __launch_bounds__(kEmitThreads, 1)
 maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_v,
                   const __grid_constant__ CUtensorMap tmap_n, const Params p) {
+    static_assert(!kFp8 || kMode == 0, "the e4m3 forward is the max-mean reduction only");
     constexpr bool kEmitN = kMode != 0;
+    constexpr int kKbElems = kFp8 ? 128 : kBlockK;                          // elements per 128-byte k-block row
     constexpr int kVStageBytes = (kMaxN / kCtaGroup) * kBlockK * 2;       // 32 KB / 16 KB
     // the dense-regulariser modes give the last 32 KB of the ring to the epilogue's store staging: four emission warps x
     // two 4 KB boxes (32 rows x 64 columns).  (Two 2 KB boxes of 32 columns per emission warp, i.e. 5 ring stages
@@ -390,7 +431,7 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
                         if (new_m && sb == 0 && issuer) {
                             if (is_leader) mbar_expect_tx(bar_q_full + 8 * kb, kQkbBytes * kCtaGroup);
                             tma_load_2d<kCtaGroup>(q_smem + kb * kQkbBytes, &tmap_q, q_full_sig + 8 * kb,
-                                                   kb * kBlockK, t.m * kTileRows + (int)cta_rank * kBlockM);
+                                                   kb * kKbElems, t.m * kTileRows + (int)cta_rank * kBlockM);
                         }
                         ok = mbar_wait(bar_v_empty + 8 * stage, phase ^ 1, p.abort_flag, 2);
                         if (!ok) break;
@@ -398,7 +439,7 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
                             if (is_leader) mbar_expect_tx(bar_v_full + 8 * stage, v_tx_bytes * kCtaGroup);
                             // patches beyond Nv (last sub-tile) are zero-filled by TMA and masked in the epilogue
                             tma_load_3d<kCtaGroup>(v_smem + stage * kVStageBytes, &tmap_v, v_full_sig + 8 * stage,
-                                                   kb * kBlockK, sb * kMaxN + (int)cta_rank * n_half, t.j);
+                                                   kb * kKbElems, sb * kMaxN + (int)cta_rank * n_half, t.j);
                         }
                         __syncwarp();
                         if (++stage == kStages) { stage = 0; phase ^= 1; }
@@ -415,7 +456,7 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
         // the issuing thread, not the tensor pipe, set the pace: ncu showed it busy 85 % of the time.)
         if (is_leader) {
             const bool issuer = elect_one();
-            const uint32_t idesc = make_idesc(kTileRows, p.n_umma);
+            const uint32_t idesc = kFp8 ? make_idesc_e4m3(kTileRows, p.n_umma) : make_idesc(kTileRows, p.n_umma);
             const uint32_t tmem0 = __shfl_sync(0xffffffffu, tmem_base, 0);
             const uint64_t a_desc0 = make_smem_desc(q_smem);
             const uint64_t b_desc0 = make_smem_desc(v_smem);
@@ -441,8 +482,12 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
                     if (issuer) {
 #pragma unroll
                         for (int k = 0; k < kBlockK / kUmmaK; ++k) {
-                            // +32 bytes per K=16 step inside the 128-byte swizzle row (address field is >>4)
-                            umma_bf16<kCtaGroup>(d_tmem, a_desc + 2u * k, b_desc + 2u * k, idesc, (uint32_t)((kb | k) != 0));
+                            // +32 bytes per K=16 (bf16) / K=32 (e4m3) step inside the 128-byte swizzle row (address
+                            // field is >>4)
+                            if constexpr (kFp8)
+                                umma_e4m3<kCtaGroup>(d_tmem, a_desc + 2u * k, b_desc + 2u * k, idesc, (uint32_t)((kb | k) != 0));
+                            else
+                                umma_bf16<kCtaGroup>(d_tmem, a_desc + 2u * k, b_desc + 2u * k, idesc, (uint32_t)((kb | k) != 0));
                         }
                         umma_commit<kCtaGroup>(bar_v_empty + 8 * stage);      // frees the V stage in both CTAs
                     }
@@ -593,6 +638,7 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             if (t.m != prev_m) {
                 r_orig = (r < M_eff) ? (p.pack_off ? p.rowmap[r] : r) : -1;
                 rs = (r_orig >= 0) ? p.row_scale[r_orig] : 0.f;
+                if constexpr (kFp8) { if (r_orig >= 0) rs = (p.q_scale[r_orig] * rs) * Tval; }     // t_a
                 qi = (r_orig >= 0) ? r_orig / p.Nq : 0x7fffffff;
                 idx_off = (r_orig >= 0) ? (size_t)qi * p.nq_pad + (r_orig - qi * p.Nq) : 0;
                 if (p.pack_off && r_orig >= 0) piece = (row0 >> 5) - (p.pack_off[qi] >> 5);
@@ -600,6 +646,21 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             }
           for (int sb = 0; sb < n_sub; ++sb, ++t_cnt) {
             const uint32_t acc = t_cnt & 1u, acc_phase = (t_cnt >> 1) & 1u;
+            // e4m3: this sub-tile's 256 patch scales into the warp's slot (lane l: columns 8l .. 8l+7), loaded
+            // while the MMAs run; 0 beyond the last patch (those columns are masked anyway)
+            const uint32_t sg_smem = q_smem + 4u * kQkbBytes + (uint32_t)quarter * 1024u;
+            const float4* sg_gen = reinterpret_cast<const float4*>(smem_gen + (sg_smem - smem_base));
+            if constexpr (kFp8) {
+                const int c0 = sb * kMaxN + 8 * lane;
+                const float* src = p.col_scale + (size_t)t.j * p.Nv;
+                uint32_t s[8];
+#pragma unroll
+                for (int e = 0; e < 8; ++e) s[e] = __float_as_uint(c0 + e < p.Nv ? __ldg(src + c0 + e) : 0.f);
+                __syncwarp();                                 // every lane is done with the previous sub-tile's scales
+                sts128(sg_smem + (uint32_t)lane * 32u, s[0], s[1], s[2], s[3]);
+                sts128(sg_smem + (uint32_t)lane * 32u + 16u, s[4], s[5], s[6], s[7]);
+                __syncwarp();
+            }
             bool ok = mbar_wait(bar_t_full + 8 * acc, acc_phase, p.abort_flag, 6);
             ok = __all_sync(0xffffffffu, ok);
             if (!ok) { alive = false; break; }
@@ -613,7 +674,21 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             //      are masked by Nv — which keeps every load unconditional (see tmem_ld32_raw). ----
             constexpr int kCh = kMaxN / 32;
             float mx = -INFINITY;
-            {
+            if constexpr (kFp8) {
+                // the same loads; every column scaled by its patch scale before the (NaN-propagating) max
+                uint32_t bufA[32], bufB[32];
+                tmem_ld32_raw(taddr, bufA);
+                tmem_wait_ld();
+#pragma unroll
+                for (int c = 0; c < kCh; c += 2) {
+                    tmem_ld32_raw(taddr + (c + 1) * 32, bufB);
+                    mx = fmax_nan(mx, chunk_max32_scaled(bufA, sg_gen + 8 * c, c * 32, Nv));
+                    tmem_wait_ld();
+                    if (c + 2 < kCh) tmem_ld32_raw(taddr + (c + 2) * 32, bufA);          // compile-time condition
+                    mx = fmax_nan(mx, chunk_max32_scaled(bufB, sg_gen + 8 * (c + 1), (c + 1) * 32, Nv));
+                    tmem_wait_ld();
+                }
+            } else {
                 uint32_t bufA[32], bufB[32];
                 tmem_ld32_raw(taddr, bufA);
                 tmem_wait_ld();
@@ -628,14 +703,16 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
                 }
             }
             float R;
-            const float theta = argmax_threshold<true>(mx, Tval, &R);
+            float theta = 0.f;
+            if constexpr (kFp8) R = mx;
+            else theta = argmax_threshold<true>(mx, Tval, &R);
 
             // ---- pass 2: first column whose accumulator reaches the threshold (the reference's first-index
             //      argmax).  Same pipelined loads, walking the chunks from the last to the first so the lowest
             //      qualifying column is the one that sticks; inside a chunk four independent 8-column
             //      compare/select chains instead of one 256-long dependent chain. ----
             int best = (int)kNoCol;
-            if (p.idx != nullptr) {
+            if (!kFp8 && p.idx != nullptr) {
                 constexpr int kHalfCh = kSolo ? kCh : kCh / 2;
                 const int cb = kSolo ? 0 : half * kHalfCh;       // this warp's chunks: [cb, cb + kHalfCh)
                 uint32_t bufA[32], bufB[32];
@@ -674,7 +751,8 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             if (half == 1) continue;                             // the lower-half warp owns the outputs
             // Equal rounded maxima in two sub-tiles: the earlier one holds the first index (torch.max), and
             // inside a sub-tile `best` already is the first column of that rounded value.
-            if (sb == 0 || R > R_run) { R_run = R; best_run = best + sb * kMaxN; }
+            if constexpr (kFp8) R_run = sb == 0 ? R : fmax_nan(R_run, R);
+            else if (sb == 0 || R > R_run) { R_run = R; best_run = best + sb * kMaxN; }
           }
             if (!alive) break;
             if (half == 1) continue;
@@ -756,10 +834,52 @@ static int encode_map(CUtensorMap* map, const void* base, int rank, const cuuint
     return encode_tmap_bf16(map, base, rank, dims, strides, box, true);
 }
 
-template <int kCtaGroup, bool kSub, int kMode = 0>
+// uint8 (e4m3 codes) tiled tensor map, SWIZZLE_128B: 128-element (128-byte) inner box
+static int encode_map_u8(CUtensorMap* map, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
+                         const cuuint32_t* box) {
+    PFN_tmapEncodeTiled fn = get_encode_fn();
+    if (!fn) return fail_msg(TRIAD_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
+    cuuint32_t estr[3] = {1, 1, 1};
+    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, (cuuint32_t)rank, const_cast<void*>(base), dims, strides, box, estr,
+                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+        char buf[96];
+        snprintf(buf, sizeof buf, "cuTensorMapEncodeTiled (uint8) failed (CUresult %d)", (int)r);
+        return fail_msg(TRIAD_ERR_CUDA, buf);
+    }
+    return TRIAD_OK;
+}
+
+// Tile order (TileIter).  V up to ~48 MB: any order, V stays in L2.  Larger: if there are enough query tiles to
+// give every cluster a few items per ~16 MB image chunk, ALL clusters walk the same chunk at the same time —
+// V is read from HBM once per pass whatever its size (cfg 4: 2.1 GB), and even at cfg 2 (67 MB, nominally
+// L2-sized) the hot set shrinks from V + Q to one chunk + the query tiles (measured 3.34 -> 3.17 ms).
+// Otherwise (retrieval: one or a few query tiles against a huge gallery) each cluster keeps to its own images
+// and runs all query tiles against a handful of them back to back, so the re-reads hit L2.
+// img_bytes = Nv * D * element size.
+static void pick_tile_order(Params& p, size_t img_bytes, int Bv, int n_m, int n_clusters) {
+    const size_t v_bytes = (size_t)Bv * img_bytes;
+    p.C = Bv;
+    p.sync = 0;
+    if (v_bytes > (size_t)48 << 20) {
+        size_t c16 = ((size_t)16 << 20) / img_bytes;
+        if (c16 < 1) c16 = 1;
+        if ((size_t)n_m * c16 >= (size_t)4 * n_clusters) {
+            p.C = (int)(c16 > (size_t)Bv ? (size_t)Bv : c16);
+            p.sync = 1;
+        } else {
+            size_t c = ((size_t)48 << 20) / ((size_t)n_clusters * img_bytes);
+            p.C = (int)(c < 1 ? 1 : (c > 64 ? 64 : c));
+            if (p.C > Bv) p.C = Bv;
+        }
+    }
+}
+
+template <int kCtaGroup, bool kSub, int kMode = 0, bool kFp8 = false>
 static int launch_t(const CUtensorMap& mq, const CUtensorMap& mv, const CUtensorMap& mn, const Params& p, int n_clusters,
                     cudaStream_t st) {
-    auto kern = maxmean_tc_kernel<kCtaGroup, kSub, kMode>;
+    auto kern = maxmean_tc_kernel<kCtaGroup, kSub, kMode, kFp8>;
     TRIAD_SET_MAX_SMEM(kern, kSmemBytes);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(n_clusters * kCtaGroup));
@@ -804,29 +924,8 @@ int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, cons
     p.idx16 = Nv > 256;
     p.num_kb = D / kBlockK;
     p.n_m = n_m;
-    // Tile order (TileIter).  V up to ~48 MB: any order, V stays in L2.  Larger: if there are enough query tiles to
-    // give every cluster a few items per ~16 MB image chunk, ALL clusters walk the same chunk at the same time —
-    // V is read from HBM once per pass whatever its size (cfg 4: 2.1 GB), and even at cfg 2 (67 MB, nominally
-    // L2-sized) the hot set shrinks from V + Q to one chunk + the query tiles (measured 3.34 -> 3.17 ms).
-    // Otherwise (retrieval: one or a few query tiles against a huge gallery) each cluster keeps to its own images
-    // and runs all query tiles against a handful of them back to back, so the re-reads hit L2.
-    const size_t img_bytes = (size_t)Nv * D * 2;
-    const size_t v_bytes = (size_t)Bv * img_bytes;
     int n_clusters = sms / cta_group;
-    p.C = Bv;
-    p.sync = 0;
-    if (v_bytes > (size_t)48 << 20) {
-        size_t c16 = ((size_t)16 << 20) / img_bytes;
-        if (c16 < 1) c16 = 1;
-        if ((size_t)n_m * c16 >= (size_t)4 * n_clusters) {
-            p.C = (int)(c16 > (size_t)Bv ? (size_t)Bv : c16);
-            p.sync = 1;
-        } else {
-            size_t c = ((size_t)48 << 20) / ((size_t)n_clusters * img_bytes);
-            p.C = (int)(c < 1 ? 1 : (c > 64 ? 64 : c));
-            if (p.C > Bv) p.C = Bv;
-        }
-    }
+    pick_tile_order(p, (size_t)Nv * D * 2, Bv, n_m, n_clusters);
     if (flags & TRIAD_FWD_SYNC_CHUNKS) { p.C = Bv < 3 ? Bv : 3; p.sync = 1; }     // tests: tiny chunks on small shapes
     PartLayout pl = part_layout(M, Nq);
     p.G = pl.G; p.S = pl.S;
@@ -838,6 +937,7 @@ int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, cons
     p.rowmap = pack_maps ? pack_maps + p.Bq + 1 : nullptr;
     p.pieces = packed_pieces(Nq);
     p.n_out = nullptr; p.ldn = 0; p.lo = 0.f; p.coef = 0.f; p.write_n = 0; p.n_partials = nullptr;
+    p.col_scale = nullptr; p.q_scale = nullptr;
     if (emit) {
         if (n_sub > 1 || Nv % 8 != 0 || pack_maps) return fail_msg(TRIAD_ERR_UNSUPPORTED, "dense-regulariser forward: needs Nv <= 256, Nv % 8 == 0");
         if (emit->with_maxmean && (!idx || !part || inv_T)) return fail_msg(TRIAD_ERR_BAD_ARG, "dense-regulariser + max-mean forward: needs idx and the partial buffer");
@@ -882,6 +982,65 @@ int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, cons
     }
     if (n_sub > 1) return cta_group == 2 ? launch_t<2, true>(mq, mv, mn, p, n_clusters, st) : launch_t<1, true>(mq, mv, mn, p, n_clusters, st);
     return cta_group == 2 ? launch_t<2, false>(mq, mv, mn, p, n_clusters, st) : launch_t<1, false>(mq, mv, mn, p, n_clusters, st);
+}
+
+bool tc_e4m3_supported(int Nv, int D) { return Nv >= 1 && Nv <= 65535 && D % 128 == 0 && D >= 128 && D <= 512; }
+
+int launch_maxmean_tc_e4m3(const void* q_codes, const float* q_scale, const void* g_codes, const float* g_scale,
+                           const float* row_scale, const float* T, int M, int Bv, int Nq, int Nv, int D,
+                           float* part, int* abort_flag, cudaStream_t st) {
+    using namespace tc;
+    if (!tc_e4m3_supported(Nv, D)) return fail_msg(TRIAD_ERR_UNSUPPORTED, "tcgen05 e4m3 forward: needs D in {128, 256, 384, 512}");
+    // one row tile of <= 128 tokens: cta_group::1, as for bf16 (fwd_impl)
+    const int cta_group = M <= 128 ? 1 : 2;
+    const int tile_rows = kBlockM * cta_group;
+    const int n_m = ceil_div(M, tile_rows);
+    const int n_sub = ceil_div(Nv, kMaxN);
+    if ((long long)n_m * Bv * n_sub >= 0x7fffffffLL) return fail_msg(TRIAD_ERR_UNSUPPORTED, "tcgen05 e4m3 forward: too many tiles");
+
+    int dev = 0, sms = 0;
+    TRIAD_CUDA_CHECK(cudaGetDevice(&dev));
+    TRIAD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+
+    Params p;
+    memset(&p, 0, sizeof p);
+    p.M = M; p.Bv = Bv; p.Nq = Nq; p.Nv = Nv;
+    p.n_umma = n_sub > 1 ? kMaxN : (Nv + 15) / 16 * 16;
+    p.n_sub = n_sub;
+    p.num_kb = D / 128;
+    p.n_m = n_m;
+    int n_clusters = sms / cta_group;
+    pick_tile_order(p, (size_t)Nv * D, Bv, n_m, n_clusters);      // an e4m3 image is Nv*D bytes
+    PartLayout pl = part_layout(M, Nq);
+    p.G = pl.G; p.S = pl.S;
+    p.nq_pad = nq_padded(Nq);
+    p.inv_T = 1;                                                    // retrieval divides by T
+    p.row_scale = row_scale; p.T = T; p.part = part; p.idx = nullptr; p.abort_flag = abort_flag;
+    p.Bq = M / Nq;
+    p.pieces = packed_pieces(Nq);
+    p.col_scale = g_scale; p.q_scale = q_scale;
+
+    CUtensorMap mq, mv;
+    {
+        cuuint64_t dims[2] = {(cuuint64_t)D, (cuuint64_t)M};
+        cuuint64_t strides[1] = {(cuuint64_t)D};
+        cuuint32_t box[2] = {128u, (cuuint32_t)kBlockM};
+        int rc = encode_map_u8(&mq, q_codes, 2, dims, strides, box);
+        if (rc) return rc;
+    }
+    {
+        cuuint64_t dims[3] = {(cuuint64_t)D, (cuuint64_t)Nv, (cuuint64_t)Bv};
+        cuuint64_t strides[2] = {(cuuint64_t)D, (cuuint64_t)Nv * D};
+        cuuint32_t box[3] = {128u, (cuuint32_t)(p.n_umma / cta_group), 1};
+        int rc = encode_map_u8(&mv, g_codes, 3, dims, strides, box);
+        if (rc) return rc;
+    }
+    const long long total = (long long)n_m * Bv;
+    if ((long long)n_clusters > total) n_clusters = (int)total;
+    if (n_clusters < 1) n_clusters = 1;
+    if (n_sub > 1)
+        return cta_group == 2 ? launch_t<2, true, 0, true>(mq, mv, mq, p, n_clusters, st) : launch_t<1, true, 0, true>(mq, mv, mq, p, n_clusters, st);
+    return cta_group == 2 ? launch_t<2, false, 0, true>(mq, mv, mq, p, n_clusters, st) : launch_t<1, false, 0, true>(mq, mv, mq, p, n_clusters, st);
 }
 
 }  // namespace triad

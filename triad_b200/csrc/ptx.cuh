@@ -107,6 +107,22 @@ __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint
             ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
     }
 }
+// D[tmem] (+)= A[smem] * B[smem]^T, e4m3 x e4m3 -> fp32 (K = 32 per instruction: the same 32 bytes of a 128-byte
+// swizzle row as one bf16 K = 16 step, so the descriptors and their per-step advance are those of umma_bf16)
+template <int kCtaGroup>
+__device__ __forceinline__ void umma_e4m3(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
+    if constexpr (kCtaGroup == 1) {
+        asm volatile(
+            "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+            "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}"
+            ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
+    } else {
+        asm volatile(
+            "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+            "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}"
+            ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
+    }
+}
 // One lane of a fully active warp (the lowest): lets a WHOLE warp run a role's loop with warp-uniform control
 // flow — descriptors and barrier addresses then live in uniform registers — while only this lane issues the
 // single-thread instructions (tcgen05.mma / tcgen05.commit / TMA).
@@ -197,6 +213,14 @@ __device__ __forceinline__ uint32_t make_idesc(int M, int N) {
     d |= 1u << 4;                  // c_format = F32
     d |= 1u << 7;                  // a_format = BF16
     d |= 1u << 10;                 // b_format = BF16
+    d |= (uint32_t)(N >> 3) << 17;
+    d |= (uint32_t)(M >> 4) << 24;
+    return d;
+}
+// kind::f8f6f4 instruction descriptor: D=f32, A=B=e4m3 (format code 0), both K-major, M x N
+__device__ __forceinline__ uint32_t make_idesc_e4m3(int M, int N) {
+    uint32_t d = 0;
+    d |= 1u << 4;                  // c_format = F32; a_format = b_format = E4M3 (0)
     d |= (uint32_t)(N >> 3) << 17;
     d |= (uint32_t)(M >> 4) << 24;
     return d;

@@ -335,7 +335,7 @@ def sharded_full_loss_step(q_local: torch.Tensor, v_local: torch.Tensor, tempera
     jc = max(1, min(B, budget // (M * Nv * 2)))
     N = k.n_buffer(M, jc * Nv, dev)            # one buffer, row pitch jc*Nv, reused by every chunk
     clip_rows = torch.empty(Bl, B, dtype=torch.float32, device=dev)
-    idx = torch.empty(B, Bl * ops.nq_padded(Nq), dtype=ops.idx_dtype(Nv), device=dev)
+    idx = ops.idx_buffer(B, Bl, Nq, Nv, dev)
     nsums = torch.zeros(2, dtype=torch.float64, device=dev)
     dq_dense = torch.empty(M, D, dtype=torch.float32, device=dev)
     dv_part = torch.empty(B * Nv, D, dtype=torch.float32, device=dev)    # this rank's rows against every image

@@ -109,6 +109,17 @@ def nq_padded(Nq: int) -> int:
     return (Nq + 15) // 16 * 16
 
 
+def idx_buffer(Bv: int, Bq: int, Nq: int, Nv: int, device) -> torch.Tensor:
+    """Argmax index buffer [Bv, Bq*nq_padded(Nq)] for a forward.  The kernels never write the entries a >= Nq of a
+    query's run (the padding up to nq_pad); they are set to 0 here so that the whole buffer is defined, and two
+    forwards of the same inputs give equal buffers whatever memory they were allocated from."""
+    nqp = nq_padded(Nq)
+    idx = torch.empty(Bv, Bq * nqp, dtype=idx_dtype(Nv), device=device)
+    if nqp != Nq:
+        idx.view(Bv, Bq, nqp)[:, :, Nq:].zero_()
+    return idx
+
+
 def idx_to_reference_layout(idx: torch.Tensor, Bq: int, Nq: int) -> torch.Tensor:
     """Library layout [Bv, Bq*nq_pad] -> the reference's torch.max(token_sims, dim=3)[1]: (Bq,Bv,Nq) int64."""
     Bv = idx.shape[0]
@@ -129,7 +140,7 @@ def maxmean_fwd(q: torch.Tensor, v: torch.Tensor, scale: torch.Tensor, T: torch.
         raise ValueError("embedding dims differ")
     dt = _dtype_code(q)
     clip = torch.empty(Bq, Bv, dtype=torch.float32, device=q.device)
-    idx = torch.empty(Bv, Bq * nq_padded(Nq), dtype=idx_dtype(Nv), device=q.device) if want_idx else None
+    idx = idx_buffer(Bv, Bq, Nq, Nv, q.device) if want_idx else None
     nws = lib.triad_maxmean_fwd_workspace_bytes_ex(Bq, Bv, Nq, Nv, D, dt, int(flags))
     with _on(q):
         ws = _Workspace.get(nws, q.device, "fwd")
@@ -168,7 +179,7 @@ def maxmean_fwd_nonneg(q: torch.Tensor, v: torch.Tensor, scale: torch.Tensor, T:
         raise ValueError("embedding dims differ")
     clip = torch.empty(Bq, Bv, dtype=torch.float32, device=q.device)
     if idx is None:
-        idx = torch.empty(Bv, Bq * nq_padded(Nq), dtype=idx_dtype(Nv), device=q.device)
+        idx = idx_buffer(Bv, Bq, Nq, Nv, q.device)
     _check_out(idx, (Bv, Bq * nq_padded(Nq)), idx_dtype(Nv), "idx")
     if N is None:
         N = torch.empty(Bq * Nq, Bv * Nv, dtype=torch.bfloat16, device=q.device)

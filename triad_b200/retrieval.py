@@ -59,10 +59,135 @@ def aggregator_tv_v2t(t_feats, v_feats, temperature) -> float:
     return _scores(t_feats, v_feats, temperature, 1).item()
 
 
-def retrieve_topk(q_feats: torch.Tensor, gallery: torch.Tensor, temperature, k: int, direction: int = 0):
-    """Top-k gallery items for one query (BASELINE cfg 5): (scores fp32 [k], ids int32 [k])."""
+class Fp8Gallery:
+    """A retrieval gallery stored as e4m3 codes with one fp32 scale per patch: about half the bytes of bf16.
+
+    ``codes`` is ``torch.float8_e4m3fn [n_img, Nv, D]`` and ``scales`` fp32 ``[n_img, Nv]``; patch p of image n stands
+    for ``scales[n, p] * codes[n, p, :]``.  Each patch row is quantized on its own (``triad_quantize_e4m3``:
+    s = amax / 448, codes = e4m3(x / s) with saturation), so quantizing a slice of a gallery gives exactly that slice of
+    the quantized gallery.  ``retrieve_topk`` and ``dist.sharded_retrieve_topk`` accept it in place of a bf16 tensor
+    (direction 0 only).  D must be 128, 256, 384 or 512."""
+
+    def __init__(self, codes: torch.Tensor, scales: torch.Tensor):
+        if codes.dtype != torch.float8_e4m3fn or codes.dim() != 3:
+            raise ValueError("Fp8Gallery: codes must be a float8_e4m3fn tensor [n_img, Nv, D]")
+        n_img, Nv, D = codes.shape
+        _check_fp8_shape(n_img, Nv, D)
+        if scales.dtype != torch.float32 or tuple(scales.shape) != (n_img, Nv):
+            raise ValueError(f"Fp8Gallery: scales must be float32 [{n_img}, {Nv}], got {scales.dtype} {tuple(scales.shape)}")
+        if codes.device != scales.device or not codes.is_contiguous() or not scales.is_contiguous():
+            raise ValueError("Fp8Gallery: codes and scales must be contiguous and on the same device")
+        self.codes = codes
+        self.scales = scales
+
+    @classmethod
+    def empty(cls, n_img: int, Nv: int, D: int, device="cuda") -> "Fp8Gallery":
+        _check_fp8_shape(n_img, Nv, D)
+        return cls(torch.empty(n_img, Nv, D, dtype=torch.float8_e4m3fn, device=device),
+                   torch.empty(n_img, Nv, dtype=torch.float32, device=device))
+
+    @property
+    def shape(self):
+        return tuple(self.codes.shape)
+
+    @property
+    def device(self) -> torch.device:
+        return self.codes.device
+
+    @property
+    def nbytes(self) -> int:
+        n_img, Nv, D = self.shape
+        return n_img * Nv * D + 4 * n_img * Nv
+
+    def __len__(self) -> int:
+        return self.shape[0]
+
+    def __getitem__(self, sl) -> "Fp8Gallery":
+        """Images [start, stop) as a view (no copy): a contiguous shard of the gallery."""
+        if not isinstance(sl, slice) or sl.step not in (None, 1):
+            raise TypeError("Fp8Gallery: only contiguous slices of images are supported")
+        return Fp8Gallery(self.codes[sl], self.scales[sl])
+
+    def put(self, i0: int, feats: torch.Tensor) -> None:
+        """Quantize the embedded images ``feats`` ([b, Nv, D] bf16 or fp32, on the gallery's device) into images
+        [i0, i0 + b).  Lets a caller build a gallery larger than its bf16 form would fit, batch by batch."""
+        n_img, Nv, D = self.shape
+        if feats.dim() != 3 or tuple(feats.shape[1:]) != (Nv, D):
+            raise ValueError(f"Fp8Gallery.put: feats must be [b, {Nv}, {D}], got {tuple(feats.shape)}")
+        b = feats.shape[0]
+        if not 0 <= i0 or i0 + b > n_img:
+            raise IndexError(f"Fp8Gallery.put: images [{i0}, {i0 + b}) outside [0, {n_img})")
+        if feats.device != self.device:
+            raise ValueError("Fp8Gallery.put: feats must be on the gallery's device")
+        if b == 0:
+            return
+        _quantize_rows(feats, self.codes[i0:i0 + b], self.scales[i0:i0 + b])
+
+
+def _check_fp8_shape(n_img: int, Nv: int, D: int) -> None:
+    if n_img < 1 or not 1 <= Nv <= 65535:
+        raise ValueError(f"Fp8Gallery: need n_img >= 1 and 1 <= Nv <= 65535, got n_img={n_img}, Nv={Nv}")
+    if D % 128 or not 128 <= D <= 512:
+        raise ValueError(f"Fp8Gallery: D must be 128, 256, 384 or 512, got {D}")
+
+
+def _quantize_rows(x: torch.Tensor, codes: torch.Tensor, scales: torch.Tensor) -> None:
+    """triad_quantize_e4m3 of the rows of x (last dim D) into codes / scales of the same row count."""
     lib = _lib.load()
-    s = _scores(q_feats, gallery, temperature, direction)
+    x = x.contiguous()
+    dt = ops._dtype_code(x)
+    D = x.shape[-1]
+    rows = x.numel() // D
+    with ops._on(x):
+        check(lib.triad_quantize_e4m3(x.data_ptr(), dt, rows, D, codes.data_ptr(), scales.data_ptr(), ops._stream(x.device)),
+              "triad_quantize_e4m3")
+
+
+def quantize_gallery(feats: torch.Tensor) -> Fp8Gallery:
+    """Fp8Gallery of the embedded gallery ``feats`` ([n_img, Nv, D] bf16 or fp32)."""
+    if feats.dim() != 3:
+        raise ValueError(f"quantize_gallery: feats must be [n_img, Nv, D], got {tuple(feats.shape)}")
+    g = Fp8Gallery.empty(*feats.shape, device=feats.device)
+    g.put(0, feats)
+    return g
+
+
+def _scores_fp8(q_feats: torch.Tensor, gallery: Fp8Gallery, temperature, direction: int) -> torch.Tensor:
+    """scores[n] of one query (Nq, D) against an e4m3 gallery: the query is quantized per token on the device, then
+    scored with the tensor cores' kind::f8f6f4 MMA (triad_retrieve_scores_e4m3)."""
+    if direction != 0:
+        raise ValueError("an Fp8Gallery supports direction 0 (mean over query tokens of max over patches) only")
+    n_img, Nv, D = gallery.shape
+    if q_feats.dim() != 2 or q_feats.shape[1] != D:
+        raise ValueError(f"query must be [Nq, {D}], got {tuple(q_feats.shape)}")
+    lib = _lib.load()
+    q = q_feats.contiguous()
+    Nq = q.shape[0]
+    dev = gallery.device
+    q_codes = torch.empty(Nq, D, dtype=torch.uint8, device=dev)
+    q_scales = torch.empty(Nq, dtype=torch.float32, device=dev)
+    _quantize_rows(q, q_codes, q_scales)
+    T = ops.temperature_tensor(temperature, dev)
+    out = torch.empty(n_img, dtype=torch.float32, device=dev)
+    nws = lib.triad_retrieve_e4m3_workspace_bytes(Nq, n_img, Nv, D)
+    with ops._on(out):
+        ws = ops._Workspace.get(nws, dev, "retrieve_e4m3")
+        check(lib.triad_retrieve_scores_e4m3(q_codes.data_ptr(), q_scales.data_ptr(), Nq, gallery.codes.data_ptr(),
+                                             gallery.scales.data_ptr(), n_img, Nv, D, T.data_ptr(), out.data_ptr(),
+                                             ws.data_ptr(), ws.numel(), ops._stream(dev)), "triad_retrieve_scores_e4m3")
+    return out
+
+
+def retrieve_topk(q_feats: torch.Tensor, gallery, temperature, k: int, direction: int = 0):
+    """Top-k gallery items for one query (BASELINE cfg 5): (scores fp32 [k], ids int32 [k]).
+
+    ``gallery`` is an embedding tensor [n_img, Nv, D] or an ``Fp8Gallery`` (e4m3 codes with per-patch scales; the
+    query is then quantized per token in the same call, and only direction 0 is supported)."""
+    if isinstance(gallery, Fp8Gallery):
+        s = _scores_fp8(q_feats, gallery, temperature, direction)
+    else:
+        s = _scores(q_feats, gallery, temperature, direction)
+    lib = _lib.load()
     n = s.numel()
     out_s = torch.empty(k, dtype=torch.float32, device=s.device)
     out_i = torch.empty(k, dtype=torch.int32, device=s.device)
