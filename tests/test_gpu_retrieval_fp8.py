@@ -250,7 +250,7 @@ def _acc_rel(acc_bits):
 # C. scores and top-k against fp64 on every path
 # ----------------------------------------------------------------------------------------------------------------
 def _fp8_path(Nq, n, Nv, D, sms=_SMS):
-    """(kernel, tile order, C, sub-tiles): launch_maxmean_tc_e4m3 with the e4m3 image size Nv*D."""
+    """(kernel, tile order, C, sub-tiles): launch_maxmean_tc's e4m3 path with the e4m3 image size Nv*D."""
     cta = 1 if Nq <= 128 else 2
     n_m = -(-Nq // (128 * cta))
     img = Nv * D

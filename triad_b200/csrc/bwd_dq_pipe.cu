@@ -270,7 +270,7 @@ int launch_dq_pipe(const void* v, const void* idx, const float* g, const float* 
     cuuint64_t dims[3] = {(cuuint64_t)D, (cuuint64_t)Nv, (cuuint64_t)Bv};
     cuuint64_t strides[2] = {(cuuint64_t)D * 2, (cuuint64_t)Nv * D * 2};
     cuuint32_t box[3] = {(cuuint32_t)kSlice, (cuuint32_t)Nv, 1};
-    int rc = encode_tmap_bf16(&mv, v, 3, dims, strides, box, false);
+    int rc = encode_tmap(&mv, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, v, 3, dims, strides, box, Swizzle::kNone);
     if (rc) return rc;
     Params p;
     p.idx = (const uint8_t*)idx; p.g = g; p.row_scale = row_scale; p.T = Tp;

@@ -21,7 +21,15 @@ int fail_msg(int status, const char* msg) {
     return status;
 }
 
-// forward workspace: [0,256) control block (int abort flag), then the partial sums
+int device_sms(int* sms) {
+    int dev = 0;
+    *sms = 148;
+    TRIAD_CUDA_CHECK(cudaGetDevice(&dev));
+    TRIAD_CUDA_CHECK(cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev));
+    return TRIAD_OK;
+}
+
+// forward workspace: control block (kCtrlBlockBytes), then the partial sums
 static size_t fwd_part_bytes(int M, int Bv, int Nq) {
     PartLayout pl = part_layout(M, Nq);
     return align_up((size_t)Bv * pl.G * pl.S * sizeof(float), 256);
@@ -65,7 +73,7 @@ extern "C" int triad_row_scale(const int64_t* mask, int Bq, int Nq, float* row_s
     return launch_row_scale(mask, Bq, Nq, row_scale, (cudaStream_t)stream);
 }
 
-// packed forward (TRIAD_FWD_PACK_ROWS): [0,256) control | partial sums (packed layout) | packing maps | packed q
+// packed forward (TRIAD_FWD_PACK_ROWS): control block | partial sums (packed layout) | packing maps | packed q
 static size_t fwd_part_bytes_packed(int Bq, int Bv, int Nq) {
     return align_up((size_t)Bv * Bq * packed_pieces(Nq) * sizeof(float), 256);
 }
@@ -73,9 +81,9 @@ static size_t fwd_part_bytes_packed(int Bq, int Bv, int Nq) {
 extern "C" size_t triad_maxmean_fwd_workspace_bytes_ex(int Bq, int Bv, int Nq, int Nv, int D, int dtype, int flags) {
     (void)Nv;
     if (Bq <= 0 || Bv <= 0 || Nq <= 0) return 0;
-    size_t n = 256 + fwd_part_bytes(Bq * Nq, Bv, Nq);
+    size_t n = kCtrlBlockBytes + fwd_part_bytes(Bq * Nq, Bv, Nq);
     if ((flags & TRIAD_FWD_PACK_ROWS) && dtype == TRIAD_DTYPE_BF16 && D > 0) {
-        const size_t packed = 256 + fwd_part_bytes_packed(Bq, Bv, Nq) + pack_map_bytes(Bq, Nq) +
+        const size_t packed = kCtrlBlockBytes + fwd_part_bytes_packed(Bq, Bv, Nq) + pack_map_bytes(Bq, Nq) +
                               align_up((size_t)Bq * Nq * D * 2, 256);
         if (packed > n) n = packed;
     }
@@ -85,6 +93,11 @@ extern "C" size_t triad_maxmean_fwd_workspace_bytes_ex(int Bq, int Bv, int Nq, i
 extern "C" size_t triad_maxmean_fwd_workspace_bytes(int Bq, int Bv, int Nq, int Nv, int D, int dtype) {
     return triad_maxmean_fwd_workspace_bytes_ex(Bq, Bv, Nq, Nv, D, dtype, 0);
 }
+
+// cta_group of the unpacked tcgen05 forwards.  A single row tile of <= 128 tokens (one text query against a gallery):
+// cta_group::1 — a pair would spend a 256-row MMA on <= 128 rows, and at one tile per image that MMA time equals the
+// HBM time of the image, leaving no slack to overlap; alone, each SM streams its own images at twice that rate.
+static int fwd_cta_group(int M, int flags) { return ((flags & TRIAD_FWD_FORCE_1CTA) || M <= 128) ? 1 : 2; }
 
 static int fwd_impl(const void* q, const void* v, const float* row_scale, const float* temperature, int inv_T,
                     int Bq, int Bv, int Nq, int Nv, int D, int dtype, float* clip, void* idx,
@@ -99,14 +112,14 @@ static int fwd_impl(const void* q, const void* v, const float* row_scale, const 
 
     const int M = Bq * Nq;
     int* abort_flag = (int*)ws;
-    float* part = (float*)((char*)ws + 256);
-    TRIAD_CUDA_CHECK(cudaMemsetAsync(abort_flag, 0, 256, st));
+    float* part = (float*)((char*)ws + kCtrlBlockBytes);
+    TRIAD_CUDA_CHECK(cudaMemsetAsync(abort_flag, 0, kCtrlBlockBytes, st));
 
     const bool use_tc = dtype == TRIAD_DTYPE_BF16 && !(flags & TRIAD_FWD_FORCE_SIMT) && tc_supported(Nv, D);
     int rc;
     if (use_tc && (flags & TRIAD_FWD_PACK_ROWS)) {
         // masked text queries: drop the zero-weight rows before the tensor cores (pack.cu)
-        char* maps = (char*)ws + 256 + fwd_part_bytes_packed(Bq, Bv, Nq);
+        char* maps = (char*)ws + kCtrlBlockBytes + fwd_part_bytes_packed(Bq, Bv, Nq);
         void* qp = maps + pack_map_bytes(Bq, Nq);
         rc = launch_pack_map(row_scale, Bq, Nq, maps, st);
         if (rc) return rc;
@@ -115,17 +128,14 @@ static int fwd_impl(const void* q, const void* v, const float* row_scale, const 
         if (idx) TRIAD_CUDA_CHECK(cudaMemsetAsync(idx, 0, (size_t)Bv * Bq * nq_padded(Nq) * (Nv > 256 ? 2 : 1), st));
         const int cta_group = (flags & TRIAD_FWD_FORCE_1CTA) ? 1 : 2;
         rc = launch_maxmean_tc(qp, v, row_scale, temperature, inv_T, M, Bv, Nq, Nv, D, part, idx, abort_flag, cta_group, flags,
-                               (const int*)maps, nullptr, st);
+                               (const int*)maps, nullptr, nullptr, st);
         if (rc) return rc;
         if (flags & TRIAD_FWD_TEST_TRIP_WATCHDOG) TRIAD_CUDA_CHECK(cudaMemsetAsync(abort_flag, 1, 4, st));
         return launch_finalize_clip_packed(part, (const int*)maps, Bq, Bv, Nq, clip, abort_flag, st);
     }
     if (use_tc) {
-        // A single row tile of <= 128 tokens (one text query against a gallery): cta_group::1 — a pair would
-        // spend a 256-row MMA on <= 128 rows, and at one tile per image that MMA time equals the HBM time of
-        // the image, leaving no slack to overlap; alone, each SM streams its own images at twice that rate.
-        const int cta_group = ((flags & TRIAD_FWD_FORCE_1CTA) || M <= 128) ? 1 : 2;
-        rc = launch_maxmean_tc(q, v, row_scale, temperature, inv_T, M, Bv, Nq, Nv, D, part, idx, abort_flag, cta_group, flags, nullptr, nullptr, st);
+        rc = launch_maxmean_tc(q, v, row_scale, temperature, inv_T, M, Bv, Nq, Nv, D, part, idx, abort_flag,
+                               fwd_cta_group(M, flags), flags, nullptr, nullptr, nullptr, st);
     } else {
         rc = launch_maxmean_simt(q, v, row_scale, temperature, inv_T, M, Bv, Nq, Nv, D, dtype, part, idx, st);
     }
@@ -143,12 +153,12 @@ extern "C" int triad_maxmean_fwd(const void* q, const void* v, const float* row_
 
 // ---------------------------------------------------------------------------------------------
 // max-mean forward + dense non-negative-pressure regulariser from ONE pass over the similarities (bf16, tcgen05)
-// workspace: [0,256) control | max-mean partial sums | regulariser partials
+// workspace: control block | max-mean partial sums | regulariser partials
 // ---------------------------------------------------------------------------------------------
 extern "C" size_t triad_maxmean_fwd_nonneg_workspace_bytes(int Bq, int Bv, int Nq, int Nv, int D) {
     (void)Nv; (void)D;
     if (Bq <= 0 || Bv <= 0 || Nq <= 0) return 0;
-    return 256 + fwd_part_bytes(Bq * Nq, Bv, Nq) + (size_t)kNonnegFusedPartials * 2 * sizeof(double);
+    return kCtrlBlockBytes + fwd_part_bytes(Bq * Nq, Bv, Nq) + (size_t)kNonnegFusedPartials * 2 * sizeof(double);
 }
 
 extern "C" int triad_maxmean_fwd_nonneg(const void* q, const void* v, const float* row_scale, const float* temperature,
@@ -159,28 +169,22 @@ extern "C" int triad_maxmean_fwd_nonneg(const void* q, const void* v, const floa
         return fail_msg(TRIAD_ERR_BAD_ARG, "maxmean_fwd_nonneg: null pointer");
     if (Bq <= 0 || Bv <= 0 || Nq <= 0 || Nv <= 0 || D <= 0) return fail_msg(TRIAD_ERR_BAD_SHAPE, "maxmean_fwd_nonneg: bad shape");
     if ((long long)Bq * Nq > 0x7fffffffLL) return fail_msg(TRIAD_ERR_BAD_SHAPE, "maxmean_fwd_nonneg: Bq*Nq overflows int32");
-    if (!tc_supported(Nv, D) || Nv > 256 || Nv % 8 != 0)
+    if (!tc_emit_supported(Nv, D))
         return fail_msg(TRIAD_ERR_UNSUPPORTED, "maxmean_fwd_nonneg: needs D % 64 == 0, D <= 512, Nv <= 256, Nv % 8 == 0");
     if (!(lo < 0.f)) return fail_msg(TRIAD_ERR_BAD_ARG, "maxmean_fwd_nonneg: lo must be negative");
     if (ldn < (long long)Bv * Nv || ldn % 8 != 0 || (long long)ldn * 2 >= (1ll << 40)) return fail_msg(TRIAD_ERR_BAD_SHAPE, "maxmean_fwd_nonneg: ldn");
     if (((uintptr_t)q | (uintptr_t)v | (uintptr_t)n_out | (uintptr_t)ws) & 15) return fail_msg(TRIAD_ERR_ALIGNMENT, "maxmean_fwd_nonneg: 16-byte alignment");
     if (ws_bytes < triad_maxmean_fwd_nonneg_workspace_bytes(Bq, Bv, Nq, Nv, D)) return fail_msg(TRIAD_ERR_WORKSPACE, "maxmean_fwd_nonneg: workspace too small");
     cudaStream_t st = (cudaStream_t)stream;
-    int dev = 0, sms = 0;
-    TRIAD_CUDA_CHECK(cudaGetDevice(&dev));
-    TRIAD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    if (sms * 8 > kNonnegFusedPartials) return fail_msg(TRIAD_ERR_UNSUPPORTED, "maxmean_fwd_nonneg: too many SMs for the partial buffer");
     const int M = Bq * Nq;
     int* abort_flag = (int*)ws;
-    float* part = (float*)((char*)ws + 256);
-    double* npart = (double*)((char*)ws + 256 + fwd_part_bytes(M, Bv, Nq));
-    TRIAD_CUDA_CHECK(cudaMemsetAsync(abort_flag, 0, 256, st));
-    EmitNArgs e{n_out, ldn, lo, coef, 1, npart, 1};
+    float* part = (float*)((char*)ws + kCtrlBlockBytes);
+    double* npart = (double*)((char*)ws + kCtrlBlockBytes + fwd_part_bytes(M, Bv, Nq));
+    TRIAD_CUDA_CHECK(cudaMemsetAsync(abort_flag, 0, kCtrlBlockBytes, st));
+    EmitNArgs e{n_out, ldn, lo, coef, 1, npart, sums, 1};
     const int cta_group = (flags & TRIAD_FWD_FORCE_1CTA) ? 1 : 2;
-    int rc = launch_maxmean_tc(q, v, row_scale, temperature, 0, M, Bv, Nq, Nv, D, part, idx, abort_flag, cta_group, flags,
-                               nullptr, &e, st);
-    if (rc) return rc;
-    rc = launch_nonneg_finish(npart, sms * 8, sums, st);
+    const int rc = launch_maxmean_tc(q, v, row_scale, temperature, 0, M, Bv, Nq, Nv, D, part, idx, abort_flag, cta_group,
+                                     flags, nullptr, &e, nullptr, st);
     if (rc) return rc;
     if (flags & TRIAD_FWD_TEST_TRIP_WATCHDOG) TRIAD_CUDA_CHECK(cudaMemsetAsync(abort_flag, 1, 4, st));
     return launch_finalize_clip(part, Bq, Bv, Nq, clip, abort_flag, st);
@@ -237,12 +241,12 @@ extern "C" int triad_retrieve_scores(const void* q, int Nq, const void* gallery,
 
 // ---------------------------------------------------------------------------------------------
 // retrieval scores on an e4m3 gallery (direction 0, divides by T)
-// workspace: row weights [Nq] | [0,256) control | partial sums
+// workspace: row weights [Nq] | control block | partial sums
 // ---------------------------------------------------------------------------------------------
 extern "C" size_t triad_retrieve_e4m3_workspace_bytes(int Nq, int n_img, int Nv, int D) {
     (void)Nv; (void)D;
     if (Nq <= 0 || n_img <= 0) return 0;
-    return align_up((size_t)Nq * 4, 256) + 256 + fwd_part_bytes(Nq, n_img, Nq);
+    return align_up((size_t)Nq * 4, 256) + kCtrlBlockBytes + fwd_part_bytes(Nq, n_img, Nq);
 }
 
 extern "C" int triad_retrieve_scores_e4m3(const void* q_codes, const float* q_scales, int Nq, const void* g_codes,
@@ -262,12 +266,13 @@ extern "C" int triad_retrieve_scores_e4m3(const void* q_codes, const float* q_sc
     float* rs = (float*)ws;
     char* fws = (char*)ws + align_up((size_t)Nq * 4, 256);
     int* abort_flag = (int*)fws;
-    float* part = (float*)(fws + 256);
-    TRIAD_CUDA_CHECK(cudaMemsetAsync(abort_flag, 0, 256, st));
+    float* part = (float*)(fws + kCtrlBlockBytes);
+    TRIAD_CUDA_CHECK(cudaMemsetAsync(abort_flag, 0, kCtrlBlockBytes, st));
     int rc = launch_row_scale(nullptr, 1, Nq, rs, st);
     if (rc) return rc;
-    rc = launch_maxmean_tc_e4m3(q_codes, q_scales, g_codes, g_scales, rs, temperature, Nq, n_img, Nq, Nv, D, part,
-                                abort_flag, st);
+    const E4m3Args e4m3{q_scales, g_scales};
+    rc = launch_maxmean_tc(q_codes, g_codes, rs, temperature, 1, Nq, n_img, Nq, Nv, D, part, nullptr, abort_flag,
+                           fwd_cta_group(Nq, 0), 0, nullptr, nullptr, &e4m3, st);
     if (rc) return rc;
     return launch_finalize_clip(part, 1, n_img, Nq, scores, abort_flag, st);
 }

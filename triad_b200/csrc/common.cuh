@@ -1,5 +1,6 @@
 // Shared declarations for the triad_b200 CUDA library (sm_100a only).
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <stdint.h>
@@ -44,8 +45,42 @@ void count_launch();                                // triad_launch_count(): ker
         ::triad::count_launch();                                            \
     } while (0)
 
+// Launches kKernel as clusters of cta_group CTAs with smem bytes of dynamic shared memory, and counts the launch.
+template <auto kKernel, typename... Args>
+int launch_clusters(int cta_group, int n_clusters, int threads, uint32_t smem, cudaStream_t st, const Args&... args) {
+    TRIAD_SET_MAX_SMEM(kKernel, smem);
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(n_clusters * cta_group));
+    cfg.blockDim = dim3(threads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = cta_group;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    TRIAD_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kKernel, args...));
+    count_launch();
+    return TRIAD_OK;
+}
+
+// Multiprocessor count of the current device.  On a CUDA error it returns TRIAD_ERR_CUDA and leaves *sms = 148 (a
+// B200): the workspace-size functions, which cannot report an error, size for that.
+int device_sms(int* sms);
+
+// Tiled tensor map over bf16, fp32 or uint8 elements (rank 2 or 3, element strides 1, 256-byte L2 promotion, zero fill).
+enum class Swizzle { kNone, k128B };
+int encode_tmap(CUtensorMap* map, CUtensorMapDataType type, const void* base, int rank, const cuuint64_t* dims,
+                const cuuint64_t* strides, const cuuint32_t* box, Swizzle swizzle);
+
 static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
+
+// The control block at the start of a workspace, cleared before each call: the kernels' watchdog abort flag at [0]
+// (and the backward's dT ticket at [16]).
+constexpr size_t kCtrlBlockBytes = 256;
 
 // ---- forward partial-sum layout ---------------------------------------------------------
 // The forward kernels reduce row maxima per 32-row GROUP (one warp of the epilogue) and per
@@ -88,14 +123,21 @@ int launch_maxmean_simt(const void* q, const void* v, const float* row_scale, co
                         float* part, void* idx, cudaStream_t st);   // idx: [Bv][M/Nq][nq_padded(Nq)]
 // dense-regulariser modes of the tcgen05 forward (maxmean_tc.cu, kMode): the epilogue writes N = dL/d<q,v> of the
 // non-negative-pressure term — instead of reducing each tile (with_maxmean = 0) or next to the max-mean reduction
-// (with_maxmean = 1: clip partials, idx and N from ONE pass over the similarities); partials: [SMs*8][2] doubles
-struct EmitNArgs { void* n_out; long long ldn; float lo, coef; int write_n; double* partials; int with_maxmean; };
+// (with_maxmean = 1: clip partials, idx and N from ONE pass over the similarities).  Every epilogue warp of every CTA
+// owns one slot of [SMs * kEmitEpiWarps][2] double partials; the launch clears them and adds them to sums[0..1].
+struct EmitNArgs { void* n_out; long long ldn; float lo, coef; int write_n; double* partials; double* sums; int with_maxmean; };
+constexpr int kEmitEpiWarps = 8;                                      // epilogue warps 4-11 of the emitting kernel
+constexpr int kNonnegFusedPartials = 512 * kEmitEpiWarps;             // partial slots: devices of up to 512 SMs
+bool tc_emit_supported(int Nv, int D);
+// e4m3 retrieval operands (kFp8): q and v hold e4m3 codes, scaled per token (q_scale [M]) and per patch
+// (g_scale [Bv][Nv]); divides by T, no idx, D in {128, 256, 384, 512}
+struct E4m3Args { const float* q_scale; const float* g_scale; };
+bool tc_e4m3_supported(int Nv, int D);
 int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, const float* T,
                       int inv_T, int M, int Bv, int Nq, int Nv, int D,
                       float* part, void* idx, int* abort_flag, int cta_group, int flags, const int* pack_maps,
-                      const EmitNArgs* emit, cudaStream_t st);
+                      const EmitNArgs* emit, const E4m3Args* e4m3, cudaStream_t st);
 // sums[0..1] += the per-warp partials of a dense-regulariser forward, in slot order (dense_reg.cu)
-constexpr int kNonnegFusedPartials = 4096;                      // >= SMs * 8 epilogue warps
 int launch_nonneg_finish(const double* partials, int n, double* sums, cudaStream_t st);
 int launch_finalize_clip(const float* part, int Bq, int Bv, int Nq, float* clip, const int* abort_flag, cudaStream_t st);
 // packed rows (pack.cu): maps = off[Bq+1] | rowmap[Bq*Nq] | scratch
@@ -109,12 +151,6 @@ int launch_finalize_clip_packed(const float* part, const int* pack_off, int Bq, 
 // - (group of the query's first packed row); a query of <= Nq kept rows spans at most (Nq+30)/32 + 1 groups
 static inline int packed_pieces(int Nq) { return (Nq + 30) / 32 + 1; }
 bool tc_supported(int Nv, int D);
-// e4m3 retrieval forward (maxmean_tc.cu, kFp8): q_codes [M][D], g_codes [Bv][Nv][D] (e4m3 bytes), q_scale [M],
-// g_scale [Bv][Nv]; divides by T; no idx.  D in {128, 256, 384, 512}
-bool tc_e4m3_supported(int Nv, int D);
-int launch_maxmean_tc_e4m3(const void* q_codes, const float* q_scale, const void* g_codes, const float* g_scale,
-                           const float* row_scale, const float* T, int M, int Bv, int Nq, int Nv, int D,
-                           float* part, int* abort_flag, cudaStream_t st);
 // rows x D (fp32 or bf16) -> e4m3 codes [rows][D] + one fp32 scale per row (quant_e4m3.cu); D % 16 == 0, D <= 512
 int launch_quantize_e4m3(const void* x, int dtype, long long rows, int D, void* codes, float* scales, cudaStream_t st);
 // tiled dQ of the backward, bf16 only.  Nv <= 256 (uint8 winners): the software-pipelined shared-memory gather

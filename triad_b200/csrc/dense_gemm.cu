@@ -277,25 +277,22 @@ static int pick_splits(int n_tiles, int nkb, int n_clusters) {
 }
 
 }  // namespace dgemm
-
-int encode_tmap_f32_3d(CUtensorMap* map, const void* base, const cuuint64_t* dims, const cuuint64_t* strides, const cuuint32_t* box);
-
 }  // namespace triad
 
 using namespace triad;
 
-static int device_sms() {
-    int dev = 0, sms = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    return sms < 2 ? 2 : sms;
+// CTA pairs the split plans are made for (the workspace sizes depend on the plan, so a failed query plans for a B200)
+static int plan_clusters() {
+    int sms;
+    device_sms(&sms);
+    return max(1, sms / 2);
 }
 
 static int plan_splits(int M, int Kc, int mode, int* n_tiles, int* nkb, int* kb_per_split) {
-    const int sms = device_sms();
     const int rows_out = mode == 0 ? M : Kc, K = mode == 0 ? Kc : M;
     *n_tiles = ceil_div(rows_out, dgemm::kTileM);
     *nkb = ceil_div(K, dgemm::kBlockK);
-    int splits = dgemm::pick_splits(*n_tiles, *nkb, sms / 2);
+    int splits = dgemm::pick_splits(*n_tiles, *nkb, plan_clusters());
     *kb_per_split = ceil_div(*nkb, splits);
     return ceil_div(*nkb, *kb_per_split);             // no empty split
 }
@@ -303,7 +300,7 @@ static int plan_splits(int M, int Kc, int mode, int* n_tiles, int* nkb, int* kb_
 // The head backward's plan: with fewer (row tile, column slice) units than CTA pairs (the weight gradients: K = the
 // token count, 1-4 units) the K range is cut so that every pair gets one item; otherwise the shared heuristic.
 static int plan_head_splits(int M, int Kc, int D, int mode, int* n_tiles, int* n_slices, int* nkb, int* kb_per_split) {
-    const int clusters = device_sms() / 2;
+    const int clusters = plan_clusters();
     const int rows_out = mode == 0 ? M : Kc, K = mode == 0 ? Kc : M;
     *n_tiles = ceil_div(rows_out, dgemm::kTileM);
     *n_slices = ceil_div(D, 2 * dgemm::kHalfN);
@@ -319,14 +316,14 @@ extern "C" size_t triad_dense_grad_gemm_workspace_bytes(int M, int Kc, int D, in
     if (M <= 0 || Kc <= 0 || D <= 0) return 0;
     int n_tiles, nkb, kbs;
     const int splits = plan_splits(M, Kc, mode, &n_tiles, &nkb, &kbs);
-    return 256 + (size_t)splits * (size_t)(mode == 0 ? M : Kc) * (size_t)D * sizeof(float);
+    return kCtrlBlockBytes + (size_t)splits * (size_t)(mode == 0 ? M : Kc) * (size_t)D * sizeof(float);
 }
 
 namespace triad {
 size_t head_gemm_workspace_bytes(int M, int Kc, int D, int mode) {
     int n_tiles, n_slices, nkb, kbs;
     const int splits = plan_head_splits(M, Kc, D, mode, &n_tiles, &n_slices, &nkb, &kbs);
-    return 256 + (size_t)splits * (size_t)(mode == 0 ? M : Kc) * (size_t)D * sizeof(float);
+    return kCtrlBlockBytes + (size_t)splits * (size_t)(mode == 0 ? M : Kc) * (size_t)D * sizeof(float);
 }
 }  // namespace triad
 
@@ -335,9 +332,9 @@ size_t head_gemm_workspace_bytes(int M, int Kc, int D, int mode) {
 static int dgemm_launch(dgemm::Params p, const void* n_mat, long long ldn, int M, int Kc, const void* x, int D, int mode,
                         void* out, int out_kind, void* ws, size_t ws_bytes, cudaStream_t st) {
     using namespace dgemm;
-    int dev = 0, sms = 0;
-    TRIAD_CUDA_CHECK(cudaGetDevice(&dev));
-    TRIAD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    int rc = device_sms(&sms);
+    if (rc) return rc;
     const int rows_out = mode == 0 ? M : Kc;          // rows of the product
     const int K = mode == 0 ? Kc : M;                 // contraction length
     int n_clusters = sms / 2;
@@ -345,60 +342,44 @@ static int dgemm_launch(dgemm::Params p, const void* n_mat, long long ldn, int M
     p.D = D;
     p.abort_flag = (int*)ws;
     const size_t part_bytes = (size_t)p.splits * rows_out * D * sizeof(float);
-    if (ws_bytes < 256 + part_bytes) return fail_msg(TRIAD_ERR_WORKSPACE, "dense_grad_gemm: workspace too small");
-    float* part = (float*)((char*)ws + 256);
-    TRIAD_CUDA_CHECK(cudaMemsetAsync(ws, 0, 256, st));
+    if (ws_bytes < kCtrlBlockBytes + part_bytes) return fail_msg(TRIAD_ERR_WORKSPACE, "dense_grad_gemm: workspace too small");
+    float* part = (float*)((char*)ws + kCtrlBlockBytes);
+    TRIAD_CUDA_CHECK(cudaMemsetAsync(ws, 0, kCtrlBlockBytes, st));
 
     CUtensorMap ma, mb, mc;
-    int rc;
     if (mode == 0) {       // A = N, K-major: dims {Kc, M}, box {64 k, 128 rows}
         cuuint64_t dims[2] = {(cuuint64_t)Kc, (cuuint64_t)M};
         cuuint64_t strides[1] = {(cuuint64_t)ldn * 2};
         cuuint32_t box[2] = {64, 128};
-        rc = encode_tmap_bf16(&ma, n_mat, 2, dims, strides, box, true);
+        rc = encode_tmap(&ma, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, n_mat, 2, dims, strides, box, Swizzle::k128B);
     } else {               // A = N^T read MN-major from the same rows: dims {Kc (the product's rows), M (k)}, box {64, 64}
         cuuint64_t dims[2] = {(cuuint64_t)Kc, (cuuint64_t)M};
         cuuint64_t strides[1] = {(cuuint64_t)ldn * 2};
         cuuint32_t box[2] = {64, 64};
-        rc = encode_tmap_bf16(&ma, n_mat, 2, dims, strides, box, true);
+        rc = encode_tmap(&ma, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, n_mat, 2, dims, strides, box, Swizzle::k128B);
     }
     if (rc) return rc;
     {                      // B = V2 / Q2, [K][D], MN-major: dims {D, K}, box {64 n, 64 k}
         cuuint64_t dims[2] = {(cuuint64_t)D, (cuuint64_t)K};
         cuuint64_t strides[1] = {(cuuint64_t)D * 2};
         cuuint32_t box[2] = {64, 64};
-        rc = encode_tmap_bf16(&mb, x, 2, dims, strides, box, true);
+        rc = encode_tmap(&mb, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, x, 2, dims, strides, box, Swizzle::k128B);
         if (rc) return rc;
     }
     {                      // fp32 partials [splits][rows_out][D]: box {32 cols, 32 rows, 1}
         cuuint64_t dims[3] = {(cuuint64_t)D, (cuuint64_t)rows_out, (cuuint64_t)p.splits};
         cuuint64_t strides[2] = {(cuuint64_t)D * 4, (cuuint64_t)rows_out * D * 4};
         cuuint32_t box[3] = {32, 32, 1};
-        rc = encode_tmap_f32_3d(&mc, part, dims, strides, box);
+        rc = encode_tmap(&mc, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, part, 3, dims, strides, box, Swizzle::k128B);
         if (rc) return rc;
     }
     const int n_items = p.n_tiles * p.n_slices * p.splits;
     if (n_clusters > n_items) n_clusters = n_items;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(n_clusters * 2));
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = kSmemBytes;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-#define TRIAD_DGEMM_LAUNCH(AMN, HALVES)                                                         \
-    do {                                                                                       \
-        auto kern = dgemm_kernel<AMN, HALVES>;                                                 \
-        TRIAD_SET_MAX_SMEM(kern, kSmemBytes);                                                  \
-        TRIAD_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kern, ma, mb, mc, p));                       \
-    } while (0)
-    if (mode == 0) { if (p.n_halves == 2) TRIAD_DGEMM_LAUNCH(false, 2); else TRIAD_DGEMM_LAUNCH(false, 1); }
-    else           { if (p.n_halves == 2) TRIAD_DGEMM_LAUNCH(true, 2);  else TRIAD_DGEMM_LAUNCH(true, 1); }
-#undef TRIAD_DGEMM_LAUNCH
-    count_launch();
+    if (mode == 0) rc = p.n_halves == 2 ? launch_clusters<dgemm_kernel<false, 2>>(2, n_clusters, kThreads, kSmemBytes, st, ma, mb, mc, p)
+                                        : launch_clusters<dgemm_kernel<false, 1>>(2, n_clusters, kThreads, kSmemBytes, st, ma, mb, mc, p);
+    else           rc = p.n_halves == 2 ? launch_clusters<dgemm_kernel<true, 2>>(2, n_clusters, kThreads, kSmemBytes, st, ma, mb, mc, p)
+                                        : launch_clusters<dgemm_kernel<true, 1>>(2, n_clusters, kThreads, kSmemBytes, st, ma, mb, mc, p);
+    if (rc) return rc;
     const size_t n4 = (size_t)rows_out * D / 4;
     size_t want = (n4 + 255) / 256;
     const int blocks = (int)(want > (size_t)(148 * 16) ? (size_t)(148 * 16) : (want < 1 ? 1 : want));

@@ -182,9 +182,7 @@ extern "C" int triad_nonneg_chunk(void* S, size_t n, int dtype, const float* tem
 // Fused variant for bf16 (D % 64 == 0, D <= 512, Nv <= 256, Nv % 8 == 0): the tcgen05 forward kernel itself
 // produces N = dL/d<q,v> (maxmean_tc.cu, kEmitN) — no materialised S chunk, no separate elementwise pass.
 // ---------------------------------------------------------------------------------------------
-static const int kFusedPartials = kNonnegFusedPartials;         // >= SMs * 8 epilogue warps
-
-extern "C" size_t triad_nonneg_fused_workspace_bytes(void) { return 256 + (size_t)kFusedPartials * 2 * sizeof(double); }
+extern "C" size_t triad_nonneg_fused_workspace_bytes(void) { return kCtrlBlockBytes + (size_t)kNonnegFusedPartials * 2 * sizeof(double); }
 
 extern "C" int triad_nonneg_fused_chunk(const void* q, const void* v, const float* temperature,
                                         int Bq, int Bv, int Nq, int Nv, int D, float lo, float coef,
@@ -194,23 +192,14 @@ extern "C" int triad_nonneg_fused_chunk(const void* q, const void* v, const floa
     if (Bq <= 0 || Bv <= 0 || Nq <= 0 || Nv <= 0 || D <= 0) return fail_msg(TRIAD_ERR_BAD_SHAPE, "nonneg_fused: bad shape");
     if (!(lo < 0.f)) return fail_msg(TRIAD_ERR_BAD_ARG, "nonneg_fused: lo must be negative");
     if ((long long)Bq * Nq > 0x7fffffffLL) return fail_msg(TRIAD_ERR_BAD_SHAPE, "nonneg_fused: Bq*Nq overflows int32");
-    if (!tc_supported(Nv, D) || Nv > 256 || Nv % 8 != 0) return fail_msg(TRIAD_ERR_UNSUPPORTED, "nonneg_fused: needs D % 64 == 0, D <= 512, Nv <= 256, Nv % 8 == 0");
+    if (!tc_emit_supported(Nv, D)) return fail_msg(TRIAD_ERR_UNSUPPORTED, "nonneg_fused: needs D % 64 == 0, D <= 512, Nv <= 256, Nv % 8 == 0");
     if (write_grad && (ldn < (long long)Bv * Nv || ldn % 8 != 0)) return fail_msg(TRIAD_ERR_BAD_SHAPE, "nonneg_fused: ldn");
     if (write_grad && (long long)ldn * 2 >= (1ll << 40)) return fail_msg(TRIAD_ERR_BAD_SHAPE, "nonneg_fused: row pitch beyond the tensor map's 2^40 bytes");
     if (((uintptr_t)q | (uintptr_t)v | (uintptr_t)n_out | (uintptr_t)ws) & 15) return fail_msg(TRIAD_ERR_ALIGNMENT, "nonneg_fused: 16-byte alignment");
     if (ws_bytes < triad_nonneg_fused_workspace_bytes()) return fail_msg(TRIAD_ERR_WORKSPACE, "nonneg_fused: workspace too small");
     cudaStream_t st = (cudaStream_t)stream;
-    int dev = 0, sms = 0;
-    TRIAD_CUDA_CHECK(cudaGetDevice(&dev));
-    TRIAD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    if (sms * 8 > kFusedPartials) return fail_msg(TRIAD_ERR_UNSUPPORTED, "nonneg_fused: too many SMs for the partial buffer");
-    TRIAD_CUDA_CHECK(cudaMemsetAsync(ws, 0, 256, st));
-    double* partials = (double*)((char*)ws + 256);
-    EmitNArgs e{n_out, ldn, lo, coef, write_grad ? 1 : 0, partials, 0};
-    const int rc = launch_maxmean_tc(q, v, nullptr, temperature, 0, Bq * Nq, Bv, Nq, Nv, D, nullptr, nullptr, (int*)ws, 2, 0,
-                                     nullptr, &e, st);
-    if (rc) return rc;
-    dense::nonneg_finish_kernel<<<1, 32, 0, st>>>(partials, sms * 8, sums);
-    TRIAD_LAUNCH_CHECK("nonneg_finish_kernel");
-    return TRIAD_OK;
+    TRIAD_CUDA_CHECK(cudaMemsetAsync(ws, 0, kCtrlBlockBytes, st));
+    EmitNArgs e{n_out, ldn, lo, coef, write_grad ? 1 : 0, (double*)((char*)ws + kCtrlBlockBytes), sums, 0};
+    return launch_maxmean_tc(q, v, nullptr, temperature, 0, Bq * Nq, Bv, Nq, Nv, D, nullptr, nullptr, (int*)ws, 2, 0,
+                             nullptr, &e, nullptr, st);
 }

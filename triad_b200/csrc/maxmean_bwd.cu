@@ -956,7 +956,7 @@ extern "C" int triad_maxmean_bwd(const void* q, const void* v, const void* idx, 
     if (!ws || ws_bytes < ((dv || (flags & TRIAD_BWD_PACK_ROWS)) ? triad_maxmean_bwd_workspace_bytes(Bq, Bv, Nq, Nv, D, dtype) : kCtrlBytes))
         return fail_msg(TRIAD_ERR_WORKSPACE, "maxmean_bwd: workspace too small");
     cudaStream_t st = (cudaStream_t)stream;
-    TRIAD_CUDA_CHECK(cudaMemsetAsync(ws, 0, 256, st));      // abort flag + dT ticket
+    TRIAD_CUDA_CHECK(cudaMemsetAsync(ws, 0, kCtrlBlockBytes, st));      // abort flag + dT ticket
     if (flags & TRIAD_BWD_TEST_TRIP_WATCHDOG) TRIAD_CUDA_CHECK(cudaMemsetAsync(ws, 1, 4, st));
     const bool wide = Nv > 256;
     const size_t pmo = triad_maxmean_bwd_workspace_bytes(Bq, Bv, Nq, Nv, D, dtype) - pack_map_bytes(Bq, Nq);

@@ -162,7 +162,6 @@ __device__ __forceinline__ void first_ge32(const uint32_t (&r)[32], int col0, in
 // are clipped by the tensor map {Nv, images, M}.  Round 1's version (per-lane 16-byte stores out of a transposing
 // staging buffer) spent 4 dependent STS -> LDS -> STG round trips per chunk: 3.8 ms per pass against 2.45 ms for
 // the plain forward.
-constexpr int kEmitEpiWarps = 8;                                    // epilogue warps 4-11; one n_partials slot each
 constexpr int kEmitThreads = (kEpiWarp0 + kEmitEpiWarps) * 32;      // 384
 constexpr uint32_t kStgBytesPerWarp = 32 * 128;                     // one 32 x 64 bf16 box
 constexpr uint32_t kStgBytes = 4 * 2 * kStgBytesPerWarp;            // four emission warps x two boxes: 32 KB, carved
@@ -776,81 +775,6 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-typedef CUresult (*PFN_tmapEncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                        const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                        CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static PFN_tmapEncodeTiled get_encode_fn() {
-    static PFN_tmapEncodeTiled fn = nullptr;
-    if (fn) return fn;
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) != cudaSuccess || qres != cudaDriverEntryPointSuccess)
-        return nullptr;
-    fn = (PFN_tmapEncodeTiled)p;
-    return fn;
-}
-
-}  // namespace tc
-
-// bf16 tiled tensor map, rank 2 or 3; swizzle: 0 none (plain row tiles), 1 SWIZZLE_128B (UMMA operands, 64-column store
-// boxes), 2 SWIZZLE_64B (32-column store boxes)
-int encode_tmap_bf16(CUtensorMap* map, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
-                     const cuuint32_t* box, int swizzle) {
-    tc::PFN_tmapEncodeTiled fn = tc::get_encode_fn();
-    if (!fn) return fail_msg(TRIAD_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
-    cuuint32_t estr[3] = {1, 1, 1};
-    const CUtensorMapSwizzle sw = swizzle == 1 ? CU_TENSOR_MAP_SWIZZLE_128B : swizzle == 2 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_NONE;
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        char buf[96];
-        snprintf(buf, sizeof buf, "cuTensorMapEncodeTiled failed (CUresult %d)", (int)r);
-        return fail_msg(TRIAD_ERR_CUDA, buf);
-    }
-    return TRIAD_OK;
-}
-
-// fp32, rank 3, SWIZZLE_128B (32-column boxes: the fp32 partial tiles of dense_gemm.cu)
-int encode_tmap_f32_3d(CUtensorMap* map, const void* base, const cuuint64_t* dims, const cuuint64_t* strides, const cuuint32_t* box) {
-    tc::PFN_tmapEncodeTiled fn = tc::get_encode_fn();
-    if (!fn) return fail_msg(TRIAD_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(base), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        char buf[96];
-        snprintf(buf, sizeof buf, "cuTensorMapEncodeTiled (fp32) failed (CUresult %d)", (int)r);
-        return fail_msg(TRIAD_ERR_CUDA, buf);
-    }
-    return TRIAD_OK;
-}
-
-namespace tc {
-
-static int encode_map(CUtensorMap* map, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
-                      const cuuint32_t* box) {
-    return encode_tmap_bf16(map, base, rank, dims, strides, box, true);
-}
-
-// uint8 (e4m3 codes) tiled tensor map, SWIZZLE_128B: 128-element (128-byte) inner box
-static int encode_map_u8(CUtensorMap* map, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
-                         const cuuint32_t* box) {
-    PFN_tmapEncodeTiled fn = get_encode_fn();
-    if (!fn) return fail_msg(TRIAD_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, (cuuint32_t)rank, const_cast<void*>(base), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        char buf[96];
-        snprintf(buf, sizeof buf, "cuTensorMapEncodeTiled (uint8) failed (CUresult %d)", (int)r);
-        return fail_msg(TRIAD_ERR_CUDA, buf);
-    }
-    return TRIAD_OK;
-}
-
 // Tile order (TileIter).  V up to ~48 MB: any order, V stays in L2.  Larger: if there are enough query tiles to
 // give every cluster a few items per ~16 MB image chunk, ALL clusters walk the same chunk at the same time —
 // V is read from HBM once per pass whatever its size (cfg 4: 2.1 GB), and even at cfg 2 (67 MB, nominally
@@ -879,53 +803,46 @@ static void pick_tile_order(Params& p, size_t img_bytes, int Bv, int n_m, int n_
 template <int kCtaGroup, bool kSub, int kMode = 0, bool kFp8 = false>
 static int launch_t(const CUtensorMap& mq, const CUtensorMap& mv, const CUtensorMap& mn, const Params& p, int n_clusters,
                     cudaStream_t st) {
-    auto kern = maxmean_tc_kernel<kCtaGroup, kSub, kMode, kFp8>;
-    TRIAD_SET_MAX_SMEM(kern, kSmemBytes);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(n_clusters * kCtaGroup));
-    cfg.blockDim = dim3(kEmitThreads);
-    cfg.dynamicSmemBytes = kSmemBytes;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = kCtaGroup;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    TRIAD_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kern, mq, mv, mn, p));
-    count_launch();
-    return TRIAD_OK;
+    return launch_clusters<maxmean_tc_kernel<kCtaGroup, kSub, kMode, kFp8>>(kCtaGroup, n_clusters, kEmitThreads, kSmemBytes,
+                                                                            st, mq, mv, mn, p);
 }
 
 }  // namespace tc
 
 bool tc_supported(int Nv, int D) { return Nv >= 1 && Nv <= 65535 && D % tc::kBlockK == 0 && D >= tc::kBlockK && D <= tc::kMaxKB * tc::kBlockK; }
+bool tc_emit_supported(int Nv, int D) { return tc_supported(Nv, D) && Nv <= tc::kMaxN && Nv % 8 == 0; }
+bool tc_e4m3_supported(int Nv, int D) { return Nv >= 1 && Nv <= 65535 && D % 128 == 0 && D >= 128 && D <= 512; }
 
 int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, const float* T,
                       int inv_T, int M, int Bv, int Nq, int Nv, int D,
                       float* part, void* idx, int* abort_flag, int cta_group, int flags, const int* pack_maps,
-                      const EmitNArgs* emit, cudaStream_t st) {
+                      const EmitNArgs* emit, const E4m3Args* e4m3, cudaStream_t st) {
     using namespace tc;
-    if (!tc_supported(Nv, D)) return fail_msg(TRIAD_ERR_UNSUPPORTED, "tcgen05 forward: needs D in {64,...,512} (multiple of 64)");
+    if (e4m3 ? !tc_e4m3_supported(Nv, D) : !tc_supported(Nv, D))
+        return fail_msg(TRIAD_ERR_UNSUPPORTED, e4m3 ? "tcgen05 e4m3 forward: needs D in {128, 256, 384, 512}"
+                                                    : "tcgen05 forward: needs D in {64,...,512} (multiple of 64)");
     const int tile_rows = kBlockM * cta_group;
     const int n_m = ceil_div(M, tile_rows);
     const int n_sub = ceil_div(Nv, kMaxN);
     if ((long long)n_m * Bv * n_sub >= 0x7fffffffLL) return fail_msg(TRIAD_ERR_UNSUPPORTED, "tcgen05 forward: too many tiles");
 
-    int dev = 0, sms = 0;
-    TRIAD_CUDA_CHECK(cudaGetDevice(&dev));
-    TRIAD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    int rc = device_sms(&sms);
+    if (rc) return rc;
 
+    // one 128-byte swizzle row of a k-block holds 64 bf16 or 128 e4m3 elements
+    const int elt = e4m3 ? 1 : 2, kb_elems = 128 / elt;
+    const CUtensorMapDataType ttype = e4m3 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
     Params p;
+    memset(&p, 0, sizeof p);
     p.M = M; p.Bv = Bv; p.Nq = Nq; p.Nv = Nv;
     p.n_umma = n_sub > 1 ? kMaxN : (Nv + 15) / 16 * 16;
     p.n_sub = n_sub;
-    p.idx16 = Nv > 256;
-    p.num_kb = D / kBlockK;
+    p.idx16 = !e4m3 && Nv > 256;
+    p.num_kb = D / kb_elems;
     p.n_m = n_m;
     int n_clusters = sms / cta_group;
-    pick_tile_order(p, (size_t)Nv * D * 2, Bv, n_m, n_clusters);
+    pick_tile_order(p, (size_t)Nv * D * elt, Bv, n_m, n_clusters);
     if (flags & TRIAD_FWD_SYNC_CHUNKS) { p.C = Bv < 3 ? Bv : 3; p.sync = 1; }     // tests: tiny chunks on small shapes
     PartLayout pl = part_layout(M, Nq);
     p.G = pl.G; p.S = pl.S;
@@ -936,29 +853,27 @@ int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, cons
     p.pack_off = pack_maps;                                   // q then points at the PACKED rows
     p.rowmap = pack_maps ? pack_maps + p.Bq + 1 : nullptr;
     p.pieces = packed_pieces(Nq);
-    p.n_out = nullptr; p.ldn = 0; p.lo = 0.f; p.coef = 0.f; p.write_n = 0; p.n_partials = nullptr;
-    p.col_scale = nullptr; p.q_scale = nullptr;
     if (emit) {
-        if (n_sub > 1 || Nv % 8 != 0 || pack_maps) return fail_msg(TRIAD_ERR_UNSUPPORTED, "dense-regulariser forward: needs Nv <= 256, Nv % 8 == 0");
+        if (!tc_emit_supported(Nv, D) || pack_maps) return fail_msg(TRIAD_ERR_UNSUPPORTED, "dense-regulariser forward: needs Nv <= 256, Nv % 8 == 0");
         if (emit->with_maxmean && (!idx || !part || inv_T)) return fail_msg(TRIAD_ERR_BAD_ARG, "dense-regulariser + max-mean forward: needs idx and the partial buffer");
+        if (sms * kEmitEpiWarps > kNonnegFusedPartials) return fail_msg(TRIAD_ERR_UNSUPPORTED, "dense-regulariser forward: too many SMs for the partial buffer");
         p.n_out = (__nv_bfloat16*)emit->n_out; p.ldn = emit->ldn; p.lo = emit->lo; p.coef = emit->coef;
         p.write_n = emit->write_n; p.n_partials = emit->partials;
     }
+    if (e4m3) { p.col_scale = e4m3->g_scale; p.q_scale = e4m3->q_scale; }
 
     CUtensorMap mq, mv;
     {
         cuuint64_t dims[2] = {(cuuint64_t)D, (cuuint64_t)M};
-        cuuint64_t strides[1] = {(cuuint64_t)D * 2};
-        cuuint32_t box[2] = {(cuuint32_t)kBlockK, (cuuint32_t)kBlockM};
-        int rc = encode_map(&mq, q, 2, dims, strides, box);
-        if (rc) return rc;
+        cuuint64_t strides[1] = {(cuuint64_t)D * elt};
+        cuuint32_t box[2] = {(cuuint32_t)kb_elems, (cuuint32_t)kBlockM};
+        if ((rc = encode_tmap(&mq, ttype, q, 2, dims, strides, box, Swizzle::k128B))) return rc;
     }
     {
         cuuint64_t dims[3] = {(cuuint64_t)D, (cuuint64_t)Nv, (cuuint64_t)Bv};
-        cuuint64_t strides[2] = {(cuuint64_t)D * 2, (cuuint64_t)Nv * D * 2};
-        cuuint32_t box[3] = {(cuuint32_t)kBlockK, (cuuint32_t)(p.n_umma / cta_group), 1};
-        int rc = encode_map(&mv, v, 3, dims, strides, box);
-        if (rc) return rc;
+        cuuint64_t strides[2] = {(cuuint64_t)D * elt, (cuuint64_t)Nv * D * elt};
+        cuuint32_t box[3] = {(cuuint32_t)kb_elems, (cuuint32_t)(p.n_umma / cta_group), 1};
+        if ((rc = encode_tmap(&mv, ttype, v, 3, dims, strides, box, Swizzle::k128B))) return rc;
     }
     // N[row][image][patch] as a rank-3 tensor {Nv, images, M} (row pitch ldn): the epilogue's 32-row x 64-column store
     // boxes are clipped at the image's last patch and at the last row by the TMA unit itself
@@ -967,8 +882,7 @@ int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, cons
         cuuint64_t dims[3] = {(cuuint64_t)Nv, (cuuint64_t)Bv, (cuuint64_t)M};
         cuuint64_t strides[2] = {(cuuint64_t)Nv * 2, (cuuint64_t)emit->ldn * 2};
         cuuint32_t box[3] = {64, 1, 32};
-        int rc = encode_tmap_bf16(&mn, emit->n_out, 3, dims, strides, box, 1);
-        if (rc) return rc;
+        if ((rc = encode_tmap(&mn, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, emit->n_out, 3, dims, strides, box, Swizzle::k128B))) return rc;
     }
     const long long total = (long long)n_m * Bv;
     if ((long long)n_clusters > total) n_clusters = (int)total;
@@ -977,70 +891,17 @@ int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, cons
         // one slot per epilogue warp of every CTA, written only by the emission warps of CTAs that get work: clear all
         TRIAD_CUDA_CHECK(cudaMemsetAsync(emit->partials, 0, (size_t)sms * kEmitEpiWarps * 2 * sizeof(double), st));
         if (emit->with_maxmean)
-            return cta_group == 2 ? launch_t<2, false, 2>(mq, mv, mn, p, n_clusters, st) : launch_t<1, false, 2>(mq, mv, mn, p, n_clusters, st);
-        return cta_group == 2 ? launch_t<2, false, 1>(mq, mv, mn, p, n_clusters, st) : launch_t<1, false, 1>(mq, mv, mn, p, n_clusters, st);
+            rc = cta_group == 2 ? launch_t<2, false, 2>(mq, mv, mn, p, n_clusters, st) : launch_t<1, false, 2>(mq, mv, mn, p, n_clusters, st);
+        else
+            rc = cta_group == 2 ? launch_t<2, false, 1>(mq, mv, mn, p, n_clusters, st) : launch_t<1, false, 1>(mq, mv, mn, p, n_clusters, st);
+        return rc ? rc : launch_nonneg_finish(emit->partials, sms * kEmitEpiWarps, emit->sums, st);
     }
-    if (n_sub > 1) return cta_group == 2 ? launch_t<2, true>(mq, mv, mn, p, n_clusters, st) : launch_t<1, true>(mq, mv, mn, p, n_clusters, st);
-    return cta_group == 2 ? launch_t<2, false>(mq, mv, mn, p, n_clusters, st) : launch_t<1, false>(mq, mv, mn, p, n_clusters, st);
-}
-
-bool tc_e4m3_supported(int Nv, int D) { return Nv >= 1 && Nv <= 65535 && D % 128 == 0 && D >= 128 && D <= 512; }
-
-int launch_maxmean_tc_e4m3(const void* q_codes, const float* q_scale, const void* g_codes, const float* g_scale,
-                           const float* row_scale, const float* T, int M, int Bv, int Nq, int Nv, int D,
-                           float* part, int* abort_flag, cudaStream_t st) {
-    using namespace tc;
-    if (!tc_e4m3_supported(Nv, D)) return fail_msg(TRIAD_ERR_UNSUPPORTED, "tcgen05 e4m3 forward: needs D in {128, 256, 384, 512}");
-    // one row tile of <= 128 tokens: cta_group::1, as for bf16 (fwd_impl)
-    const int cta_group = M <= 128 ? 1 : 2;
-    const int tile_rows = kBlockM * cta_group;
-    const int n_m = ceil_div(M, tile_rows);
-    const int n_sub = ceil_div(Nv, kMaxN);
-    if ((long long)n_m * Bv * n_sub >= 0x7fffffffLL) return fail_msg(TRIAD_ERR_UNSUPPORTED, "tcgen05 e4m3 forward: too many tiles");
-
-    int dev = 0, sms = 0;
-    TRIAD_CUDA_CHECK(cudaGetDevice(&dev));
-    TRIAD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-
-    Params p;
-    memset(&p, 0, sizeof p);
-    p.M = M; p.Bv = Bv; p.Nq = Nq; p.Nv = Nv;
-    p.n_umma = n_sub > 1 ? kMaxN : (Nv + 15) / 16 * 16;
-    p.n_sub = n_sub;
-    p.num_kb = D / 128;
-    p.n_m = n_m;
-    int n_clusters = sms / cta_group;
-    pick_tile_order(p, (size_t)Nv * D, Bv, n_m, n_clusters);      // an e4m3 image is Nv*D bytes
-    PartLayout pl = part_layout(M, Nq);
-    p.G = pl.G; p.S = pl.S;
-    p.nq_pad = nq_padded(Nq);
-    p.inv_T = 1;                                                    // retrieval divides by T
-    p.row_scale = row_scale; p.T = T; p.part = part; p.idx = nullptr; p.abort_flag = abort_flag;
-    p.Bq = M / Nq;
-    p.pieces = packed_pieces(Nq);
-    p.col_scale = g_scale; p.q_scale = q_scale;
-
-    CUtensorMap mq, mv;
-    {
-        cuuint64_t dims[2] = {(cuuint64_t)D, (cuuint64_t)M};
-        cuuint64_t strides[1] = {(cuuint64_t)D};
-        cuuint32_t box[2] = {128u, (cuuint32_t)kBlockM};
-        int rc = encode_map_u8(&mq, q_codes, 2, dims, strides, box);
-        if (rc) return rc;
+    if (!e4m3) {
+        if (n_sub > 1) return cta_group == 2 ? launch_t<2, true>(mq, mv, mn, p, n_clusters, st) : launch_t<1, true>(mq, mv, mn, p, n_clusters, st);
+        return cta_group == 2 ? launch_t<2, false>(mq, mv, mn, p, n_clusters, st) : launch_t<1, false>(mq, mv, mn, p, n_clusters, st);
     }
-    {
-        cuuint64_t dims[3] = {(cuuint64_t)D, (cuuint64_t)Nv, (cuuint64_t)Bv};
-        cuuint64_t strides[2] = {(cuuint64_t)D, (cuuint64_t)Nv * D};
-        cuuint32_t box[3] = {128u, (cuuint32_t)(p.n_umma / cta_group), 1};
-        int rc = encode_map_u8(&mv, g_codes, 3, dims, strides, box);
-        if (rc) return rc;
-    }
-    const long long total = (long long)n_m * Bv;
-    if ((long long)n_clusters > total) n_clusters = (int)total;
-    if (n_clusters < 1) n_clusters = 1;
-    if (n_sub > 1)
-        return cta_group == 2 ? launch_t<2, true, 0, true>(mq, mv, mq, p, n_clusters, st) : launch_t<1, true, 0, true>(mq, mv, mq, p, n_clusters, st);
-    return cta_group == 2 ? launch_t<2, false, 0, true>(mq, mv, mq, p, n_clusters, st) : launch_t<1, false, 0, true>(mq, mv, mq, p, n_clusters, st);
+    if (n_sub > 1) return cta_group == 2 ? launch_t<2, true, 0, true>(mq, mv, mn, p, n_clusters, st) : launch_t<1, true, 0, true>(mq, mv, mn, p, n_clusters, st);
+    return cta_group == 2 ? launch_t<2, false, 0, true>(mq, mv, mn, p, n_clusters, st) : launch_t<1, false, 0, true>(mq, mv, mn, p, n_clusters, st);
 }
 
 }  // namespace triad

@@ -654,7 +654,7 @@ patch_expand_kernel(const uint4* __restrict__ gy, const uint8_t* __restrict__ ke
 
 using namespace triad;
 
-extern "C" size_t triad_project_workspace_bytes(void) { return 256; }
+extern "C" size_t triad_project_workspace_bytes(void) { return kCtrlBlockBytes; }
 
 extern "C" int triad_project_tokens(const void* x, const void* w1, const float* b1, const float* ln_g, const float* ln_b,
                                     float ln_eps, const void* w2, const float* b2, int M, int Din, int Dout, int l2_normalize,
@@ -665,29 +665,29 @@ extern "C" int triad_project_tokens(const void* x, const void* w1, const float* 
     if (Din % kBlockK != 0 || Dout % 16 != 0 || Dout > kHidden)
         return fail_msg(TRIAD_ERR_UNSUPPORTED, "project_tokens: needs Din % 64 == 0, Dout % 16 == 0, Dout <= 512 (hidden width is 512)");
     if (((uintptr_t)x | (uintptr_t)w1 | (uintptr_t)w2 | (uintptr_t)out | (uintptr_t)ws) & 15) return fail_msg(TRIAD_ERR_ALIGNMENT, "project_tokens: 16-byte alignment");
-    if (ws_bytes < 256) return fail_msg(TRIAD_ERR_WORKSPACE, "project_tokens: workspace too small");
+    if (ws_bytes < kCtrlBlockBytes) return fail_msg(TRIAD_ERR_WORKSPACE, "project_tokens: workspace too small");
     cudaStream_t st = (cudaStream_t)stream;
-    TRIAD_CUDA_CHECK(cudaMemsetAsync(ws, 0, 256, st));
+    TRIAD_CUDA_CHECK(cudaMemsetAsync(ws, 0, kCtrlBlockBytes, st));
     CUtensorMap mx, mw1, mw2;
     {
         cuuint64_t dims[2] = {(cuuint64_t)Din, (cuuint64_t)M};
         cuuint64_t strides[1] = {(cuuint64_t)Din * 2};
         cuuint32_t box[2] = {(cuuint32_t)kBlockK, (cuuint32_t)kBlockM};
-        int rc = encode_tmap_bf16(&mx, x, 2, dims, strides, box, true);
+        int rc = encode_tmap(&mx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, x, 2, dims, strides, box, Swizzle::k128B);
         if (rc) return rc;
     }
     {
         cuuint64_t dims[2] = {(cuuint64_t)Din, (cuuint64_t)kHidden};
         cuuint64_t strides[1] = {(cuuint64_t)Din * 2};
         cuuint32_t box[2] = {(cuuint32_t)kBlockK, (cuuint32_t)kHalfN};
-        int rc = encode_tmap_bf16(&mw1, w1, 2, dims, strides, box, true);
+        int rc = encode_tmap(&mw1, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, w1, 2, dims, strides, box, Swizzle::k128B);
         if (rc) return rc;
     }
     {
         cuuint64_t dims[2] = {(cuuint64_t)kHidden, (cuuint64_t)Dout};
         cuuint64_t strides[1] = {(cuuint64_t)kHidden * 2};
         cuuint32_t box[2] = {(cuuint32_t)kBlockK, (cuuint32_t)kHalfN};
-        int rc = encode_tmap_bf16(&mw2, w2, 2, dims, strides, box, true);
+        int rc = encode_tmap(&mw2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, w2, 2, dims, strides, box, Swizzle::k128B);
         if (rc) return rc;
     }
     Params p;
@@ -704,7 +704,7 @@ struct BwdWs { size_t gh, ln, part, gemm, total; };
 static BwdWs bwd_ws_layout(int M, int Din, int Dout) {
     using namespace proj;
     BwdWs w;
-    w.gh = 256;
+    w.gh = kCtrlBlockBytes;
     w.ln = w.gh + align_up((size_t)M * kHidden * 2, 256);
     w.part = w.ln + align_up((size_t)M * kHidden * 2, 256);
     w.gemm = w.part + align_up((size_t)ceil_div(M, kBlockM) * kPartRows * kHidden * 4, 256);
@@ -742,32 +742,32 @@ extern "C" int triad_project_tokens_bwd(const void* x, const void* w1, const flo
     __nv_bfloat16* gh = (__nv_bfloat16*)(wsb + L.gh);
     __nv_bfloat16* ln = (__nv_bfloat16*)(wsb + L.ln);
     float* part = (float*)(wsb + L.part);
-    TRIAD_CUDA_CHECK(cudaMemsetAsync(ws, 0, 256, st));
+    TRIAD_CUDA_CHECK(cudaMemsetAsync(ws, 0, kCtrlBlockBytes, st));
     CUtensorMap mx, mw1, mgy, mw2;
     int rc;
     {
         cuuint64_t dims[2] = {(cuuint64_t)Din, (cuuint64_t)M};
         cuuint64_t strides[1] = {(cuuint64_t)Din * 2};
         cuuint32_t box[2] = {(cuuint32_t)kBlockK, (cuuint32_t)kBlockM};
-        if ((rc = encode_tmap_bf16(&mx, x, 2, dims, strides, box, true))) return rc;
+        if ((rc = encode_tmap(&mx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, x, 2, dims, strides, box, Swizzle::k128B))) return rc;
     }
     {
         cuuint64_t dims[2] = {(cuuint64_t)Din, (cuuint64_t)kHidden};
         cuuint64_t strides[1] = {(cuuint64_t)Din * 2};
         cuuint32_t box[2] = {(cuuint32_t)kBlockK, (cuuint32_t)kHalfN};
-        if ((rc = encode_tmap_bf16(&mw1, w1, 2, dims, strides, box, true))) return rc;
+        if ((rc = encode_tmap(&mw1, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, w1, 2, dims, strides, box, Swizzle::k128B))) return rc;
     }
     {                      // gy as GEMM 2's K-major A operand: {64 k, 128 rows}
         cuuint64_t dims[2] = {(cuuint64_t)Dout, (cuuint64_t)M};
         cuuint64_t strides[1] = {(cuuint64_t)Dout * 2};
         cuuint32_t box[2] = {(cuuint32_t)kBlockK, (cuuint32_t)kBlockM};
-        if ((rc = encode_tmap_bf16(&mgy, gy, 2, dims, strides, box, true))) return rc;
+        if ((rc = encode_tmap(&mgy, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, gy, 2, dims, strides, box, Swizzle::k128B))) return rc;
     }
     {                      // W2 [Dout][512] as the MN-major B operand: {64 n, 64 k}
         cuuint64_t dims[2] = {(cuuint64_t)kHidden, (cuuint64_t)Dout};
         cuuint64_t strides[1] = {(cuuint64_t)kHidden * 2};
         cuuint32_t box[2] = {64, 64};
-        if ((rc = encode_tmap_bf16(&mw2, w2, 2, dims, strides, box, true))) return rc;
+        if ((rc = encode_tmap(&mw2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, w2, 2, dims, strides, box, Swizzle::k128B))) return rc;
     }
     BwdParams p;
     p.b1 = b1; p.ln_g = ln_g; p.ln_b = ln_b; p.gy = (const __nv_bfloat16*)gy;

@@ -6,11 +6,6 @@
 #include <stdint.h>
 
 namespace triad {
-
-// host: bf16 tiled tensor map (defined in maxmean_tc.cu)
-int encode_tmap_bf16(CUtensorMap* map, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
-                     const cuuint32_t* box, int swizzle /* 0: none, 1: SWIZZLE_128B, 2: SWIZZLE_64B */);
-
 namespace ptx {
 
 constexpr unsigned long long kWatchdogNs = 4000000000ull;
