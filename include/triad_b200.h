@@ -255,6 +255,33 @@ size_t triad_retrieve_e4m3_workspace_bytes(int Nq, int n_img, int Nv, int D);
 int triad_retrieve_scores_e4m3(const void* q_codes, const float* q_scales, int Nq, const void* g_codes,
                                const float* g_scales, int n_img, int Nv, int D, const float* temperature,
                                float* scores, void* ws, size_t ws_bytes, void* stream);
+/* ---- retrieval on a ragged caption gallery (bf16, items of 1..256 tokens) ------------------------------------
+ * Layout: the captions' token rows in 256-row slots, slots [n_slots * 256][D] bf16.  Captions are placed greedily
+ * in order; one that does not fit in the rest of the current slot starts a new slot (no caption straddles a slot);
+ * the rows after a slot's last caption are zero.
+ * triad_ragged_plan (host only, no CUDA call): from lengths[n_cap] (host, each 1..256, else TRIAD_ERR_BAD_SHAPE)
+ * writes the host arrays slot_meta [n_slots][20] int32 = {first caption id, caption count, used rows, 0,
+ * caption-start mask [8] (bit r%32 of word r/32: a caption starts at row r), caption-end mask [8] (its last row)}
+ * and cap_info [n_cap][2] int32 = {first row (slot * 256 + offset), length}, and *n_slots.  slot_meta needs room
+ * for n_cap slots (the most there can be). */
+int triad_ragged_plan(const int32_t* lengths, int n_cap, int32_t* slot_meta, int32_t* cap_info, int* n_slots);
+/* dst[r] = bf16(src[rowmap[r]]) for r < dst_rows (a multiple of 256), a zero row where rowmap[r] < 0 or
+ * rowmap[r] >= src_rows; src [src_rows][D] fp32 or bf16 (dtype), D % 8 == 0, src and dst 16-byte aligned. */
+int triad_ragged_pack(const void* src, int dtype, long long src_rows, int D, const int32_t* rowmap, long long dst_rows,
+                      void* dst, void* stream);
+/* scores[c] for one query q [Nq][D] bf16 against the n_cap captions of a ragged gallery (slot_meta and cap_info as
+ * triad_ragged_plan wrote them, on the device), divided by T:
+ *   direction 0: mean over the query's tokens of the max over caption c's tokens (the V->T ranking, the
+ *                reference's aggregator_tv_v2t with the image as query);
+ *   direction 1: mean over caption c's tokens of the max over the query's tokens (aggregator_tv_t2v).
+ * Each similarity is rounded as the dense retrieval forward rounds it, bf16(bf16(acc) * (1/T)).  The sums are
+ * deterministic (fixed-order partials, no float atomics) and do not depend on where a caption sits in the slots.  D in {64, ..., 512} (multiple of 64,
+ * TRIAD_ERR_UNSUPPORTED otherwise), 1 <= Nq <= 65535; q, slots and ws 16-byte aligned.  No host synchronisation;
+ * a watchdog timeout gives NaN scores. */
+size_t triad_retrieve_ragged_workspace_bytes(int Nq, int n_slots, int n_cap, int direction);
+int triad_retrieve_scores_ragged(const void* q, int Nq, const void* slots, const int32_t* slot_meta,
+                                 const int32_t* cap_info, int n_slots, int n_cap, int D, const float* temperature,
+                                 int direction, float* scores, void* ws, size_t ws_bytes, void* stream);
 /* top-k of scores (descending, ties -> lower id first, like a stable argsort of -scores;
  * -0.0 and +0.0 are equal scores): out_scores fp32 [k] = scores[out_ids], bit for bit,
  * out_ids int32 [k].  NaN scores have no defined place.  ws: triad_topk_workspace_bytes(n). */

@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIBNAME = "libtriad_b200.so"
 
-SOURCES = ["capi.cu", "maxmean_simt.cu", "maxmean_tc.cu", "infonce.cu", "maxmean_bwd.cu", "bwd_dq_tile.cu", "bwd_dq_pipe.cu", "retrieve.cu", "dense_reg.cu", "pack.cu", "proj_head.cu", "pospair.cu", "dense_gemm.cu", "quant_e4m3.cu", "tmap.cu"]
+SOURCES = ["capi.cu", "maxmean_simt.cu", "maxmean_tc.cu", "infonce.cu", "maxmean_bwd.cu", "bwd_dq_tile.cu", "bwd_dq_pipe.cu", "retrieve.cu", "dense_reg.cu", "pack.cu", "proj_head.cu", "pospair.cu", "dense_gemm.cu", "quant_e4m3.cu", "tmap.cu", "ragged.cu"]
 HEADERS = ["common.cuh", "ptx.cuh", "triad_round.h", os.path.join("..", "..", "include", "triad_b200.h")]
 
 NVCC_FLAGS = [

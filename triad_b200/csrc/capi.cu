@@ -97,7 +97,7 @@ extern "C" size_t triad_maxmean_fwd_workspace_bytes(int Bq, int Bv, int Nq, int 
 // cta_group of the unpacked tcgen05 forwards.  A single row tile of <= 128 tokens (one text query against a gallery):
 // cta_group::1 — a pair would spend a 256-row MMA on <= 128 rows, and at one tile per image that MMA time equals the
 // HBM time of the image, leaving no slack to overlap; alone, each SM streams its own images at twice that rate.
-static int fwd_cta_group(int M, int flags) { return ((flags & TRIAD_FWD_FORCE_1CTA) || M <= 128) ? 1 : 2; }
+int triad::fwd_cta_group(int M, int flags) { return ((flags & TRIAD_FWD_FORCE_1CTA) || M <= 128) ? 1 : 2; }
 
 static int fwd_impl(const void* q, const void* v, const float* row_scale, const float* temperature, int inv_T,
                     int Bq, int Bv, int Nq, int Nv, int D, int dtype, float* clip, void* idx,

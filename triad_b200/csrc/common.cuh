@@ -133,10 +133,22 @@ bool tc_emit_supported(int Nv, int D);
 // (g_scale [Bv][Nv]); divides by T, no idx, D in {128, 256, 384, 512}
 struct E4m3Args { const float* q_scale; const float* g_scale; };
 bool tc_e4m3_supported(int Nv, int D);
+// ragged caption gallery (ragged.cu): captions packed whole into kSlotRows-row slots, zero rows at a slot's end.
+// slot_meta [slots][kSlotMetaInts] int32: first caption id, caption count, used rows, 0, the caption-start mask (bit
+// r of word r/32 = a caption starts at row r), the caption-end mask (its last row); cap_info [captions][2] int32:
+// first row (slot * kSlotRows + offset), length (1..kSlotRows)
+constexpr int kSlotRows = 256;
+constexpr int kSlotMetaCap0 = 0, kSlotMetaCount = 1, kSlotMetaUsed = 2, kSlotMetaStarts = 4, kSlotMetaEnds = 12;
+constexpr int kSlotMetaInts = 20;
+// direction 0: q = the query's tokens, v = the slots (Bv = slots, Nv = kSlotRows), partials part[caption][group];
+// direction 1: q = the slot rows (M = slots * kSlotRows), v = the query (Bv = 1), one weighted row max per slot row
+struct RaggedArgs { const int* slot_meta; const int* cap_info; int direction; };
 int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, const float* T,
                       int inv_T, int M, int Bv, int Nq, int Nv, int D,
                       float* part, void* idx, int* abort_flag, int cta_group, int flags, const int* pack_maps,
-                      const EmitNArgs* emit, const E4m3Args* e4m3, cudaStream_t st);
+                      const EmitNArgs* emit, const E4m3Args* e4m3, cudaStream_t st, const RaggedArgs* ragged = nullptr);
+// cta_group of the unpacked tcgen05 forwards (capi.cu)
+int fwd_cta_group(int M, int flags);
 // sums[0..1] += the per-warp partials of a dense-regulariser forward, in slot order (dense_reg.cu)
 int launch_nonneg_finish(const double* partials, int n, double* sums, cudaStream_t st);
 int launch_finalize_clip(const float* part, int Bq, int Bv, int Nq, float* clip, const int* abort_flag, cudaStream_t st);

@@ -86,6 +86,10 @@ struct Params {
     // kFp8 (e4m3 retrieval): per-patch scales [Bv][Nv] of the gallery codes, per-token scales [M] of the query codes
     const float* col_scale;
     const float* q_scale;
+    // kMode 3 / 4 (ragged caption gallery, ragged.cu): per-slot metadata [slots][kSlotMetaInts] and per-caption
+    // {first slot row, length} [captions]
+    const int* slot_meta;
+    const int* cap_info;
 };
 
 __device__ __forceinline__ float fmax3(float a, float b, float c) { return fmaxf(fmaxf(a, b), c); }
@@ -151,6 +155,44 @@ __device__ __forceinline__ void first_ge32(const uint32_t (&r)[32], int col0, in
     }
     const int lo = min(min(b[0], b[1]), min(b[2], b[3]));
     if (lo < min(lim, 32)) best = col0 + lo;            // 64 = "none"; columns >= lim are padding
+}
+
+// ---- ragged caption gallery, direction 0 (kMode 3): segmented row maximum over one 256-row slot -------------------
+// r[b] of a 32-column chunk, b warp-uniform but not a compile-time constant: a five-level select tree keeps r in
+// registers (an indexed access would put it in local memory)
+__device__ __forceinline__ float pick32(const uint32_t (&r)[32], int b) {
+    uint32_t a[16];
+#pragma unroll
+    for (int i = 0; i < 16; ++i) a[i] = (b & 1) ? r[2 * i + 1] : r[2 * i];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) a[i] = (b & 2) ? a[2 * i + 1] : a[2 * i];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) a[i] = (b & 4) ? a[2 * i + 1] : a[2 * i];
+#pragma unroll
+    for (int i = 0; i < 2; ++i) a[i] = (b & 8) ? a[2 * i + 1] : a[2 * i];
+    return __uint_as_float((b & 16) ? a[1] : a[0]);
+}
+// One 32-column chunk of the slot: `starts` / `ends` are the chunk's words of the slot's caption-start and
+// caption-end masks (warp-uniform).  A running maximum restarts at every caption start; r[i] becomes the maximum of
+// the open caption up to column i, so at every end column it is that caption's row maximum.  Each caption that ends
+// in the chunk is weighted (val = round_sim(max) * row weight, as the dense epilogue) and reduced over the warp's 32
+// query rows into its partial part[caption][32-row group] (store_group_partials with one slot per group), captions
+// numbered from `cap` in slot order.
+__device__ __forceinline__ void ragged_chunk(uint32_t (&r)[32], uint32_t starts, uint32_t ends, float& run, int& cap,
+                                             bool valid, float Tval, float rs, const Params& p, int row0, int lane) {
+#pragma unroll
+    for (int i = 0; i < 32; ++i) {
+        const float x = __uint_as_float(r[i]);
+        run = ((starts >> i) & 1u) ? x : fmaxf(run, x);
+        r[i] = __float_as_uint(run);
+    }
+    while (ends != 0u) {                                    // warp-uniform: one iteration per caption ending here
+        const int b = __ffs(ends) - 1;
+        ends &= ends - 1u;
+        const float val = valid ? round_sim<true>(pick32(r, b), Tval) * rs : 0.f;
+        store_group_partials(p.part, cap, row0 >> 5, p.G, 1, row0, p.M, p.Nq, val, lane);
+        ++cap;
+    }
 }
 
 // ---- dense-regulariser epilogue (kMode 1: instead of the max-mean reduction; kMode 2: next to it) -----------------
@@ -340,18 +382,33 @@ struct TileIter {
 // patch scale before the max and the row by t_a = fp32(fp32(q_scale * row_scale) * (1/T)) after it.  The scales of
 // the current 256-patch sub-tile are staged per epilogue warp in the upper half of the query region (num_kb <= 4
 // leaves it unused).
+// kMode 3 / 4: a ragged caption gallery (ragged.cu), stored as 256-row slots that each hold whole captions.
+//   kMode 3 (direction 0: mean over the query's tokens of the max over each caption's tokens): rows = the query's
+//   tokens, "images" = the slots (Nv = 256).  The epilogue walks each row's 256 columns with a running maximum that
+//   restarts at every caption start (ragged_chunk) and reduces each caption's row maxima over the warp's 32 rows into
+//   part[caption][group]; no idx.
+//   kMode 4 (direction 1: mean over each caption's tokens of the max over the query's tokens): rows = the slot rows,
+//   the one "image" = the query (sub-tiles when it has more than 256 tokens).  The row's caption and its weight
+//   1/length come from the slot metadata in place (the gallery is not copied); each slot row's weighted maximum is
+//   stored as it is, part[row] (the zero rows at a slot's end store nothing), and the finalize sums each caption's
+//   rows in token order.  A warp reduction would add a caption's rows in an order set by its offset within a 32-row
+//   group, so the same caption packed after another prefix could score differently in the last bit; this order
+//   depends on the caption alone.  cta_group::2 only (the rows are whole 256-row slots).
+constexpr int kModeRaggedMax = 3, kModeRaggedMean = 4;
 template <int kCtaGroup, bool kSub, int kMode = 0, bool kFp8 = false>
 __global__ void __launch_bounds__(kEmitThreads, 1)
 maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_v,
                   const __grid_constant__ CUtensorMap tmap_n, const Params p) {
     static_assert(!kFp8 || kMode == 0, "the e4m3 forward is the max-mean reduction only");
-    constexpr bool kEmitN = kMode != 0;
+    static_assert(kMode != kModeRaggedMax || !kSub, "ragged direction 0: one 256-row slot per tile");
+    constexpr bool kEmitN = kMode == 1 || kMode == 2;
+    constexpr bool kRagged = kMode == kModeRaggedMax || kMode == kModeRaggedMean;
     constexpr int kKbElems = kFp8 ? 128 : kBlockK;                          // elements per 128-byte k-block row
     constexpr int kVStageBytes = (kMaxN / kCtaGroup) * kBlockK * 2;       // 32 KB / 16 KB
     // the dense-regulariser modes give the last 32 KB of the ring to the epilogue's store staging: four emission warps x
     // two 4 KB boxes (32 rows x 64 columns).  (Two 2 KB boxes of 32 columns per emission warp, i.e. 5 ring stages
     // instead of 4, were measured: no faster, twice the bulk stores.)
-    constexpr uint32_t kStgTotal = kMode != 0 ? kStgBytes : 0u;
+    constexpr uint32_t kStgTotal = kEmitN ? kStgBytes : 0u;
     constexpr int kStages = (kVRingBytes - kStgTotal) / kVStageBytes;                  // 3 / 6  (2 / 4)
     constexpr int kTileRows = kBlockM * kCtaGroup;
 
@@ -634,7 +691,22 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
         while (alive && it.next(t)) {
             const int row0 = t.m * kTileRows + (int)cta_rank * kBlockM + quarter * 32;
             const int r = row0 + lane;                   // GEMM row (packed row number when rows are packed)
-            if (t.m != prev_m) {
+            if constexpr (kMode == kModeRaggedMean) {
+                // the warp's 32 rows are word w of their slot's caption-start mask: the row's caption is the number
+                // of starts up to it, counted from the slot's first caption
+                if (t.m != prev_m) {
+                    const int* meta = p.slot_meta + (size_t)(row0 >> 8) * kSlotMetaInts;
+                    const int w = (row0 >> 5) & 7;
+                    int before = 0;
+                    for (int i = 0; i < w; ++i) before += __popc((uint32_t)__ldg(meta + kSlotMetaStarts + i));
+                    const uint32_t sw = (uint32_t)__ldg(meta + kSlotMetaStarts + w);
+                    const bool valid = (row0 & (kSlotRows - 1)) + lane < __ldg(meta + kSlotMetaUsed);
+                    const int cap = __ldg(meta + kSlotMetaCap0) + before + __popc(sw & (0xffffffffu >> (31 - lane))) - 1;
+                    r_orig = valid ? r : -1;
+                    rs = valid ? 1.0f / (float)__ldg(p.cap_info + 2 * (size_t)cap + 1) : 0.f;
+                    prev_m = t.m;
+                }
+            } else if (t.m != prev_m) {
                 r_orig = (r < M_eff) ? (p.pack_off ? p.rowmap[r] : r) : -1;
                 rs = (r_orig >= 0) ? p.row_scale[r_orig] : 0.f;
                 if constexpr (kFp8) { if (r_orig >= 0) rs = (p.q_scale[r_orig] * rs) * Tval; }     // t_a
@@ -666,6 +738,33 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             tc_fence_after();
             const int Nv = p.Nv - sb * kMaxN;                // patches of this sub-tile that exist (may exceed 256)
             const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * kMaxN;
+
+            if constexpr (kMode == kModeRaggedMax) {
+                // ---- segmented walk of the slot's used columns, two 32-column chunks per step; the mask words
+                //      are read with the same address in every lane (one broadcast load each) ----
+                const int* meta = p.slot_meta + (size_t)t.j * kSlotMetaInts;
+                const int used = __ldg(meta + kSlotMetaUsed);
+                int cap = __ldg(meta + kSlotMetaCap0);
+                float run = -INFINITY;
+#pragma unroll 1
+                for (int c = 0; c < kMaxN / 32 && c * 32 < used; c += 2) {
+                    uint32_t bufA[32], bufB[32];
+                    tmem_ld32_raw(taddr + c * 32, bufA);
+                    tmem_ld32_raw(taddr + (c + 1) * 32, bufB);
+                    const int2 sw = __ldg(reinterpret_cast<const int2*>(meta + kSlotMetaStarts + c));
+                    const int2 ew = __ldg(reinterpret_cast<const int2*>(meta + kSlotMetaEnds + c));
+                    tmem_wait_ld();
+                    ragged_chunk(bufA, (uint32_t)sw.x, (uint32_t)ew.x, run, cap, r_orig >= 0, Tval, rs, p, row0, lane);
+                    ragged_chunk(bufB, (uint32_t)sw.y, (uint32_t)ew.y, run, cap, r_orig >= 0, Tval, rs, p, row0, lane);
+                }
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) {
+                    if constexpr (kCtaGroup == 2) mbar_arrive_cluster(t_empty_sig + 8 * acc);
+                    else mbar_arrive_local(bar_t_empty + 8 * acc);
+                }
+                continue;
+            }
 
             // ---- pass 1: row maximum over the raw accumulators.  32-column loads, software pipelined
             //      (chunk c+1 in flight while chunk c is reduced), four independent FMNMX3 chains per chunk.
@@ -704,6 +803,7 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             float R;
             float theta = 0.f;
             if constexpr (kFp8) R = mx;
+            else if constexpr (kRagged) R = round_sim<true>(mx, Tval);       // no idx: no threshold
             else theta = argmax_threshold<true>(mx, Tval, &R);
 
             // ---- pass 2: first column whose accumulator reaches the threshold (the reference's first-index
@@ -711,7 +811,7 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             //      qualifying column is the one that sticks; inside a chunk four independent 8-column
             //      compare/select chains instead of one 256-long dependent chain. ----
             int best = (int)kNoCol;
-            if (!kFp8 && p.idx != nullptr) {
+            if (!kFp8 && !kRagged && p.idx != nullptr) {
                 constexpr int kHalfCh = kSolo ? kCh : kCh / 2;
                 const int cb = kSolo ? 0 : half * kHalfCh;       // this warp's chunks: [cb, cb + kHalfCh)
                 uint32_t bufA[32], bufB[32];
@@ -735,7 +835,7 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
                 if constexpr (kCtaGroup == 2) mbar_arrive_cluster(t_empty_sig + 8 * acc);
                 else mbar_arrive_local(bar_t_empty + 8 * acc);
             }
-            if (p.idx != nullptr && !kSolo) {
+            if (p.idx != nullptr && !kSolo && !kRagged) {
                 // pair exchange (double buffered by tile parity: the upper-half warp may already be one tile ahead)
                 const uint32_t slot = xch_smem + ((t_cnt & 1u) * 128u + (uint32_t)(quarter * 32 + lane)) * 2u;
                 if (half == 1) asm volatile("st.shared.u16 [%0], %1;" ::"r"(slot), "h"((uint16_t)best) : "memory");
@@ -754,13 +854,15 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             else if (sb == 0 || R > R_run) { R_run = R; best_run = best + sb * kMaxN; }
           }
             if (!alive) break;
-            if (half == 1) continue;
-            if (p.idx != nullptr && r_orig >= 0) {
+            if (half == 1 || kMode == kModeRaggedMax) continue;     // kMode 3 stored its partials during the walk
+            if (!kRagged && p.idx != nullptr && r_orig >= 0) {
                 if (p.idx16) reinterpret_cast<uint16_t*>(p.idx)[(size_t)t.j * idx_pitch + idx_off] = (uint16_t)best_run;
                 else p.idx[(size_t)t.j * idx_pitch + idx_off] = (uint8_t)best_run;
             }
             const float val = (r_orig >= 0) ? R_run * rs : 0.f;
-            if (p.pack_off == nullptr) store_group_partials(p.part, t.j, row0 >> 5, p.G, p.S, row0, p.M, p.Nq, val, lane);
+            if constexpr (kMode == kModeRaggedMean) {
+                if (r_orig >= 0) p.part[r] = val;                  // one weighted row maximum per slot row
+            } else if (p.pack_off == nullptr) store_group_partials(p.part, t.j, row0 >> 5, p.G, p.S, row0, p.M, p.Nq, val, lane);
             else store_group_partials_packed(p.part, t.j, p.Bq, p.pieces, qi, piece, val, lane);
         }
     }
@@ -816,7 +918,7 @@ bool tc_e4m3_supported(int Nv, int D) { return Nv >= 1 && Nv <= 65535 && D % 128
 int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, const float* T,
                       int inv_T, int M, int Bv, int Nq, int Nv, int D,
                       float* part, void* idx, int* abort_flag, int cta_group, int flags, const int* pack_maps,
-                      const EmitNArgs* emit, const E4m3Args* e4m3, cudaStream_t st) {
+                      const EmitNArgs* emit, const E4m3Args* e4m3, cudaStream_t st, const RaggedArgs* ragged) {
     using namespace tc;
     if (e4m3 ? !tc_e4m3_supported(Nv, D) : !tc_supported(Nv, D))
         return fail_msg(TRIAD_ERR_UNSUPPORTED, e4m3 ? "tcgen05 e4m3 forward: needs D in {128, 256, 384, 512}"
@@ -887,6 +989,18 @@ int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, cons
     const long long total = (long long)n_m * Bv;
     if ((long long)n_clusters > total) n_clusters = (int)total;
     if (n_clusters < 1) n_clusters = 1;
+    if (ragged) {
+        p.slot_meta = ragged->slot_meta;
+        p.cap_info = ragged->cap_info;
+        if (ragged->direction == 0) {
+            p.S = 1;                                          // part[caption][group]
+            return cta_group == 2 ? launch_t<2, false, kModeRaggedMax>(mq, mv, mn, p, n_clusters, st)
+                                  : launch_t<1, false, kModeRaggedMax>(mq, mv, mn, p, n_clusters, st);
+        }
+        if (cta_group != 2) return fail_msg(TRIAD_ERR_UNSUPPORTED, "ragged direction 1: cta_group::2 only");
+        return n_sub > 1 ? launch_t<2, true, kModeRaggedMean>(mq, mv, mn, p, n_clusters, st)
+                         : launch_t<2, false, kModeRaggedMean>(mq, mv, mn, p, n_clusters, st);
+    }
     if (emit) {
         // one slot per epilogue warp of every CTA, written only by the emission warps of CTAs that get work: clear all
         TRIAD_CUDA_CHECK(cudaMemsetAsync(emit->partials, 0, (size_t)sms * kEmitEpiWarps * 2 * sizeof(double), st));

@@ -8,6 +8,7 @@ swapped), and the rank of the diagonal is computed on the device.
 """
 from __future__ import annotations
 
+import ctypes
 from collections import defaultdict
 from typing import Dict, List, Sequence
 
@@ -178,15 +179,177 @@ def _scores_fp8(q_feats: torch.Tensor, gallery: Fp8Gallery, temperature, directi
     return out
 
 
+SLOT_ROWS = 256           # rows of one slot of a RaggedGallery, and the longest caption it stores
+_SLOT_META_INTS = 20      # triad_ragged_plan: first caption, count, used rows, 0, start mask [8], end mask [8]
+
+
+def ragged_plan(lengths) -> tuple:
+    """(slot_meta int32 [n_slots, 20], cap_info int32 [n_cap, 2]) of captions with these lengths, on the host
+    (triad_ragged_plan): greedy in order, a caption that does not fit in the rest of the current 256-row slot starts
+    a new one.  cap_info[c] = (first row = slot * 256 + offset, length).  Lengths must be 1..256."""
+    lens = np.ascontiguousarray(np.asarray(lengths, dtype=np.int64).reshape(-1))
+    if lens.size == 0:
+        raise ValueError("RaggedGallery: need at least one caption")
+    if lens.min() < 1 or lens.max() > SLOT_ROWS:
+        raise ValueError(f"RaggedGallery: caption lengths must be 1..{SLOT_ROWS}, got {int(lens.min())}..{int(lens.max())}")
+    lens = lens.astype(np.int32)
+    n = lens.size
+    meta = np.zeros((n, _SLOT_META_INTS), dtype=np.int32)
+    info = np.zeros((n, 2), dtype=np.int32)
+    n_slots = ctypes.c_int(0)
+    check(_lib.load().triad_ragged_plan(lens.ctypes.data, n, meta.ctypes.data, info.ctypes.data, ctypes.byref(n_slots)),
+          "triad_ragged_plan")
+    return meta[:n_slots.value].copy(), info
+
+
+class RaggedGallery:
+    """A gallery of items with different token counts (captions truncated to their valid tokens), stored without
+    padding: the token rows of whole captions in 256-row slots, ``slots`` bf16 [n_slots * 256, D].
+
+    Captions are placed greedily in order; one that does not fit in the rest of the current slot starts a new slot,
+    so no caption straddles a slot, and a slot's rows after its last caption are zero.  ``meta`` (int32
+    [n_slots, 20]) and ``cap_info`` (int32 [n_cap, 2]) describe the layout (``ragged_plan``).  fp32 features are
+    rounded to bf16 when the gallery is built.  Caption lengths must be 1..256.
+
+    ``retrieve_topk`` and ``dist.sharded_retrieve_topk`` accept it in place of a dense tensor, in both directions;
+    ids are caption numbers.  ``len()`` and ``shape[0]`` are the caption count; ``shape`` is (n_cap, D)."""
+
+    def __init__(self, slots: torch.Tensor, meta: torch.Tensor, cap_info: torch.Tensor, lengths: np.ndarray):
+        self.slots = slots
+        self.meta = meta
+        self.cap_info = cap_info
+        self.lengths = lengths
+
+    @classmethod
+    def _build(cls, src: torch.Tensor, src_rows: np.ndarray, lengths: np.ndarray) -> "RaggedGallery":
+        """Caption c is rows src_rows[sum(lengths[:c]) : ...] of src ([rows, D] fp32 or bf16, on the device)."""
+        meta, info = ragged_plan(lengths)
+        D = src.shape[1]
+        n_slots = meta.shape[0]
+        dev = src.device
+        rowmap = np.full(n_slots * SLOT_ROWS, -1, dtype=np.int32)
+        firsts = np.repeat(info[:, 0].astype(np.int64), lengths)
+        within = np.arange(int(lengths.sum()), dtype=np.int64) - np.repeat(np.cumsum(lengths) - lengths, lengths)
+        rowmap[firsts + within] = src_rows
+        slots = torch.empty(n_slots * SLOT_ROWS, D, dtype=torch.bfloat16, device=dev)
+        src = src.contiguous()
+        if src.dtype not in (torch.float32, torch.bfloat16):
+            src = src.float()
+        rm = torch.from_numpy(rowmap).to(dev)
+        with ops._on(src):
+            check(_lib.load().triad_ragged_pack(src.data_ptr(), ops._dtype_code(src), src.shape[0], D, rm.data_ptr(),
+                                                slots.shape[0], slots.data_ptr(), ops._stream(dev)), "triad_ragged_pack")
+        return cls(slots, torch.from_numpy(meta).to(dev), torch.from_numpy(info).to(dev), lengths.astype(np.int32))
+
+    @classmethod
+    def from_padded(cls, feats: torch.Tensor, attention_mask) -> "RaggedGallery":
+        """Captions from the text embedder's output: feats [b, L, D] and attention_mask [b, L]; caption i keeps the
+        rows whose mask is non-zero, in order (the reference's truncation for right-padded masks)."""
+        if feats.dim() != 3:
+            raise ValueError(f"RaggedGallery.from_padded: feats must be [b, L, D], got {tuple(feats.shape)}")
+        b, L, D = feats.shape
+        mask = (torch.as_tensor(attention_mask).detach().to("cpu").numpy() != 0)
+        if mask.shape != (b, L):
+            raise ValueError(f"RaggedGallery.from_padded: attention_mask must be [{b}, {L}], got {mask.shape}")
+        lengths = mask.sum(axis=1)
+        src_rows = np.flatnonzero(mask.reshape(-1)).astype(np.int32)
+        return cls._build(feats.reshape(b * L, D), src_rows, lengths)
+
+    @classmethod
+    def from_list(cls, feats: Sequence[torch.Tensor]) -> "RaggedGallery":
+        """Captions from a list of [L_i, D] tensors (what the reference's embed_tv_subset returns)."""
+        if len(feats) == 0:
+            raise ValueError("RaggedGallery.from_list: need at least one caption")
+        if any(t.dim() != 2 for t in feats) or len({t.shape[1] for t in feats}) != 1:
+            raise ValueError("RaggedGallery.from_list: captions must be [L_i, D] with one D")
+        lengths = np.array([t.shape[0] for t in feats], dtype=np.int64)
+        src = torch.cat([t.to(feats[0].dtype) for t in feats])
+        return cls._build(src, np.arange(src.shape[0], dtype=np.int32), lengths)
+
+    @classmethod
+    def cat(cls, galleries: Sequence["RaggedGallery"]) -> "RaggedGallery":
+        """The captions of several galleries, in order (caption ids continue from one gallery to the next).  Slots
+        are independent, so this concatenates slot arrays: a large gallery can be built batch by batch."""
+        if len(galleries) == 0:
+            raise ValueError("RaggedGallery.cat: need at least one gallery")
+        D, dev = galleries[0].shape[1], galleries[0].device
+        if any(g.shape[1] != D or g.device != dev for g in galleries):
+            raise ValueError("RaggedGallery.cat: galleries must share D and device")
+        metas, infos = [], []
+        cap_off = slot_off = 0
+        for g in galleries:
+            m = g.meta.clone()
+            m[:, 0] += cap_off
+            i = g.cap_info.clone()
+            i[:, 0] += slot_off * SLOT_ROWS
+            metas.append(m)
+            infos.append(i)
+            cap_off += len(g)
+            slot_off += g.n_slots
+        return cls(torch.cat([g.slots for g in galleries]), torch.cat(metas), torch.cat(infos),
+                   np.concatenate([g.lengths for g in galleries]))
+
+    @property
+    def n_slots(self) -> int:
+        return self.meta.shape[0]
+
+    @property
+    def shape(self):
+        return (self.cap_info.shape[0], self.slots.shape[1])
+
+    @property
+    def device(self) -> torch.device:
+        return self.slots.device
+
+    @property
+    def nbytes(self) -> int:
+        return self.slots.numel() * 2 + self.meta.numel() * 4 + self.cap_info.numel() * 4
+
+    def __len__(self) -> int:
+        return self.cap_info.shape[0]
+
+
+def _scores_ragged(q_feats: torch.Tensor, gallery: RaggedGallery, temperature, direction: int) -> torch.Tensor:
+    """scores[c] of one query (Nq, D) against every caption of a ragged gallery (triad_retrieve_scores_ragged); the
+    query is rounded to bf16 like the gallery."""
+    n_cap, D = gallery.shape
+    if q_feats.dim() != 2 or q_feats.shape[1] != D:
+        raise ValueError(f"query must be [Nq, {D}], got {tuple(q_feats.shape)}")
+    if direction not in (0, 1):
+        raise ValueError(f"direction must be 0 or 1, got {direction}")
+    lib = _lib.load()
+    dev = gallery.device
+    q = q_feats.to(device=dev, dtype=torch.bfloat16).contiguous()
+    Nq = q.shape[0]
+    T = ops.temperature_tensor(temperature, dev)
+    out = torch.empty(n_cap, dtype=torch.float32, device=dev)
+    nws = lib.triad_retrieve_ragged_workspace_bytes(Nq, gallery.n_slots, n_cap, direction)
+    with ops._on(out):
+        ws = ops._Workspace.get(nws, dev, "retrieve_ragged")
+        check(lib.triad_retrieve_scores_ragged(q.data_ptr(), Nq, gallery.slots.data_ptr(), gallery.meta.data_ptr(),
+                                               gallery.cap_info.data_ptr(), gallery.n_slots, n_cap, D, T.data_ptr(),
+                                               direction, out.data_ptr(), ws.data_ptr(), ws.numel(), ops._stream(dev)),
+              "triad_retrieve_scores_ragged")
+    return out
+
+
 def retrieve_topk(q_feats: torch.Tensor, gallery, temperature, k: int, direction: int = 0):
     """Top-k gallery items for one query (BASELINE cfg 5): (scores fp32 [k], ids int32 [k]).
 
-    ``gallery`` is an embedding tensor [n_img, Nv, D] or an ``Fp8Gallery`` (e4m3 codes with per-patch scales; the
-    query is then quantized per token in the same call, and only direction 0 is supported)."""
+    ``gallery`` is an embedding tensor [n_img, Nv, D], an ``Fp8Gallery`` (e4m3 codes with per-patch scales; the
+    query is then quantized per token in the same call, and only direction 0 is supported) or a ``RaggedGallery``
+    (captions of different lengths, both directions; the query is rounded to bf16)."""
     if isinstance(gallery, Fp8Gallery):
         s = _scores_fp8(q_feats, gallery, temperature, direction)
+    elif isinstance(gallery, RaggedGallery):
+        s = _scores_ragged(q_feats, gallery, temperature, direction)
     else:
         s = _scores(q_feats, gallery, temperature, direction)
+    return _topk(s, k)
+
+
+def _topk(s: torch.Tensor, k: int):
+    """(scores, ids) of the k largest entries of s, ties to the lower id (triad_topk)."""
     lib = _lib.load()
     n = s.numel()
     out_s = torch.empty(k, dtype=torch.float32, device=s.device)
