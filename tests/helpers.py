@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests (test infrastructure)."""
+import math
 import os
 
 import numpy as np
@@ -29,6 +30,52 @@ def _as64(x):
 def rel_err(a, b):
     a, b = _as64(a), _as64(b)
     return ((a - b).norm() / b.norm().clamp(min=1e-30)).item()
+
+
+def model_sims(raw, T, dtype):
+    """The similarities S of the rounding model, from the exact dot products raw = <q, v> (fp64), returned in fp64.
+    bf16 inputs: S = bf16(bf16(<q, v>) * T), as the reference computes them under autocast (the matmul rounds its fp32
+    accumulator to bf16, the product with the fp32 temperature is rounded again; oracle.maxmean_forward).  fp32 inputs:
+    S = T * <q, v>, unrounded."""
+    if dtype == torch.bfloat16:
+        T32 = torch.tensor(float(T), dtype=torch.float32, device=raw.device)
+        return (raw.float().bfloat16().float() * T32).bfloat16().double()
+    return raw * float(T)
+
+
+def bf16_ulp(x):
+    """One bf16 ulp of each element of x (fp64): 2^(floor(log2 |x|) - 7)."""
+    return torch.exp2(torch.floor(torch.log2(x.abs().clamp(min=1e-30))) - 7)
+
+
+def ambiguous_bf16_rounding(raw, sq, D, width=4.0):
+    """True where an fp32 accumulator of the D-term dot product raw = <q, v> (fp64, exact) may round to bf16 either
+    way: raw lies within `width` sigma of a bf16 rounding midpoint, sigma being the accumulator's random-walk rounding
+    error 2^-24 * sqrt(D * <q^2, v^2>) (sq = <q^2, v^2>)."""
+    acc_err = width * 2.0 ** -24 * math.sqrt(D) * sq.sqrt()
+    a, r = raw.abs(), raw.float().bfloat16().double().abs()
+    # the two midpoints around r; below a power of two the grid is twice as fine
+    up, down = r + bf16_ulp(r) / 2, r - bf16_ulp(r * (1 - 2.0 ** -9)) / 2
+    return torch.minimum((a - up).abs(), (a - down).abs()) < acc_err
+
+
+def certify_near_ties(q, v, got, ref):
+    """Argmax disagreements between two evaluations of the bf16 similarities, got and ref ((Bq, Bv, Nq) winner
+    indices of q (Bq, Nq, D) against v (Bv, Nv, D)).  A disagreement is a genuine tie of the doubly rounded
+    S = bf16(bf16(acc) * T) that the fp32 accumulation order can flip only when the two candidates' EXACT dot products
+    (fp64) are less than 2 bf16 ulps of the accumulator apart.  (Two accumulators that round to the same or to ADJACENT
+    bf16 values can land in the same output bin after the multiply by T moves them into the next binade, where the
+    output grid is twice as coarse; anything further apart cannot tie.)  Returns (count, worst gap in ulps): the
+    caller bounds both."""
+    bad = (got != ref).nonzero()
+    if bad.shape[0] == 0:
+        return 0, 0.0
+    i, j, a = bad.unbind(1)
+    qa = q[i, a].double()
+    x = (qa * v[j, got[i, j, a]].double()).sum(-1)
+    y = (qa * v[j, ref[i, j, a]].double()).sum(-1)
+    ulp = torch.exp2(torch.floor(torch.log2(torch.maximum(x.abs(), y.abs()).clamp(min=1e-300))) - 7)
+    return int(bad.shape[0]), ((x - y).abs() / ulp).max().item()
 
 
 def round_bf16_st(t):

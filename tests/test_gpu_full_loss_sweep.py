@@ -48,6 +48,7 @@ import pytest
 import torch
 
 from oracle import oracle as O
+from tests import helpers as H
 
 pytestmark = pytest.mark.gpu
 
@@ -173,8 +174,7 @@ def _rounded_sims(q, v, T):
     raw = torch.einsum("iad,jpd->ijap", q64, v64)
     S = raw * T64
     if q.dtype == torch.bfloat16:
-        T32 = torch.tensor(float(T), dtype=torch.float32, device="cuda")
-        Sr = (raw.detach().float().bfloat16().float() * T32).bfloat16().double()
+        Sr = H.model_sims(raw.detach(), T, q.dtype)
         S = S + (Sr - S).detach()
     return raw, S, T64, q64, v64
 
@@ -184,27 +184,20 @@ def _rounding_slack_weights(q, v, raw):
     if q.dtype != torch.bfloat16:
         return None
     with torch.no_grad():
-        # rounding errors of an fp32 sum of D products add like a random walk: 4 sigma of it
-        acc_err = 4 * 2.0 ** -24 * math.sqrt(q.shape[-1]) * torch.einsum("iad,jpd->ijap", q.double() ** 2, v.double() ** 2).sqrt()
-        r = raw.float().bfloat16().double()
-        ulp = torch.exp2(torch.floor(torch.log2(r.abs().clamp(min=1e-30))) - 7)
-        ambiguous = (ulp / 2 - (raw - r).abs()).abs() < acc_err
+        sq = torch.einsum("iad,jpd->ijap", q.double() ** 2, v.double() ** 2)
+        ulp = H.bf16_ulp(raw.float().bfloat16().double())
+        ambiguous = H.ambiguous_bf16_rounding(raw, sq, q.shape[-1])
         return torch.where(ambiguous, 2 * ulp, torch.zeros_like(ulp))
 
 
-def _certified_winners(c, raw, S, got, scale):
+def _certified_winners(c, q, v, S, got, scale):
     """The GPU's winners where they are certified near-ties of the reference's own argmax; the reference's argmax on
     zero-weight rows (nothing depends on them; a packed forward leaves them unwritten)."""
     ref = S.detach().argmax(dim=3)
     live = (scale > 0)[:, None, :].expand_as(ref)
     got = torch.where(live, got.clamp(0, c.Nv - 1), ref)
-    bad = (got != ref).nonzero().tolist()
-    worst = 0.0
-    for i, j, a in bad:
-        x, y = raw[i, j, a, got[i, j, a]].item(), raw[i, j, a, ref[i, j, a]].item()
-        ulp = 2.0 ** (math.floor(math.log2(max(abs(x), abs(y), 1e-300))) - 7)
-        worst = max(worst, abs(x - y) / ulp)
-    assert len(bad) <= max(2, 1e-4 * ref.numel()), len(bad)
+    n_bad, worst = H.certify_near_ties(q, v, got, ref)
+    assert n_bad <= max(2, 1e-4 * ref.numel()), n_bad
     assert worst < 2.0, worst
     return got
 
@@ -498,7 +491,7 @@ def test_full_loss_against_fp64(case, entry, monkeypatch):
     else:
         route, vals, grads, got_idx = _run_sharded(c, entry[len("sharded_"):], q, v, mask, thr, w)
     raw, S, _, _, _ = _rounded_sims(q, v, c.T)
-    winners = _certified_winners(c, raw.detach(), S.detach(), got_idx, _row_scale64(c, mask))
+    winners = _certified_winners(c, q, v, S.detach(), got_idx, _row_scale64(c, mask))
     del raw, S
     ref, rgrads = _reference(c, q, v, mask, thr, w, winners)
     _anti_vacuity(c, ref)
@@ -540,7 +533,7 @@ def test_single_token_av():
     for variant in ("one", "several"):
         route, vals, grads, got_idx = _run_sharded(c, variant, q, v, None, 0.3, 0.1)
         assert vals["pos"] == 0.0
-        winners = _certified_winners(c, raw.detach(), S.detach(), got_idx, _row_scale64(c, None))
+        winners = _certified_winners(c, q, v, S.detach(), got_idx, _row_scale64(c, None))
         ref, rgrads = _reference(c, q, v, None, 0.3, 0.1, winners, drop_single_row_smooth=True)
         rgrads = {"total": rgrads["total"]}
         _compare(c, vals, grads, ref, rgrads)

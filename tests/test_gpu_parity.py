@@ -13,7 +13,7 @@ import torch
 
 from oracle import oracle as O
 from oracle.cases import CASES, build_inputs, projection
-from tests.helpers import check_inputs_reproduce, load_golden, rel_err
+from tests.helpers import certify_near_ties, check_inputs_reproduce, load_golden, rel_err
 
 pytestmark = pytest.mark.gpu
 
@@ -636,22 +636,6 @@ def _report(name, payload):
             f.write(line + "\n")
 
 
-def _certify_near_ties(qd, vd, T, got, ref):
-    """Every argmax disagreement must be a genuine tie of the reference's doubly rounded similarities
-    S = bf16(bf16(acc) * T) that fp32 accumulation order can flip: the two candidates' EXACT dot products (fp64 on the
-    GPU) are less than 2 bf16 ulps of the accumulator apart.  (Two accumulators that round to the same or to ADJACENT
-    bf16 values can land in the same output bin after the multiply by T moves them into the next binade, where the
-    output grid is twice as coarse; anything further apart cannot tie.)  Returns (count, worst gap in ulps)."""
-    bad = (got != ref).nonzero()
-    worst = 0.0
-    for i, j, a in bad.tolist():
-        s = qd[i, a].double() @ vd[j].double().t()                         # raw <q,v>: what the tensor core accumulates
-        x, y = s[got[i, j, a]].item(), s[ref[i, j, a]].item()
-        ulp = 2.0 ** (math.floor(math.log2(max(abs(x), abs(y), 1e-300))) - 7)
-        worst = max(worst, abs(x - y) / ulp)
-    return int(bad.shape[0]), worst
-
-
 def test_argmax_flip_count_vs_reference_cuda_path():
     """The deployment path of the reference is torch-CUDA eager (cuBLAS bf16 matmul, src/model.py:384-391 under
     train.py:76).  B=32 x 250 x 256 x 512 bf16: winners of the fused kernel vs (a) the reference's OWN methods run on
@@ -681,9 +665,9 @@ def test_argmax_flip_count_vs_reference_cuda_path():
             src = "restatement of model.py:384-391 on CUDA (oracle/_ref not staged)"
         assert tok_ref.dtype == torch.bfloat16 and clip_ref.dtype == torch.bfloat16
         idx_cuda = tok_ref.max(dim=3).indices
-    n_cuda, worst_cuda = _certify_near_ties(qd, vd, T, got, idx_cuda)
+    n_cuda, worst_cuda = certify_near_ties(qd, vd, got, idx_cuda)
     cpu = O.maxmean_forward(q, v, T)
-    n_cpu, worst_cpu = _certify_near_ties(qd, vd, T, got, cpu["idx"].cuda())
+    n_cpu, worst_cpu = certify_near_ties(qd, vd, got, cpu["idx"].cuda())
     n_ref_vs_cpu = int((idx_cuda.cpu() != cpu["idx"]).sum())           # the two reference paths disagree with each other too
     numel = got.numel()
     _report("argmax_flip_count", {"rows": numel, "vs": src, "mismatch_vs_reference_cuda": n_cuda,
@@ -711,7 +695,7 @@ def test_full_size_cfg3_masked():
     sl = [0, 1, 77, 255, 300, 511]
     ref = O.maxmean_forward(q[sl], v, T, mask[sl])
     got = tok.argmax()[sl]
-    n_bad, worst = _certify_near_ties(qd.detach()[sl], vd.detach(), T, got, ref["idx"].cuda())
+    n_bad, worst = certify_near_ties(qd.detach()[sl], vd.detach(), got, ref["idx"].cuda())
     _report("cfg3_full_size", {"rows": got.numel(), "mismatch_vs_cpu_oracle": n_bad, "worst_gap_bf16_ulps": worst})
     assert n_bad <= max(2, 1e-4 * got.numel()) and worst < 2.0
     assert rel_err(tok.clip.detach()[sl].cpu(), ref["clip"]) < 5e-5
@@ -748,14 +732,14 @@ def test_cfg4_rank_shape_slice():
     qi = 517
     ref = O.maxmean_forward(qd[qi:qi + 1].cpu(), vd.cpu(), T)
     got = idx_v[:, qi].to(torch.int64)[None]                                             # (1,Bv,Nq)
-    n1, w1 = _certify_near_ties(qd[qi:qi + 1], vd, T, got, ref["idx"].cuda())
+    n1, w1 = certify_near_ties(qd[qi:qi + 1], vd, got, ref["idx"].cuda())
     assert rel_err(clip[qi:qi + 1].cpu(), ref["clip"]) < 5e-5
     # (b) eight queries x 64 spread images
     qs = [0, 1, 255, 256, 600, 777, 1000, 1023]
     js = list(range(5, Bv, 128))
     ref2 = O.maxmean_forward(qd[qs].cpu(), vd[js].cpu(), T)
     got2 = idx_v[js][:, qs].permute(1, 0, 2).to(torch.int64)
-    n2, w2 = _certify_near_ties(qd[qs], vd[js], T, got2, ref2["idx"].cuda())
+    n2, w2 = certify_near_ties(qd[qs], vd[js], got2, ref2["idx"].cuda())
     _report("cfg4_rank_shape", {"rows": got.numel() + got2.numel(), "mismatch_vs_cpu_oracle": n1 + n2,
                                 "worst_gap_bf16_ulps": max(w1, w2)})
     assert n1 + n2 <= max(2, 1e-4 * (got.numel() + got2.numel())) and max(w1, w2) < 2.0

@@ -34,6 +34,16 @@ static inline NceWs nce_ws_carve(void* ws, int rows, int B) {
     return w;
 }
 
+// The hardest negative (the max of the off-diagonal entries) propagates NaN like the reference's torch max: fmaxf /
+// fmax return the other operand, which would report a finite hardest negative next to a NaN loss.
+__device__ __forceinline__ float nan_max(float a, float b) { return (a != a || b != b) ? a + b : fmaxf(a, b); }
+__device__ __forceinline__ double nan_max(double a, double b) { return (a != a || b != b) ? a + b : fmax(a, b); }
+__device__ __forceinline__ float warp_nan_max(float v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = nan_max(v, __shfl_xor_sync(0xffffffffu, v, o));
+    return v;
+}
+
 // ---- step 1a: one CTA = 32 rows; warps reduce rows, then threads own columns ---------------
 __global__ void __launch_bounds__(kNceThreads)
 nce_partial_kernel(const float* __restrict__ clip, int rows, int B, int rpb,
@@ -108,7 +118,7 @@ nce_finish_kernel(const float* __restrict__ clip, int rows, int B, int row0,
                 loss += (double)(rl - xc) + (double)(cl - xc);
                 sd += xc; sd2 += (double)xc * xc;
             } else {
-                so += xc; so2 += (double)xc * xc; mo = fmaxf(mo, xc);
+                so += xc; so2 += (double)xc * xc; mo = nan_max(mo, xc);
             }
             gv *= inv2B;
             gc += (double)gv * xc;
@@ -118,7 +128,7 @@ nce_finish_kernel(const float* __restrict__ clip, int rows, int B, int row0,
     __shared__ double red[kNceThreads / 32][7];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     loss = warp_sum_d(loss); sd = warp_sum_d(sd); sd2 = warp_sum_d(sd2);
-    so = warp_sum_d(so); so2 = warp_sum_d(so2); gc = warp_sum_d(gc); mo = warp_max(mo);
+    so = warp_sum_d(so); so2 = warp_sum_d(so2); gc = warp_sum_d(gc); mo = warp_nan_max(mo);
     if (lane == 0) {
         red[warp][0] = loss; red[warp][1] = sd; red[warp][2] = sd2; red[warp][3] = so;
         red[warp][4] = so2; red[warp][5] = (double)mo; red[warp][6] = gc;
@@ -127,7 +137,7 @@ nce_finish_kernel(const float* __restrict__ clip, int rows, int B, int row0,
     if (threadIdx.x < 7) {
         const int k = threadIdx.x;
         double a = red[0][k];
-        for (int w = 1; w < kNceThreads / 32; ++w) a = (k == 5) ? fmax(a, red[w][k]) : a + red[w][k];
+        for (int w = 1; w < kNceThreads / 32; ++w) a = (k == 5) ? nan_max(a, red[w][k]) : a + red[w][k];
         blk_sums[(size_t)blk * 8 + k] = a;
     }
 }
@@ -138,7 +148,7 @@ __global__ void nce_final_reduce_kernel(const double* __restrict__ blk_sums, int
     if (k >= 8) return;
     if (k == 7) { sums[7] = 0.0; return; }
     double a = blk_sums[k];
-    for (int b = 1; b < nblk; ++b) a = (k == 5) ? fmax(a, blk_sums[(size_t)b * 8 + k]) : a + blk_sums[(size_t)b * 8 + k];
+    for (int b = 1; b < nblk; ++b) a = (k == 5) ? nan_max(a, blk_sums[(size_t)b * 8 + k]) : a + blk_sums[(size_t)b * 8 + k];
     sums[k] = a;
 }
 
@@ -193,7 +203,7 @@ nce_head_kernel(const float* __restrict__ clip, int B, int rpb, const float* __r
                 loss += (double)(rl - xc) + (double)(cl - xc);
                 sd += xc; sd2 += (double)xc * xc;
             } else {
-                so += xc; so2 += (double)xc * xc; mo = fmaxf(mo, xc);
+                so += xc; so2 += (double)xc * xc; mo = nan_max(mo, xc);
             }
             gv *= inv2B;
             gc += (double)gv * xc;
@@ -204,7 +214,7 @@ nce_head_kernel(const float* __restrict__ clip, int B, int rpb, const float* __r
     __shared__ bool is_last;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     loss = warp_sum_d(loss); sd = warp_sum_d(sd); sd2 = warp_sum_d(sd2);
-    so = warp_sum_d(so); so2 = warp_sum_d(so2); gc = warp_sum_d(gc); mo = warp_max(mo);
+    so = warp_sum_d(so); so2 = warp_sum_d(so2); gc = warp_sum_d(gc); mo = warp_nan_max(mo);
     if (lane == 0) {
         red[warp][0] = loss; red[warp][1] = sd; red[warp][2] = sd2; red[warp][3] = so;
         red[warp][4] = so2; red[warp][5] = (double)mo; red[warp][6] = gc;
@@ -213,7 +223,7 @@ nce_head_kernel(const float* __restrict__ clip, int B, int rpb, const float* __r
     if (threadIdx.x < 7) {
         const int k = threadIdx.x;
         double a = red[0][k];
-        for (int w = 1; w < kNceThreads / 32; ++w) a = (k == 5) ? fmax(a, red[w][k]) : a + red[w][k];
+        for (int w = 1; w < kNceThreads / 32; ++w) a = (k == 5) ? nan_max(a, red[w][k]) : a + red[w][k];
         blk_sums[(size_t)blk * 8 + k] = a;
     }
     __syncthreads();
@@ -231,7 +241,7 @@ nce_head_kernel(const float* __restrict__ clip, int B, int rpb, const float* __r
             a = ((volatile double*)blk_sums)[k];
             for (int b = 1; b < (int)gridDim.x; ++b) {
                 const double t = ((volatile double*)blk_sums)[(size_t)b * 8 + k];
-                a = (k == 5) ? fmax(a, t) : a + t;
+                a = (k == 5) ? nan_max(a, t) : a + t;
             }
         }
         sums[k] = a;

@@ -134,7 +134,8 @@ class LazyStats(Mapping):
 
 def _stats_from_sums(sums: torch.Tensor, B: int, prefix: str) -> Dict[str, float]:
     """model.py:435-450 / :553-568 from the kernel's fp64 sums; ONE device->host copy instead of
-    the reference's five .item() calls."""
+    the reference's five .item() calls.  B = 1 has no off-diagonal entry: the negative statistics, the separation and
+    the hardest negative are NaN (where the reference's max over an empty tensor raises)."""
     s = sums.tolist()
     n_off = B * B - B
     pos_mean = s[1] / B
@@ -147,7 +148,7 @@ def _stats_from_sums(sums: torch.Tensor, B: int, prefix: str) -> Dict[str, float
         f"{prefix}_neg_sim_mean": neg_mean,
         f"{prefix}_neg_sim_std": max(neg_var, 0.0) ** 0.5 if neg_var == neg_var else neg_var,
         f"{prefix}_separation": pos_mean - neg_mean,
-        f"{prefix}_hardest_negative": s[5],
+        f"{prefix}_hardest_negative": s[5] if n_off else float("nan"),
     }
 
 
