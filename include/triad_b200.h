@@ -282,6 +282,29 @@ size_t triad_retrieve_ragged_workspace_bytes(int Nq, int n_slots, int n_cap, int
 int triad_retrieve_scores_ragged(const void* q, int Nq, const void* slots, const int32_t* slot_meta,
                                  const int32_t* cap_info, int n_slots, int n_cap, int D, const float* temperature,
                                  int direction, float* scores, void* ws, size_t ws_bytes, void* stream);
+/* ---- the ragged caption gallery stored as e4m3 codes with one fp32 scale per slot row --------------------------
+ * triad_ragged_pack_e4m3: codes[r], scales[r] = triad_quantize_e4m3 of src[rowmap[r]] for r < dst_rows (a multiple
+ * of 256), bit for bit; a zero row (scale 0, codes 0) where rowmap[r] < 0 or rowmap[r] >= src_rows.  fp32 input is
+ * quantized as it is (not rounded to bf16 first).  src [src_rows][D] fp32 or bf16 (dtype), D in {128, 256, 384, 512}
+ * (TRIAD_ERR_UNSUPPORTED otherwise); src and codes 16-byte, rowmap and scales 4-byte aligned. */
+int triad_ragged_pack_e4m3(const void* src, int dtype, long long src_rows, int D, const int32_t* rowmap,
+                           long long dst_rows, void* codes, float* scales, void* stream);
+/* scores[c] for one query, quantized per token by triad_quantize_e4m3 (q_codes [Nq][D], q_scales [Nq]), against the
+ * captions of an e4m3 ragged gallery (codes [n_slots * 256][D], scales [n_slots * 256] from triad_ragged_pack_e4m3;
+ * slot_meta and cap_info as for triad_retrieve_scores_ragged).  acc = the tensor-core dot product of the codes (fp32
+ * accumulation), s_t the scale of slot row t, sq_a the scale of query token a:
+ *   direction 0: sum_a fp32(m_ac * t_a), m_ac = max_{t in c} fp32(s_t * acc_at),
+ *                t_a = fp32(fp32(sq_a * (1/Nq)) * (1/T)), the sum in the dense forward's 32-row-group order;
+ *   direction 1: sum_{t in c, token order} fp32(m_t * w_t), m_t = max_a fp32(sq_a * acc_ta),
+ *                w_t = fp32(fp32(s_t * (1/length_c)) * (1/T)).
+ * The maxima propagate NaN: a caption row holding an inf or a NaN makes that caption's score NaN, a non-finite
+ * query token every score.  D in {128, 256, 384, 512}; the workspace is triad_retrieve_ragged_workspace_bytes;
+ * q_codes, codes and ws 16-byte, metadata 8-byte, scales and scores 4-byte aligned.  Deterministic, position
+ * independent, no host synchronisation; a watchdog timeout gives NaN scores. */
+int triad_retrieve_scores_ragged_e4m3(const void* q_codes, const float* q_scales, int Nq, const void* codes,
+                                      const float* scales, const int32_t* slot_meta, const int32_t* cap_info,
+                                      int n_slots, int n_cap, int D, const float* temperature, int direction,
+                                      float* scores, void* ws, size_t ws_bytes, void* stream);
 /* top-k of scores (descending, ties -> lower id first, like a stable argsort of -scores;
  * -0.0 and +0.0 are equal scores): out_scores fp32 [k] = scores[out_ids], bit for bit,
  * out_ids int32 [k].  NaN scores have no defined place.  ws: triad_topk_workspace_bytes(n). */

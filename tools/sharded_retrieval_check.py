@@ -3,7 +3,7 @@
 single-GPU top-k over the whole gallery — ids bit-equal on every rank, uneven shards, ties across shards.
 With --fp8 the gallery is an e4m3 Fp8Gallery and each rank scores its slice of it.  With --ragged it is a
 RaggedGallery of captions with cfg 3's lengths; each rank builds its shard from its own caption range, and both
-directions are checked."""
+directions are checked (with --fp8 too, an e4m3 RaggedGallery)."""
 import os
 import sys
 
@@ -24,7 +24,7 @@ def main():
     fp8 = "--fp8" in sys.argv[1:]
     ok = True
     if "--ragged" in sys.argv[1:]:
-        ok = check_ragged(world, rank, dev)
+        ok = check_ragged(world, rank, dev, fp8)
     for n_img, Nv, Nq, k in (() if "--ragged" in sys.argv[1:] else ((1001, 256, 77, 10), (515, 1024, 250, 20), (3, 64, 5, 8))):
         g = torch.Generator(device=dev).manual_seed(17)                 # same gallery on every rank
         q = torch.nn.functional.normalize(torch.randn(Nq, 512, generator=g, device=dev), dim=1).bfloat16()
@@ -53,7 +53,7 @@ def main():
     sys.exit(0 if flag.item() == 1 else 1)
 
 
-def check_ragged(world, rank, dev):
+def check_ragged(world, rank, dev, fp8=False):
     import numpy as np
     from triad_b200 import retrieval as R
     from triad_b200.dist import sharded_retrieve_topk
@@ -68,14 +68,14 @@ def check_ragged(world, rank, dev):
         base, rem = n_cap // world, n_cap % world
         n_loc = base + (1 if rank < rem else 0)
         id0 = rank * base + min(rank, rem)
-        shard = R.RaggedGallery.from_list(caps[id0:id0 + n_loc])
-        whole = R.RaggedGallery.from_list(caps)
+        shard = R.RaggedGallery.from_list(caps[id0:id0 + n_loc], fp8=fp8)
+        whole = R.RaggedGallery.from_list(caps, fp8=fp8)
         for d in (0, 1):
             s, ids = sharded_retrieve_topk(q, shard, 1.5, k, id0, direction=d)
             kk = min(k, n_cap)
             s0, i0 = R.retrieve_topk(q, whole, 1.5, kk, d)
             good = torch.equal(ids[:kk], i0.to(torch.int64)) and torch.equal(s[:kk], s0)
-            print(f"rank {rank}: ragged n_cap={n_cap} Nq={Nq} k={k} direction {d}: ids equal {good}", flush=True)
+            print(f"rank {rank}: {'fp8 ' if fp8 else ''}ragged n_cap={n_cap} Nq={Nq} k={k} direction {d}: ids equal {good}", flush=True)
             ok &= good
     return ok
 

@@ -79,6 +79,11 @@ SIGNATURES = {
     "triad_retrieve_ragged_workspace_bytes": (c_size_t, [c_int] * 4),
     "triad_retrieve_scores_ragged": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                              c_void_p, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "triad_ragged_pack_e4m3": (c_int, [c_void_p, c_int, ctypes.c_longlong, c_int, c_void_p, ctypes.c_longlong, c_void_p,
+                                       c_void_p, c_void_p]),
+    "triad_retrieve_scores_ragged_e4m3": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
+                                                  c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_size_t,
+                                                  c_void_p]),
     "triad_topk_workspace_bytes": (c_size_t, [c_int, c_int]),
     "triad_topk": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "triad_diag_ranks": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),

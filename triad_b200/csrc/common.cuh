@@ -163,8 +163,11 @@ int launch_finalize_clip_packed(const float* part, const int* pack_off, int Bq, 
 // - (group of the query's first packed row); a query of <= Nq kept rows spans at most (Nq+30)/32 + 1 groups
 static inline int packed_pieces(int Nq) { return (Nq + 30) / 32 + 1; }
 bool tc_supported(int Nv, int D);
-// rows x D (fp32 or bf16) -> e4m3 codes [rows][D] + one fp32 scale per row (quant_e4m3.cu); D % 16 == 0, D <= 512
-int launch_quantize_e4m3(const void* x, int dtype, long long rows, int D, void* codes, float* scales, cudaStream_t st);
+// rows x D (fp32 or bf16) -> e4m3 codes [rows][D] + one fp32 scale per row (quant_e4m3.cu); D % 16 == 0, D <= 512.
+// With a rowmap, output row r is source row rowmap[r] of the src_rows rows of x, or a zero row where it is negative
+// or not below src_rows.
+int launch_quantize_e4m3(const void* x, int dtype, long long rows, int D, void* codes, float* scales, cudaStream_t st,
+                         const int* rowmap = nullptr, long long src_rows = 0);
 // tiled dQ of the backward, bf16 only.  Nv <= 256 (uint8 winners): the software-pipelined shared-memory gather
 // (bwd_dq_pipe.cu); Nv > 256 (uint16 winners): the L1-resident gather (bwd_dq_tile.cu)
 bool dq_pipe_supported(int Nv, int D, int dtype);

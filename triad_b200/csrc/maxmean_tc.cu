@@ -194,6 +194,33 @@ __device__ __forceinline__ void ragged_chunk(uint32_t (&r)[32], uint32_t starts,
         ++cap;
     }
 }
+// e4m3 variant (kFp8): every column is first multiplied by its slot-row scale sg[c] (broadcast from shared memory, as
+// chunk_max32_scaled), the running maximum propagates NaN, and a caption's maximum is weighted by the row factor
+// rs = t_a with no bf16 rounding.  A caption row with a NaN scale makes that caption's maximum NaN and no other's,
+// since the running maximum restarts at every caption start.
+__device__ __forceinline__ void ragged_chunk_scaled(uint32_t (&r)[32], const float4* sg, uint32_t starts, uint32_t ends,
+                                                    float& run, int& cap, bool valid, float rs, const Params& p, int row0,
+                                                    int lane) {
+#pragma unroll
+    for (int g = 0; g < 8; ++g) {
+        const float4 s = sg[g];
+        const float sc[4] = {s.x, s.y, s.z, s.w};
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const int i = 4 * g + e;
+            const float x = __uint_as_float(r[i]) * sc[e];
+            run = ((starts >> i) & 1u) ? x : fmax_nan(run, x);
+            r[i] = __float_as_uint(run);
+        }
+    }
+    while (ends != 0u) {
+        const int b = __ffs(ends) - 1;
+        ends &= ends - 1u;
+        const float val = valid ? pick32(r, b) * rs : 0.f;
+        store_group_partials(p.part, cap, row0 >> 5, p.G, 1, row0, p.M, p.Nq, val, lane);
+        ++cap;
+    }
+}
 
 // ---- dense-regulariser epilogue (kMode 1: instead of the max-mean reduction; kMode 2: next to it) -----------------
 // N = coef*T*min(T*acc, 0) = (coef*T^2) * min(acc, 0) for T > 0, written as bf16.  A thread owns a ROW of the
@@ -376,7 +403,7 @@ struct TileIter {
 // the dense regulariser (emission warps 8-11 write N = dL/d<q,v> of the non-negative pressure term) in one pass over
 // the similarities — the training step with the reference's full loss needs both of the very same tiles; 1: kMode 2
 // without the max-mean warps (the regulariser-only pass).
-// kFp8: e4m3 operands (kMode 0, no idx: the retrieval forward on a quantized gallery).  A 128-byte swizzle row then
+// kFp8: e4m3 operands (kMode 0, 3 or 4, no idx: the retrieval forward on a quantized gallery).  A 128-byte swizzle row then
 // holds 128 elements, so a k-block is 128 wide (num_kb = D/128 <= 4) and one kind::f8f6f4 MMA step covers K = 32;
 // the ring, the descriptors and the issue loops are those of bf16.  The epilogue multiplies every column by its
 // patch scale before the max and the row by t_a = fp32(fp32(q_scale * row_scale) * (1/T)) after it.  The scales of
@@ -394,12 +421,15 @@ struct TileIter {
 //   rows in token order.  A warp reduction would add a caption's rows in an order set by its offset within a 32-row
 //   group, so the same caption packed after another prefix could score differently in the last bit; this order
 //   depends on the caption alone.  cta_group::2 only (the rows are whole 256-row slots).
+//   With kFp8 the column scales are the slot-row scales in kMode 3 (ragged_chunk_scaled) and the query's token scales
+//   in kMode 4, where the row weight becomes w_t = fp32(fp32(s_t * (1/length)) * (1/T)) with s_t the slot row's scale.
 constexpr int kModeRaggedMax = 3, kModeRaggedMean = 4;
 template <int kCtaGroup, bool kSub, int kMode = 0, bool kFp8 = false>
 __global__ void __launch_bounds__(kEmitThreads, 1)
 maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_v,
                   const __grid_constant__ CUtensorMap tmap_n, const Params p) {
-    static_assert(!kFp8 || kMode == 0, "the e4m3 forward is the max-mean reduction only");
+    static_assert(!kFp8 || kMode == 0 || kMode == kModeRaggedMax || kMode == kModeRaggedMean,
+                  "the e4m3 forward is the max-mean reduction, dense or ragged, only");
     static_assert(kMode != kModeRaggedMax || !kSub, "ragged direction 0: one 256-row slot per tile");
     constexpr bool kEmitN = kMode == 1 || kMode == 2;
     constexpr bool kRagged = kMode == kModeRaggedMax || kMode == kModeRaggedMean;
@@ -704,6 +734,7 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
                     const int cap = __ldg(meta + kSlotMetaCap0) + before + __popc(sw & (0xffffffffu >> (31 - lane))) - 1;
                     r_orig = valid ? r : -1;
                     rs = valid ? 1.0f / (float)__ldg(p.cap_info + 2 * (size_t)cap + 1) : 0.f;
+                    if constexpr (kFp8) { if (valid) rs = (__ldg(p.q_scale + r) * rs) * Tval; }     // w_t
                     prev_m = t.m;
                 }
             } else if (t.m != prev_m) {
@@ -754,8 +785,15 @@ maxmean_tc_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
                     const int2 sw = __ldg(reinterpret_cast<const int2*>(meta + kSlotMetaStarts + c));
                     const int2 ew = __ldg(reinterpret_cast<const int2*>(meta + kSlotMetaEnds + c));
                     tmem_wait_ld();
-                    ragged_chunk(bufA, (uint32_t)sw.x, (uint32_t)ew.x, run, cap, r_orig >= 0, Tval, rs, p, row0, lane);
-                    ragged_chunk(bufB, (uint32_t)sw.y, (uint32_t)ew.y, run, cap, r_orig >= 0, Tval, rs, p, row0, lane);
+                    if constexpr (kFp8) {
+                        ragged_chunk_scaled(bufA, sg_gen + 8 * c, (uint32_t)sw.x, (uint32_t)ew.x, run, cap, r_orig >= 0,
+                                            rs, p, row0, lane);
+                        ragged_chunk_scaled(bufB, sg_gen + 8 * (c + 1), (uint32_t)sw.y, (uint32_t)ew.y, run, cap,
+                                            r_orig >= 0, rs, p, row0, lane);
+                    } else {
+                        ragged_chunk(bufA, (uint32_t)sw.x, (uint32_t)ew.x, run, cap, r_orig >= 0, Tval, rs, p, row0, lane);
+                        ragged_chunk(bufB, (uint32_t)sw.y, (uint32_t)ew.y, run, cap, r_orig >= 0, Tval, rs, p, row0, lane);
+                    }
                 }
                 tc_fence_before();
                 __syncwarp();
@@ -994,10 +1032,16 @@ int launch_maxmean_tc(const void* q, const void* v, const float* row_scale, cons
         p.cap_info = ragged->cap_info;
         if (ragged->direction == 0) {
             p.S = 1;                                          // part[caption][group]
+            if (e4m3)
+                return cta_group == 2 ? launch_t<2, false, kModeRaggedMax, true>(mq, mv, mn, p, n_clusters, st)
+                                      : launch_t<1, false, kModeRaggedMax, true>(mq, mv, mn, p, n_clusters, st);
             return cta_group == 2 ? launch_t<2, false, kModeRaggedMax>(mq, mv, mn, p, n_clusters, st)
                                   : launch_t<1, false, kModeRaggedMax>(mq, mv, mn, p, n_clusters, st);
         }
         if (cta_group != 2) return fail_msg(TRIAD_ERR_UNSUPPORTED, "ragged direction 1: cta_group::2 only");
+        if (e4m3)
+            return n_sub > 1 ? launch_t<2, true, kModeRaggedMean, true>(mq, mv, mn, p, n_clusters, st)
+                             : launch_t<2, false, kModeRaggedMean, true>(mq, mv, mn, p, n_clusters, st);
         return n_sub > 1 ? launch_t<2, true, kModeRaggedMean>(mq, mv, mn, p, n_clusters, st)
                          : launch_t<2, false, kModeRaggedMean>(mq, mv, mn, p, n_clusters, st);
     }

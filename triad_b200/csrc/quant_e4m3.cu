@@ -51,15 +51,25 @@ __device__ __forceinline__ void load16(const __nv_bfloat16* p, float (&v)[16]) {
     }
 }
 
-template <typename T>
+// kGather: output row r quantizes source row rowmap[r], or a zero row (scale 0, codes 0) where rowmap[r] is negative or
+// not below src_rows (the ragged gallery's pack: a slot's rows after its last caption)
+template <typename T, bool kGather>
 __global__ void __launch_bounds__(256)
-quantize_e4m3_kernel(const T* __restrict__ x, long long rows, int D, uint8_t* __restrict__ codes, float* __restrict__ scales) {
+quantize_e4m3_kernel(const T* __restrict__ x, long long rows, int D, uint8_t* __restrict__ codes, float* __restrict__ scales,
+                     const int* __restrict__ rowmap, long long src_rows) {
     const int lane = threadIdx.x & 31;
     const bool act = lane < D / 16;
     const long long step = (long long)gridDim.x * 8;
     for (long long r = (long long)blockIdx.x * 8 + (threadIdx.x >> 5); r < rows; r += step) {
         float v[16];
-        if (act) load16(x + r * D + lane * 16, v);
+        bool ld = act;
+        long long src = r;
+        if constexpr (kGather) {
+            const int m = __ldg(rowmap + r);
+            ld = act && m >= 0 && m < src_rows;
+            src = m;
+        }
+        if (ld) load16(x + src * D + lane * 16, v);
         else {
 #pragma unroll
             for (int e = 0; e < 16; ++e) v[e] = 0.f;
@@ -86,13 +96,21 @@ quantize_e4m3_kernel(const T* __restrict__ x, long long rows, int D, uint8_t* __
 
 }  // namespace
 
-int launch_quantize_e4m3(const void* x, int dtype, long long rows, int D, void* codes, float* scales, cudaStream_t st) {
+int launch_quantize_e4m3(const void* x, int dtype, long long rows, int D, void* codes, float* scales, cudaStream_t st,
+                         const int* rowmap, long long src_rows) {
     long long blocks = (rows + 7) / 8;
     if (blocks > (1ll << 20)) blocks = 1ll << 20;                  // grid-stride beyond 8 M rows
-    if (dtype == TRIAD_DTYPE_BF16)
-        quantize_e4m3_kernel<__nv_bfloat16><<<(unsigned)blocks, 256, 0, st>>>((const __nv_bfloat16*)x, rows, D, (uint8_t*)codes, scales);
-    else
-        quantize_e4m3_kernel<float><<<(unsigned)blocks, 256, 0, st>>>((const float*)x, rows, D, (uint8_t*)codes, scales);
+    const unsigned g = (unsigned)blocks;
+    uint8_t* c = (uint8_t*)codes;
+    if (dtype == TRIAD_DTYPE_BF16) {
+        const __nv_bfloat16* xb = (const __nv_bfloat16*)x;
+        if (rowmap) quantize_e4m3_kernel<__nv_bfloat16, true><<<g, 256, 0, st>>>(xb, rows, D, c, scales, rowmap, src_rows);
+        else quantize_e4m3_kernel<__nv_bfloat16, false><<<g, 256, 0, st>>>(xb, rows, D, c, scales, nullptr, 0);
+    } else {
+        const float* xf = (const float*)x;
+        if (rowmap) quantize_e4m3_kernel<float, true><<<g, 256, 0, st>>>(xf, rows, D, c, scales, rowmap, src_rows);
+        else quantize_e4m3_kernel<float, false><<<g, 256, 0, st>>>(xf, rows, D, c, scales, nullptr, 0);
+    }
     TRIAD_LAUNCH_CHECK("quantize_e4m3_kernel");
     return TRIAD_OK;
 }

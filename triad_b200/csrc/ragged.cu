@@ -5,6 +5,10 @@
 // that does not fit in the rest of the current slot starts a new one, so no caption straddles a slot, and a slot's
 // rows after its last caption are zero.  The zero-padded alternative [n, 77, D] reads 77 rows per caption and
 // scores the padding; at cfg 3's lengths (U[8, 77]) about 90 % of the slot rows are caption rows.
+//
+// The slots are bf16 (triad_ragged_pack) or e4m3 codes with one fp32 scale per slot row (triad_ragged_pack_e4m3, the
+// per-row quantizer of quant_e4m3.cu gathering through the same row map); both storages share the plan, the workspace
+// and the finalize.
 #include "common.cuh"
 
 #include <string.h>
@@ -116,28 +120,30 @@ extern "C" int triad_ragged_pack(const void* src, int dtype, long long src_rows,
     return TRIAD_OK;
 }
 
+extern "C" int triad_ragged_pack_e4m3(const void* src, int dtype, long long src_rows, int D, const int32_t* rowmap,
+                                      long long dst_rows, void* codes, float* scales, void* stream) {
+    if (!src || !rowmap || !codes || !scales) return fail_msg(TRIAD_ERR_BAD_ARG, "ragged_pack_e4m3: null pointer");
+    if (dtype != TRIAD_DTYPE_F32 && dtype != TRIAD_DTYPE_BF16) return fail_msg(TRIAD_ERR_BAD_ARG, "ragged_pack_e4m3: dtype");
+    if (src_rows <= 0 || dst_rows <= 0 || dst_rows % kSlotRows != 0)
+        return fail_msg(TRIAD_ERR_BAD_SHAPE, "ragged_pack_e4m3: bad shape (need dst_rows a multiple of 256)");
+    if (src_rows > 0x7fffffffLL || dst_rows > 0x7fffffffLL) return fail_msg(TRIAD_ERR_BAD_SHAPE, "ragged_pack_e4m3: more than 2^31 rows");
+    if (!tc_e4m3_supported(kSlotRows, D)) return fail_msg(TRIAD_ERR_UNSUPPORTED, "ragged_pack_e4m3: needs D in {128, 256, 384, 512}");
+    if (((uintptr_t)src | (uintptr_t)codes) & 15) return fail_msg(TRIAD_ERR_ALIGNMENT, "ragged_pack_e4m3: src and codes 16-byte aligned");
+    if (((uintptr_t)rowmap | (uintptr_t)scales) & 3) return fail_msg(TRIAD_ERR_ALIGNMENT, "ragged_pack_e4m3: rowmap and scales 4-byte aligned");
+    return launch_quantize_e4m3(src, dtype, dst_rows, D, codes, scales, (cudaStream_t)stream, rowmap, src_rows);
+}
+
 extern "C" size_t triad_retrieve_ragged_workspace_bytes(int Nq, int n_slots, int n_cap, int direction) {
     if (Nq <= 0 || n_slots <= 0 || n_cap <= 0 || (direction != 0 && direction != 1)) return 0;
     return align_up((size_t)Nq * 4, 256) + kCtrlBlockBytes + ragged_part_bytes(Nq, n_slots, n_cap, direction);
 }
 
-extern "C" int triad_retrieve_scores_ragged(const void* q, int Nq, const void* slots, const int32_t* slot_meta,
-                                            const int32_t* cap_info, int n_slots, int n_cap, int D,
-                                            const float* temperature, int direction, float* scores,
-                                            void* ws, size_t ws_bytes, void* stream) {
-    if (!q || !slots || !slot_meta || !cap_info || !temperature || !scores || !ws)
-        return fail_msg(TRIAD_ERR_BAD_ARG, "retrieve_scores_ragged: null pointer");
-    if (direction != 0 && direction != 1) return fail_msg(TRIAD_ERR_BAD_ARG, "retrieve_scores_ragged: direction must be 0 or 1");
-    if (Nq <= 0 || Nq > 65535 || n_slots <= 0 || n_cap < n_slots || (long long)n_cap > (long long)n_slots * kSlotRows ||
-        (long long)n_slots * kSlotRows > 0x7fffffffLL || D <= 0)
-        return fail_msg(TRIAD_ERR_BAD_SHAPE, "retrieve_scores_ragged: bad shape (need 1 <= Nq <= 65535, n_slots <= n_cap <= 256 n_slots)");
-    if (!tc_supported(kSlotRows, D)) return fail_msg(TRIAD_ERR_UNSUPPORTED, "retrieve_scores_ragged: needs D in {64,...,512} (multiple of 64)");
-    if ((((uintptr_t)q | (uintptr_t)slots | (uintptr_t)ws) & 15) || (((uintptr_t)slot_meta | (uintptr_t)cap_info) & 7) ||
-        ((uintptr_t)scores & 3))
-        return fail_msg(TRIAD_ERR_ALIGNMENT, "retrieve_scores_ragged: q, slots and ws 16-byte, metadata 8-byte, scores 4-byte aligned");
-    if (ws_bytes < triad_retrieve_ragged_workspace_bytes(Nq, n_slots, n_cap, direction))
-        return fail_msg(TRIAD_ERR_WORKSPACE, "retrieve_scores_ragged: workspace too small");
-    cudaStream_t st = (cudaStream_t)stream;
+// the scores of the ragged forward (both storages): the workspace split, the kernel and the finalize; the arguments
+// have been checked.  q_scales == NULL: q and slots are bf16; otherwise both hold e4m3 codes, scaled per row by
+// q_scales and slot_scales.
+static int retrieve_ragged(const void* q, const float* q_scales, int Nq, const void* slots, const float* slot_scales,
+                           const int32_t* slot_meta, const int32_t* cap_info, int n_slots, int n_cap, int D,
+                           const float* temperature, int direction, float* scores, void* ws, cudaStream_t st) {
     float* rs = (float*)ws;
     char* fws = (char*)ws + align_up((size_t)Nq * 4, 256);
     int* abort_flag = (int*)fws;
@@ -147,14 +153,16 @@ extern "C" int triad_retrieve_scores_ragged(const void* q, int Nq, const void* s
     int rc;
     if (direction == 0) {
         // rows = the query's tokens (weight 1/Nq), images = the slots
+        const E4m3Args e4m3{q_scales, slot_scales};
         rc = launch_row_scale(nullptr, 1, Nq, rs, st);
         if (rc) return rc;
         rc = launch_maxmean_tc(q, slots, rs, temperature, 1, Nq, n_slots, Nq, kSlotRows, D, part, nullptr, abort_flag,
-                               fwd_cta_group(Nq, 0), 0, nullptr, nullptr, nullptr, st, &ragged);
+                               fwd_cta_group(Nq, 0), 0, nullptr, nullptr, q_scales ? &e4m3 : nullptr, st, &ragged);
     } else {
         // rows = the slot rows (weight 1/length of their caption), the one image = the query
+        const E4m3Args e4m3{slot_scales, q_scales};
         rc = launch_maxmean_tc(slots, q, nullptr, temperature, 1, n_slots * kSlotRows, 1, kSlotRows, Nq, D, part, nullptr,
-                               abort_flag, 2, 0, nullptr, nullptr, nullptr, st, &ragged);
+                               abort_flag, 2, 0, nullptr, nullptr, q_scales ? &e4m3 : nullptr, st, &ragged);
     }
     if (rc) return rc;
     ragged_finalize_kernel<<<ceil_div(n_cap, 256), 256, 0, st>>>(part, n_cap, ceil_div(Nq, 32),
@@ -162,4 +170,50 @@ extern "C" int triad_retrieve_scores_ragged(const void* q, int Nq, const void* s
                                                                  abort_flag);
     TRIAD_LAUNCH_CHECK("ragged_finalize_kernel");
     return TRIAD_OK;
+}
+
+static bool ragged_shape_ok(int Nq, int n_slots, int n_cap, int D) {
+    return !(Nq <= 0 || Nq > 65535 || n_slots <= 0 || n_cap < n_slots || (long long)n_cap > (long long)n_slots * kSlotRows ||
+             (long long)n_slots * kSlotRows > 0x7fffffffLL || D <= 0);
+}
+
+extern "C" int triad_retrieve_scores_ragged(const void* q, int Nq, const void* slots, const int32_t* slot_meta,
+                                            const int32_t* cap_info, int n_slots, int n_cap, int D,
+                                            const float* temperature, int direction, float* scores,
+                                            void* ws, size_t ws_bytes, void* stream) {
+    if (!q || !slots || !slot_meta || !cap_info || !temperature || !scores || !ws)
+        return fail_msg(TRIAD_ERR_BAD_ARG, "retrieve_scores_ragged: null pointer");
+    if (direction != 0 && direction != 1) return fail_msg(TRIAD_ERR_BAD_ARG, "retrieve_scores_ragged: direction must be 0 or 1");
+    if (!ragged_shape_ok(Nq, n_slots, n_cap, D))
+        return fail_msg(TRIAD_ERR_BAD_SHAPE, "retrieve_scores_ragged: bad shape (need 1 <= Nq <= 65535, n_slots <= n_cap <= 256 n_slots)");
+    if (!tc_supported(kSlotRows, D)) return fail_msg(TRIAD_ERR_UNSUPPORTED, "retrieve_scores_ragged: needs D in {64,...,512} (multiple of 64)");
+    if ((((uintptr_t)q | (uintptr_t)slots | (uintptr_t)ws) & 15) || (((uintptr_t)slot_meta | (uintptr_t)cap_info) & 7) ||
+        ((uintptr_t)scores & 3))
+        return fail_msg(TRIAD_ERR_ALIGNMENT, "retrieve_scores_ragged: q, slots and ws 16-byte, metadata 8-byte, scores 4-byte aligned");
+    if (ws_bytes < triad_retrieve_ragged_workspace_bytes(Nq, n_slots, n_cap, direction))
+        return fail_msg(TRIAD_ERR_WORKSPACE, "retrieve_scores_ragged: workspace too small");
+    return retrieve_ragged(q, nullptr, Nq, slots, nullptr, slot_meta, cap_info, n_slots, n_cap, D, temperature, direction,
+                           scores, ws, (cudaStream_t)stream);
+}
+
+extern "C" int triad_retrieve_scores_ragged_e4m3(const void* q_codes, const float* q_scales, int Nq, const void* codes,
+                                                 const float* scales, const int32_t* slot_meta, const int32_t* cap_info,
+                                                 int n_slots, int n_cap, int D, const float* temperature, int direction,
+                                                 float* scores, void* ws, size_t ws_bytes, void* stream) {
+    if (!q_codes || !q_scales || !codes || !scales || !slot_meta || !cap_info || !temperature || !scores || !ws)
+        return fail_msg(TRIAD_ERR_BAD_ARG, "retrieve_scores_ragged_e4m3: null pointer");
+    if (direction != 0 && direction != 1)
+        return fail_msg(TRIAD_ERR_BAD_ARG, "retrieve_scores_ragged_e4m3: direction must be 0 or 1");
+    if (!ragged_shape_ok(Nq, n_slots, n_cap, D))
+        return fail_msg(TRIAD_ERR_BAD_SHAPE, "retrieve_scores_ragged_e4m3: bad shape (need 1 <= Nq <= 65535, n_slots <= n_cap <= 256 n_slots)");
+    if (!tc_e4m3_supported(kSlotRows, D))
+        return fail_msg(TRIAD_ERR_UNSUPPORTED, "retrieve_scores_ragged_e4m3: needs D in {128, 256, 384, 512}");
+    if ((((uintptr_t)q_codes | (uintptr_t)codes | (uintptr_t)ws) & 15) || (((uintptr_t)slot_meta | (uintptr_t)cap_info) & 7) ||
+        (((uintptr_t)q_scales | (uintptr_t)scales | (uintptr_t)scores) & 3))
+        return fail_msg(TRIAD_ERR_ALIGNMENT, "retrieve_scores_ragged_e4m3: codes and ws 16-byte, metadata 8-byte, scales and "
+                                             "scores 4-byte aligned");
+    if (ws_bytes < triad_retrieve_ragged_workspace_bytes(Nq, n_slots, n_cap, direction))
+        return fail_msg(TRIAD_ERR_WORKSPACE, "retrieve_scores_ragged_e4m3: workspace too small");
+    return retrieve_ragged(q_codes, q_scales, Nq, codes, scales, slot_meta, cap_info, n_slots, n_cap, D, temperature,
+                           direction, scores, ws, (cudaStream_t)stream);
 }

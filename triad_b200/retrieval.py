@@ -204,47 +204,69 @@ def ragged_plan(lengths) -> tuple:
 
 class RaggedGallery:
     """A gallery of items with different token counts (captions truncated to their valid tokens), stored without
-    padding: the token rows of whole captions in 256-row slots, ``slots`` bf16 [n_slots * 256, D].
+    padding: the token rows of whole captions in 256-row slots, ``slots`` [n_slots * 256, D].
 
     Captions are placed greedily in order; one that does not fit in the rest of the current slot starts a new slot,
     so no caption straddles a slot, and a slot's rows after its last caption are zero.  ``meta`` (int32
-    [n_slots, 20]) and ``cap_info`` (int32 [n_cap, 2]) describe the layout (``ragged_plan``).  fp32 features are
-    rounded to bf16 when the gallery is built.  Caption lengths must be 1..256.
+    [n_slots, 20]) and ``cap_info`` (int32 [n_cap, 2]) describe the layout (``ragged_plan``).  Caption lengths must
+    be 1..256.
+
+    Two storages (``fp8`` of the builders):
+    - bf16 (default): ``slots`` bf16; fp32 features are rounded to bf16 when the gallery is built; ``scales`` is None.
+    - e4m3: ``slots`` float8_e4m3fn and ``scales`` fp32 [n_slots * 256], one per slot row, each row quantized on its
+      own from the features in their own dtype (``triad_ragged_pack_e4m3``, bit-equal to ``triad_quantize_e4m3`` of
+      that row; fp32 is not rounded to bf16 first).  Rows after a slot's last caption have scale 0 and zero codes.
+      About half the bytes; D must be 128, 256, 384 or 512.
 
     ``retrieve_topk`` and ``dist.sharded_retrieve_topk`` accept it in place of a dense tensor, in both directions;
     ids are caption numbers.  ``len()`` and ``shape[0]`` are the caption count; ``shape`` is (n_cap, D)."""
 
-    def __init__(self, slots: torch.Tensor, meta: torch.Tensor, cap_info: torch.Tensor, lengths: np.ndarray):
+    def __init__(self, slots: torch.Tensor, meta: torch.Tensor, cap_info: torch.Tensor, lengths: np.ndarray,
+                 scales: torch.Tensor = None):
         self.slots = slots
         self.meta = meta
         self.cap_info = cap_info
         self.lengths = lengths
+        self.scales = scales
 
     @classmethod
-    def _build(cls, src: torch.Tensor, src_rows: np.ndarray, lengths: np.ndarray) -> "RaggedGallery":
+    def _build(cls, src: torch.Tensor, src_rows: np.ndarray, lengths: np.ndarray, fp8: bool) -> "RaggedGallery":
         """Caption c is rows src_rows[sum(lengths[:c]) : ...] of src ([rows, D] fp32 or bf16, on the device)."""
-        meta, info = ragged_plan(lengths)
         D = src.shape[1]
+        if fp8 and (D % 128 or not 128 <= D <= 512):
+            raise ValueError(f"RaggedGallery: an fp8 gallery needs D of 128, 256, 384 or 512, got {D}")
+        meta, info = ragged_plan(lengths)
         n_slots = meta.shape[0]
         dev = src.device
         rowmap = np.full(n_slots * SLOT_ROWS, -1, dtype=np.int32)
         firsts = np.repeat(info[:, 0].astype(np.int64), lengths)
         within = np.arange(int(lengths.sum()), dtype=np.int64) - np.repeat(np.cumsum(lengths) - lengths, lengths)
         rowmap[firsts + within] = src_rows
-        slots = torch.empty(n_slots * SLOT_ROWS, D, dtype=torch.bfloat16, device=dev)
         src = src.contiguous()
         if src.dtype not in (torch.float32, torch.bfloat16):
             src = src.float()
         rm = torch.from_numpy(rowmap).to(dev)
+        lib = _lib.load()
+        scales = None
         with ops._on(src):
-            check(_lib.load().triad_ragged_pack(src.data_ptr(), ops._dtype_code(src), src.shape[0], D, rm.data_ptr(),
-                                                slots.shape[0], slots.data_ptr(), ops._stream(dev)), "triad_ragged_pack")
-        return cls(slots, torch.from_numpy(meta).to(dev), torch.from_numpy(info).to(dev), lengths.astype(np.int32))
+            if fp8:
+                slots = torch.empty(n_slots * SLOT_ROWS, D, dtype=torch.float8_e4m3fn, device=dev)
+                scales = torch.empty(n_slots * SLOT_ROWS, dtype=torch.float32, device=dev)
+                check(lib.triad_ragged_pack_e4m3(src.data_ptr(), ops._dtype_code(src), src.shape[0], D, rm.data_ptr(),
+                                                 slots.shape[0], slots.data_ptr(), scales.data_ptr(), ops._stream(dev)),
+                      "triad_ragged_pack_e4m3")
+            else:
+                slots = torch.empty(n_slots * SLOT_ROWS, D, dtype=torch.bfloat16, device=dev)
+                check(lib.triad_ragged_pack(src.data_ptr(), ops._dtype_code(src), src.shape[0], D, rm.data_ptr(),
+                                            slots.shape[0], slots.data_ptr(), ops._stream(dev)), "triad_ragged_pack")
+        return cls(slots, torch.from_numpy(meta).to(dev), torch.from_numpy(info).to(dev), lengths.astype(np.int32),
+                   scales)
 
     @classmethod
-    def from_padded(cls, feats: torch.Tensor, attention_mask) -> "RaggedGallery":
+    def from_padded(cls, feats: torch.Tensor, attention_mask, fp8: bool = False) -> "RaggedGallery":
         """Captions from the text embedder's output: feats [b, L, D] and attention_mask [b, L]; caption i keeps the
-        rows whose mask is non-zero, in order (the reference's truncation for right-padded masks)."""
+        rows whose mask is non-zero, in order (the reference's truncation for right-padded masks).  ``fp8`` stores
+        e4m3 codes with one scale per row instead of bf16."""
         if feats.dim() != 3:
             raise ValueError(f"RaggedGallery.from_padded: feats must be [b, L, D], got {tuple(feats.shape)}")
         b, L, D = feats.shape
@@ -253,18 +275,19 @@ class RaggedGallery:
             raise ValueError(f"RaggedGallery.from_padded: attention_mask must be [{b}, {L}], got {mask.shape}")
         lengths = mask.sum(axis=1)
         src_rows = np.flatnonzero(mask.reshape(-1)).astype(np.int32)
-        return cls._build(feats.reshape(b * L, D), src_rows, lengths)
+        return cls._build(feats.reshape(b * L, D), src_rows, lengths, fp8)
 
     @classmethod
-    def from_list(cls, feats: Sequence[torch.Tensor]) -> "RaggedGallery":
-        """Captions from a list of [L_i, D] tensors (what the reference's embed_tv_subset returns)."""
+    def from_list(cls, feats: Sequence[torch.Tensor], fp8: bool = False) -> "RaggedGallery":
+        """Captions from a list of [L_i, D] tensors (what the reference's embed_tv_subset returns).  ``fp8`` stores
+        e4m3 codes with one scale per row instead of bf16."""
         if len(feats) == 0:
             raise ValueError("RaggedGallery.from_list: need at least one caption")
         if any(t.dim() != 2 for t in feats) or len({t.shape[1] for t in feats}) != 1:
             raise ValueError("RaggedGallery.from_list: captions must be [L_i, D] with one D")
         lengths = np.array([t.shape[0] for t in feats], dtype=np.int64)
         src = torch.cat([t.to(feats[0].dtype) for t in feats])
-        return cls._build(src, np.arange(src.shape[0], dtype=np.int32), lengths)
+        return cls._build(src, np.arange(src.shape[0], dtype=np.int32), lengths, fp8)
 
     @classmethod
     def cat(cls, galleries: Sequence["RaggedGallery"]) -> "RaggedGallery":
@@ -275,6 +298,8 @@ class RaggedGallery:
         D, dev = galleries[0].shape[1], galleries[0].device
         if any(g.shape[1] != D or g.device != dev for g in galleries):
             raise ValueError("RaggedGallery.cat: galleries must share D and device")
+        if len({g.slots.dtype for g in galleries}) != 1:
+            raise ValueError("RaggedGallery.cat: galleries must share their storage (all bf16 or all fp8)")
         metas, infos = [], []
         cap_off = slot_off = 0
         for g in galleries:
@@ -286,8 +311,9 @@ class RaggedGallery:
             infos.append(i)
             cap_off += len(g)
             slot_off += g.n_slots
+        scales = None if galleries[0].scales is None else torch.cat([g.scales for g in galleries])
         return cls(torch.cat([g.slots for g in galleries]), torch.cat(metas), torch.cat(infos),
-                   np.concatenate([g.lengths for g in galleries]))
+                   np.concatenate([g.lengths for g in galleries]), scales)
 
     @property
     def n_slots(self) -> int:
@@ -303,15 +329,18 @@ class RaggedGallery:
 
     @property
     def nbytes(self) -> int:
-        return self.slots.numel() * 2 + self.meta.numel() * 4 + self.cap_info.numel() * 4
+        scale_bytes = 0 if self.scales is None else self.scales.numel() * 4
+        return (self.slots.numel() * self.slots.element_size() + scale_bytes + self.meta.numel() * 4
+                + self.cap_info.numel() * 4)
 
     def __len__(self) -> int:
         return self.cap_info.shape[0]
 
 
 def _scores_ragged(q_feats: torch.Tensor, gallery: RaggedGallery, temperature, direction: int) -> torch.Tensor:
-    """scores[c] of one query (Nq, D) against every caption of a ragged gallery (triad_retrieve_scores_ragged); the
-    query is rounded to bf16 like the gallery."""
+    """scores[c] of one query (Nq, D) against every caption of a ragged gallery: a bf16 gallery rounds the query to
+    bf16 (triad_retrieve_scores_ragged), an fp8 one quantizes it per token on the device
+    (triad_retrieve_scores_ragged_e4m3)."""
     n_cap, D = gallery.shape
     if q_feats.dim() != 2 or q_feats.shape[1] != D:
         raise ValueError(f"query must be [Nq, {D}], got {tuple(q_feats.shape)}")
@@ -319,11 +348,23 @@ def _scores_ragged(q_feats: torch.Tensor, gallery: RaggedGallery, temperature, d
         raise ValueError(f"direction must be 0 or 1, got {direction}")
     lib = _lib.load()
     dev = gallery.device
-    q = q_feats.to(device=dev, dtype=torch.bfloat16).contiguous()
-    Nq = q.shape[0]
+    Nq = q_feats.shape[0]
     T = ops.temperature_tensor(temperature, dev)
     out = torch.empty(n_cap, dtype=torch.float32, device=dev)
     nws = lib.triad_retrieve_ragged_workspace_bytes(Nq, gallery.n_slots, n_cap, direction)
+    if gallery.scales is not None:
+        q = q_feats.to(device=dev).contiguous()
+        q_codes = torch.empty(Nq, D, dtype=torch.uint8, device=dev)
+        q_scales = torch.empty(Nq, dtype=torch.float32, device=dev)
+        _quantize_rows(q, q_codes, q_scales)
+        with ops._on(out):
+            ws = ops._Workspace.get(nws, dev, "retrieve_ragged")
+            check(lib.triad_retrieve_scores_ragged_e4m3(
+                q_codes.data_ptr(), q_scales.data_ptr(), Nq, gallery.slots.data_ptr(), gallery.scales.data_ptr(),
+                gallery.meta.data_ptr(), gallery.cap_info.data_ptr(), gallery.n_slots, n_cap, D, T.data_ptr(), direction,
+                out.data_ptr(), ws.data_ptr(), ws.numel(), ops._stream(dev)), "triad_retrieve_scores_ragged_e4m3")
+        return out
+    q = q_feats.to(device=dev, dtype=torch.bfloat16).contiguous()
     with ops._on(out):
         ws = ops._Workspace.get(nws, dev, "retrieve_ragged")
         check(lib.triad_retrieve_scores_ragged(q.data_ptr(), Nq, gallery.slots.data_ptr(), gallery.meta.data_ptr(),
@@ -338,7 +379,8 @@ def retrieve_topk(q_feats: torch.Tensor, gallery, temperature, k: int, direction
 
     ``gallery`` is an embedding tensor [n_img, Nv, D], an ``Fp8Gallery`` (e4m3 codes with per-patch scales; the
     query is then quantized per token in the same call, and only direction 0 is supported) or a ``RaggedGallery``
-    (captions of different lengths, both directions; the query is rounded to bf16)."""
+    (captions of different lengths, both directions; the query is rounded to bf16 for a bf16 gallery and quantized
+    per token in the same call for an fp8 one)."""
     if isinstance(gallery, Fp8Gallery):
         s = _scores_fp8(q_feats, gallery, temperature, direction)
     elif isinstance(gallery, RaggedGallery):
